@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: rays/sec of the NeRF hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload all|render|train] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload all|render|train] [--impl reference] [--dump-outputs DIR]
 
 Headline workload = BASELINE.json configs[1]: full 800x800 novel-view render, 64 samples/ray, spherical-dome camera
 path, synthetic lego-shaped scene, seeded random-init weights.  One step = one frame per GPU: ray generation ->
@@ -16,6 +16,12 @@ The same JSON line carries sub-records measured in the same run (`--workload all
 
 `--impl reference` times the UNMODIFIED reference (baseline/_ref, staged by scripts/stage_reference.sh; its own
 render_nerf, CPU, all host threads) on a bounded sample of the same workload.  Prints ONE JSON line on rank 0.
+
+`--dump-outputs DIR` writes what the last timed step of the headline path returned to its caller, as float32
+DIR/<name>.npy on rank 0: rgb [H,W,3] and disp [H,W] of rank 0's own frame (render; with several GPUs the other
+ranks' frames are not written), or loss, rgb [B,3] and the updated parameters in state_dict order (--workload
+train).  Weights, poses, jitter and training batches are all seeded, so the same arguments give the same inputs in
+every run, and two builds can be compared output for output.
 """
 import argparse
 import json
@@ -74,6 +80,25 @@ def load_traffic(kernel_key):
         return (e["dram_bytes"], e["source"]) if e else (None, None)
     except Exception:
         return None, None
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: name -> array as out_dir/<name>.npy in float32, at most DUMP_BYTES in all.  Beyond that every
+    array keeps the same fixed, seeded sample of its rows (first axis); the row numbers go to out_dir/<name>_rows.npy."""
+    arrays = {k: np.asarray(v, dtype=np.float32) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_BYTES and a.ndim > 0:
+            # a quarter of the budget for the rows themselves: the float64 row numbers take at most twice that
+            keep = max(1, a.shape[0] * (DUMP_BYTES // 4) // total)
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))
+            np.save(os.path.join(out_dir, name + "_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def workload_config(H, W, N, world):
@@ -148,7 +173,7 @@ def dome_rays_numpy(H, W, pose_idx, begin, count):
 
 
 def reference_arm(args, rank):
-    """The reference's own CPU implementation of the path: baseline/_ref (or /root/reference in the build container)
+    """The reference's own CPU implementation of the path: the checkout oracle.ref_import.reference_root finds,
     imported unmodified, `.cuda()` no-op shim, fp32, all host threads.  Falls back to the torch-CPU port in oracle/
     only when no reference checkout is available, and says which."""
     if rank != 0:
@@ -309,8 +334,9 @@ def setup(args, local_rank, world):
     return c
 
 
-def bench_render(args, c, H, W, N, steps, warmup, fine=0, fused=False, e2e=True, api=True, precision=None):
-    """Frames-per-GPU render (weak scaling): value, MLP-kernel time, e2e through host buffers."""
+def bench_render(args, c, H, W, N, steps, warmup, fine=0, fused=False, e2e=True, api=True, precision=None, dump=False):
+    """Frames-per-GPU render (weak scaling): value, MLP-kernel time, e2e through host buffers.  dump: the frame of the
+    last timed step on the host as r["outputs"]."""
     import torch
     import torch.distributed as dist
     from nerf_simple_b200.engine import FrameRenderer
@@ -340,7 +366,7 @@ def bench_render(args, c, H, W, N, steps, warmup, fine=0, fused=False, e2e=True,
                 pending[b].wait()
             send[b][:, :3].copy_(rgb.view(-1, 3)); send[b][:, 3].copy_(disp.view(-1))
             pending[b] = dist.gather(send[b], recv[b] if rank == 0 else None, dst=0, async_op=True)
-        return rgb
+        return rgb, disp
 
     def drain():
         for b in range(2):
@@ -357,7 +383,7 @@ def bench_render(args, c, H, W, N, steps, warmup, fine=0, fused=False, e2e=True,
     t_begin = time.perf_counter()
     e0.record()
     for i in range(steps):
-        step(i, True)
+        last = step(i, True)
     drain()
     e1.record()
     c.sync_all()
@@ -365,6 +391,9 @@ def bench_render(args, c, H, W, N, steps, warmup, fine=0, fused=False, e2e=True,
     ms_step = c.max_over_ranks(e0.elapsed_time(e1)) / steps
     r = {"value": world * n_rays / (ms_step * 1e-3), "ms_per_step": ms_step, "gpu_launches": rend.launches - launches0,
          "mlp_ms": float(np.mean([a.elapsed_time(b) for a, b in rend.mlp_events])), "t_window": (t_begin, t_end), "fused": rend.fused}
+    if dump:
+        r["outputs"] = {"rgb": last[0].cpu().numpy(), "disp": last[1].cpu().numpy()}
+    del last
     rend.mlp_events.clear()
     if e2e:
         # ---- end to end through the public host-buffer API: pose on the host in, frame on the host out
@@ -446,9 +475,10 @@ def bench_sharded_frame(args, c, H, W, N, frames, warmup=2):
             "frame_assembled_on_every_rank": ok, "clocks": c.sampler.window(t_begin, t_end) if c.sampler else None}
 
 
-def bench_train(args, c, B, N, steps, warmup, loop_api=False, precision=None):
+def bench_train(args, c, B, N, steps, warmup, loop_api=False, precision=None, dump=False):
     """BASELINE configs[2] / configs[4]: training step, B rays x N samples per GPU, fwd+bwd+Adam, data-parallel
-    with one all-reduce of the flat gradient buffer per step (weak scaling)."""
+    with one all-reduce of the flat gradient buffer per step (weak scaling).  dump: loss, rgb and the updated
+    parameters of the last timed step on the host as rec["outputs"]."""
     import torch
     from nerf_simple_b200 import ops
     from nerf_simple_b200.nets import Nerf
@@ -472,12 +502,18 @@ def bench_train(args, c, B, N, steps, warmup, loop_api=False, precision=None):
     t_begin = time.perf_counter()
     e0.record()
     for _ in range(steps):
-        tr.step()                                    # one CUDA-graph replay per step
+        loss = tr.step()                             # one CUDA-graph replay per step
     e1.record()
     timed_launches = tr.launches - l0
     c.sync_all()
     t_end = time.perf_counter()
     ms_step = c.max_over_ranks(e0.elapsed_time(e1)) / steps
+    outputs = None
+    if dump:                                         # before the steps below train the net further
+        # tr._rgb: the trainer's persistent [B,3] buffer of rendered batch colours, which every step (CUDA-graph
+        # replay or eager) overwrites and its MSE loss is taken from; Trainer has no public accessor for it
+        outputs = {"loss": loss.cpu().numpy(), "rgb": tr._rgb.cpu().numpy(),
+                   "params": torch.cat([p.detach().reshape(-1) for p in net.state_dict().values()]).cpu().numpy()}
     value = world * B / (ms_step * 1e-3)
     # ---- e2e, train.py's own data flow (train.py:47-51): the batch is chosen on the HOST and arrives in pinned host
     # memory (rays 24 B + colours 12 B per ray), is copied to the device inside the timed region, and the loss is read
@@ -527,6 +563,8 @@ def bench_train(args, c, B, N, steps, warmup, loop_api=False, precision=None):
            "mlp_forward_tflops": FLOP_FWD * M / (fwd_ms * 1e-3) / 1e12,
            "mlp_backward_tflops": (FLOP_TRAIN - FLOP_FWD) * M / (bwd_ms * 1e-3) / 1e12,
            "clocks": c.sampler.window(t_begin, t_end) if c.sampler else None, "final_loss": float(lv)}
+    if outputs is not None:
+        rec["outputs"] = outputs
     if loop_api and world == 1:
         # ---- the reference's own training loop body, unchanged calls (train.py:47-57): rg.select -> CPU gather of
         # the ground truth -> render_nerf (autograd) -> MSELoss -> backward -> torch.optim.Adam, host tensors in
@@ -582,8 +620,11 @@ def b200_arm(args, rank, local_rank, world):
     H = W = args.res
     N = args.samples
     pk = load_peaks()
+    dump = args.dump_outputs is not None and rank == 0
     if args.workload == "train":
-        rec = bench_train(args, c, args.batch, N, args.steps, max(args.warmup, 20), loop_api=True)
+        rec = bench_train(args, c, args.batch, N, args.steps, max(args.warmup, 20), loop_api=True, dump=dump)
+        if dump:
+            dump_outputs(args.dump_outputs, rec.pop("outputs"))
         if rank == 0:
             rec.update({"higher_is_better": True, "vs_baseline": None, "data": "synthetic"})
             print(json.dumps(rec), flush=True)
@@ -592,7 +633,9 @@ def b200_arm(args, rank, local_rank, world):
         if world > 1:
             dist.destroy_process_group()
         return
-    r = bench_render(args, c, H, W, N, args.steps, args.warmup, fine=args.fine, fused=(args.render_path == "fused"))
+    r = bench_render(args, c, H, W, N, args.steps, args.warmup, fine=args.fine, fused=(args.render_path == "fused"), dump=dump)
+    if dump:
+        dump_outputs(args.dump_outputs, r.pop("outputs"))
     M = H * W * N
     achieved = FLOP_FWD * M / (r["mlp_ms"] * 1e-3) / 1e12
     executed = flop_fwd_exec(args.precision) * M / (r["mlp_ms"] * 1e-3) / 1e12
@@ -671,7 +714,9 @@ def main():
     ap.add_argument("--workload", default="all", choices=["all", "render", "train"])
     ap.add_argument("--batch", type=int, default=4096)
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20, help="timed steps (frames of the headline render workload)")
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed steps of the headline workload: frames (default 20), or train steps with --workload train "
+                         "(default 500: a train step is ~1 ms, enough of them for nvidia-smi to sample the clocks)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--train-steps", type=int, default=400, help="timed steps of the train sub-records")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
@@ -683,10 +728,13 @@ def main():
     ap.add_argument("--fine", type=int, default=0, help="extension: fine samples per ray (64 coarse + N fine)")
     ap.add_argument("--render-path", default="separate", choices=["separate", "fused"],
                     help="separate: raygen, sampler, fused posenc+MLP, compositing kernels; fused: one kernel per frame")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="B200 arm: write the outputs of the last timed step as DIR/<name>.npy (float32, at most 64 MB); "
+                         "with several GPUs, those of rank 0 (its own frame of the render workload)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
-    if args.workload == "train" and args.steps == 20:
-        args.steps = 500            # a train step is ~1 ms: enough of them for nvidia-smi to sample the clocks
+    if args.steps is None:
+        args.steps = 500 if args.workload == "train" else 20
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

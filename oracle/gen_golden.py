@@ -1,9 +1,8 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (read from /root/reference)
-on seeded inputs.  Run in the build container only (the reference does not travel to the GPU
-box): `python oracle/gen_golden.py`.  TEST INFRASTRUCTURE ONLY.
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference on seeded inputs, on the CPU:
+`python oracle/gen_golden.py` (the checkout oracle.ref_import.reference_root finds).  TEST INFRASTRUCTURE ONLY.
 
-The reference hard-codes `.cuda()` (utils/rendering.py:30,68); on this GPU-less container we
-patch Tensor.cuda / Module.cuda to no-ops before calling it (SURVEY.md section 8c).
+The reference hard-codes `.cuda()` (utils/rendering.py:30,68); we patch Tensor.cuda /
+Module.cuda to no-ops before calling it (SURVEY.md section 8c).
 """
 import os
 import sys
@@ -12,14 +11,13 @@ import warnings
 import numpy as np
 import torch
 
-REF = os.environ.get("NERF_REFERENCE", "/root/reference")
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "tests", "golden")
 
 
 def import_reference():
     sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), ".."))
     from oracle.ref_import import import_reference as imp     # .cuda() no-op shim + natsort stand-in
-    return imp(cpu=True, root=REF)
+    return imp(cpu=True)
 
 
 def np_(t):

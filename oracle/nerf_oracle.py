@@ -6,7 +6,7 @@ alpha compositing, forward and analytic backward.  Every function cites the
 reference file:line it follows (paths relative to the reference checkout).
 
 Parity status: PINNED.  `oracle/gen_golden.py` imports the unmodified reference
-from /root/reference (with a `.cuda()` no-op shim -- the reference hard-codes
+(oracle/ref_import.py; with a `.cuda()` no-op shim -- the reference hard-codes
 `.cuda()`, utils/rendering.py:30,68), runs it on seeded inputs and stores its
 outputs + autograd gradients under tests/golden/; tests/test_oracle.py checks this
 restatement against those vectors.  The reference itself ships no tests or golden

@@ -1,8 +1,9 @@
 """Import the UNMODIFIED reference (UCSD-Comp-Imaging/Nerf-Simple) as a live oracle / CPU baseline.
 TEST INFRASTRUCTURE ONLY: used by oracle/gen_golden.py, bench.py's reference arm and tests/.
 
-Where the reference comes from, in order: $NERF_REFERENCE, /root/reference (build container only),
-baseline/_ref (staged by scripts/stage_reference.sh; git-ignored, travels to the GPU box).
+Where the reference comes from, in order: $NERF_REFERENCE, the checkout BASELINE.json's reference_path
+names, baseline/_ref (staged from one of those by __graft_entry__.build() / scripts/stage_reference.sh;
+git-ignored).  Without any of them, callers skip or fall back as they document.
 
 Two shims, both outside the reference's files (SURVEY.md 8c):
   * cpu=True: `Tensor.cuda` / `Module.cuda` become no-ops, because the reference hard-codes `.cuda()`
@@ -14,6 +15,7 @@ Two shims, both outside the reference's files (SURVEY.md 8c):
 from __future__ import annotations
 
 import importlib
+import json
 import os
 import re
 import sys
@@ -22,11 +24,25 @@ import types
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
+def _is_checkout(path):
+    return bool(path) and os.path.isfile(os.path.join(path, "utils", "rendering.py"))
+
+
+def checkout_root():
+    """A reference checkout outside the tree: $NERF_REFERENCE, else BASELINE.json's reference_path; None if neither
+    holds one."""
+    cands = [os.environ.get("NERF_REFERENCE")]
+    try:
+        with open(os.path.join(ROOT, "BASELINE.json")) as fh:
+            cands.append(json.load(fh).get("reference_path"))
+    except (OSError, ValueError):
+        pass
+    return next((c for c in cands if _is_checkout(c)), None)
+
+
 def reference_root():
-    for cand in (os.environ.get("NERF_REFERENCE"), "/root/reference", os.path.join(ROOT, "baseline", "_ref")):
-        if cand and os.path.isfile(os.path.join(cand, "utils", "rendering.py")):
-            return cand
-    return None
+    staged = os.path.join(ROOT, "baseline", "_ref")
+    return checkout_root() or (staged if _is_checkout(staged) else None)
 
 
 def install_natsort_stub():
@@ -61,7 +77,7 @@ def import_reference(cpu=True, root=None, with_dataload=False):
     """Returns (nets, rendering, xyz[, dataload]) modules of the reference, imported from `root`."""
     root = root or reference_root()
     if root is None:
-        raise FileNotFoundError("reference checkout not found (run scripts/stage_reference.sh in the build container)")
+        raise FileNotFoundError("reference checkout not found (set NERF_REFERENCE or run scripts/stage_reference.sh)")
     if cpu:
         cuda_noop_shim()
     install_natsort_stub()

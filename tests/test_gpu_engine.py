@@ -90,3 +90,35 @@ def test_chain_kernel_is_deterministic_over_many_tiles(fused):
                 assert bool(torch.isfinite(rgb).all()) and bool(torch.isfinite(disp).all())
             else:
                 assert torch.equal(rgb, first[0]) and torch.equal(disp, first[1])
+
+
+def test_bench_dump_outputs_is_the_last_timed_frame(tmp_path):
+    """`bench.py --dump-outputs DIR` writes the frame of the last timed step, the same in every run: after 3 warm-up and
+    3 timed frames of the dome path it is frame 2 at the jitter position of the sixth frame."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from nerf_simple_b200.engine import FrameRenderer
+    from nerf_simple_b200.nets import Nerf
+    from nerf_simple_b200.xyz import poses_to_render
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = []
+    for run in ("a", "b"):
+        out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "render", "--res", "64", "--steps", "3",
+                              "--warmup", "3", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / run)],
+                             capture_output=True, text=True, timeout=600, cwd=root)
+        assert out.returncode == 0, out.stderr[-3000:]
+        assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 3
+        assert sorted(os.listdir(tmp_path / run)) == ["disp.npy", "rgb.npy"]
+        dumps.append({k: np.load(tmp_path / run / f"{k}.npy") for k in ("rgb", "disp")})
+    assert dumps[0]["rgb"].dtype == np.float32 and dumps[0]["rgb"].shape == (64, 64, 3) and dumps[0]["disp"].shape == (64, 64)
+    assert all(np.array_equal(dumps[0][k], dumps[1][k]) for k in ("rgb", "disp"))
+    torch.manual_seed(0)
+    net = Nerf().cuda()
+    poses = torch.stack(poses_to_render(4, -30, 30)).cuda()
+    r = FrameRenderer(net, 64, 64, 64 / (2 * np.tan(0.6911112070083618 / 2)), N=64, seed=1, precision="bf16", fused=False)
+    with torch.no_grad():
+        for idx in (0, 1, 2, 0, 1, 2):
+            rgb, disp = r.render_frame(poses, idx)
+    assert np.array_equal(rgb.cpu().numpy(), dumps[0]["rgb"]) and np.array_equal(disp.cpu().numpy(), dumps[0]["disp"])

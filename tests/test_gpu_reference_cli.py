@@ -1,6 +1,6 @@
 """The reference's own CLIs, UNCHANGED, on the B200 engine (north star: "train.py/test.py and configs/lego.yaml
-drive it unchanged"; /root/reference/train.py:28-102, test.py:18-55).  baseline/_ref is the unmodified checkout
-staged by scripts/stage_reference.sh (it travels to the GPU box with the snapshot); the scripts are executed with
+drive it unchanged"; the reference's train.py:28-102, test.py:18-55).  baseline/_ref is the unmodified checkout
+staged by __graft_entry__.build() when a checkout is available (git-ignored; the test skips without it); the scripts are executed with
 `python -m nerf_simple_b200.run`, which only puts the `utils` shim package in front of sys.path."""
 import glob
 import hashlib

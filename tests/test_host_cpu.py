@@ -146,3 +146,28 @@ def test_bench_reference_arm_contract():
     assert line["config"] == bench.workload_config(800, 800, 64, 1)
     assert line["e2e"] == {"value": line["value"], "unit": "rays/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert line["gpu_launches"] == 0 and line["vs_baseline"] is None
+
+
+def test_bench_dump_outputs_format(tmp_path):
+    """`bench.py --dump-outputs`: float32 .npy files, whole arrays up to 64 MB in all, beyond that the same fixed, seeded
+    sample of rows for every array (with the row numbers), at most 64 MB."""
+    import sys
+    sys.path.insert(0, ROOT)
+    import bench
+    rng = np.random.default_rng(1)
+    small = {"loss": np.float64(0.25), "rgb": rng.random((40, 40, 3))}
+    bench.dump_outputs(str(tmp_path / "small"), small)
+    assert sorted(os.listdir(tmp_path / "small")) == ["loss.npy", "rgb.npy"]
+    got = np.load(tmp_path / "small" / "rgb.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, small["rgb"].astype(np.float32))
+    big = {"rgb": rng.random((2200, 2200, 3), dtype=np.float32), "disp": rng.random((2200, 2200), dtype=np.float32)}
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), big)
+        files = sorted(os.listdir(tmp_path / run))
+        assert files == ["disp.npy", "disp_rows.npy", "rgb.npy", "rgb_rows.npy"]
+        assert sum(os.path.getsize(tmp_path / run / f) for f in files) <= 64 << 20
+    rows = np.load(tmp_path / "a" / "rgb_rows.npy").astype(np.int64)
+    assert np.array_equal(rows, np.load(tmp_path / "a" / "disp_rows.npy")) and np.all(np.diff(rows) > 0)
+    assert np.array_equal(rows, np.load(tmp_path / "b" / "rgb_rows.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "rgb.npy"), big["rgb"][rows])
+    assert np.array_equal(np.load(tmp_path / "a" / "disp.npy"), big["disp"][rows])

@@ -216,8 +216,8 @@ def test_adam_restatement_matches_torch():
 
 
 def test_staged_reference_reproduces_goldens(golden_weights):
-    """When the real reference is available (build container: /root/reference; GPU box: baseline/_ref), run it
-    and compare with the committed fixture -- the oracle is pinned by live execution, not only by files."""
+    """When the real reference is available (oracle.ref_import.reference_root), run it and compare with the
+    committed fixture -- the oracle is pinned by live execution, not only by files."""
     import subprocess
     import sys
     import os
