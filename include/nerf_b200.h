@@ -49,8 +49,9 @@ enum {
                      10; the backward un-folds the gradients of both layers exactly (chain rule).            */
   NB200_BF16X3 = 2, /* the same tcgen05 chain with error-compensated bf16 (hi/lo images of activations and
                       weights, three MMA passes per K-block): fp32-class accuracy (<= 1e-4, also with weights
-                      scaled x1.5) on the tensor cores.  Forward / inference only: nb200_mlp_forward with
-                      saved == NULL; its packed buffer has its own size and layout. */
+                      scaled x1.5) on the tensor cores, forward and backward (layer by layer, no fold: the
+                      delta chain and the weight gradients take the same three passes).  Its packed buffer,
+                      saved tensors and scratch have their own sizes and layouts (the *_bytes queries). */
   NB200_BF16_LAYERWISE = 3 /* NB200_BF16 without the fold: every layer of utils/nets.py:34-43 is its own
                       tensor-core layer.  Same packed image, saved-tensor and scratch layouts as NB200_BF16. */
 };

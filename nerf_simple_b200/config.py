@@ -5,8 +5,8 @@ import os
 
 _state = {
     # "bf16": fused tcgen05 kernel (throughput mode, <=1e-2 parity); "fp32": SIMT parity mode (<=1e-4);
-    # "bf16x3": error-compensated bf16 on the tensor cores (<=1e-4 parity at a few hundred TFLOP/s; forward only --
-    # calls that need gradients run the fp32 kernels)
+    # "bf16x3": error-compensated bf16 on the tensor cores (<=1e-4 parity at a few hundred TFLOP/s); Trainer steps run
+    # its tensor-core backward too, autograd calls that need gradients run the fp32 kernels (ops.mlp_apply)
     "precision": os.environ.get("NERF_B200_PRECISION", "bf16"),
     # "reference": draw torch.rand(B,N) from the CPU global generator exactly like
     # utils/rendering.py:28 (bit-identical ts);  "philox": counter-based generator on the device.

@@ -1,4 +1,4 @@
-// Dispatch of the MLP entry points of the C ABI to the fp32 (SIMT) and bf16 (tcgen05) engines.
+// Dispatch of the MLP entry points of the C ABI to the fp32 (SIMT) and bf16 / bf16x3 (tcgen05) engines.
 #include "common.cuh"
 
 namespace nb200 {
@@ -14,13 +14,18 @@ int fp32_backward(int64_t M, const float* const* P, const float* d_out, const vo
 size_t tc_packed_bytes(int x3);
 size_t tc_saved_bytes(int64_t M);
 size_t tc_scratch_bytes(int64_t M, int train);
+size_t tc_saved_bytes_x3(int64_t M);
+size_t tc_scratch_bytes_x3(int64_t M, int train);
 int tc_pack_weights(const float* const* P, void* packed, int x3, cudaStream_t s);
-int tc_forward_x3(int in_mode, const float* in0, const float* in1, int64_t M, int N, const void* packed, float* out, cudaStream_t s);
+int tc_forward_x3(int in_mode, const float* in0, const float* in1, int64_t M, int N, const void* packed, float* out, void* saved,
+                  cudaStream_t s);
 int tc_forward(int in_mode, const float* in0, const float* in1, int64_t M, int N, const void* packed,
                float* out, void* saved, void* scratch, size_t scratch_bytes, int fold, cudaStream_t s);
 int tc_backward(int in_mode, const float* in0, const float* in1, int64_t M, int N, const void* packed,
                 const float* d_out, const void* saved, float* const* G, void* scratch,
                 size_t scratch_bytes, int fold, cudaStream_t s);
+int tc_backward_x3(int64_t M, const void* packed, const float* d_out, const void* saved, float* const* G, void* scratch,
+                   size_t scratch_bytes, cudaStream_t s);
 int tc_render(const float* rays, const float* poses, int H, int W, float f, int64_t ray_begin, const float* ts, uint64_t seed,
               uint64_t offset, int64_t B, int N, float tn, float tf, const void* packed, float* rgb, float* disp, float* acc,
               int fold, cudaStream_t s);
@@ -45,12 +50,14 @@ int nb200_pack_weights(int precision, const float* const* params, void* packed, 
 }
 
 size_t nb200_mlp_saved_bytes(int precision, int64_t M) {
-  if (M < 0 || precision == NB200_BF16X3) return 0;   // bf16x3 is an inference mode
+  if (M < 0) return 0;
+  if (precision == NB200_BF16X3) return nb200::tc_saved_bytes_x3(M);
   return is_bf16(precision) ? nb200::tc_saved_bytes(M) : nb200::fp32_saved_bytes(M);
 }
 
 size_t nb200_mlp_scratch_bytes(int precision, int64_t M, int train) {
-  if (M < 0 || precision == NB200_BF16X3) return 0;
+  if (M < 0) return 0;
+  if (precision == NB200_BF16X3) return nb200::tc_scratch_bytes_x3(M, train);
   return is_bf16(precision) ? nb200::tc_scratch_bytes(M, train) : nb200::fp32_scratch_bytes(M, train);
 }
 
@@ -76,10 +83,7 @@ int nb200_mlp_forward(int precision, int in_mode, const float* in0, const float*
                                nb200::as_stream(stream));
   }
   if (!packed) return NB200_ERR_ARG;
-  if (precision == NB200_BF16X3) {
-    if (saved) return NB200_ERR_UNSUPPORTED;   // forward / inference only: train in NB200_FP32 or NB200_BF16
-    return nb200::tc_forward_x3(in_mode, in0, in1, M, N, packed, out, nb200::as_stream(stream));
-  }
+  if (precision == NB200_BF16X3) return nb200::tc_forward_x3(in_mode, in0, in1, M, N, packed, out, saved, nb200::as_stream(stream));
   return nb200::tc_forward(in_mode, in0, in1, M, N, packed, out, saved, scratch, scratch_bytes,
                            precision == NB200_BF16, nb200::as_stream(stream));
 }
@@ -93,7 +97,6 @@ int nb200_mlp_backward(int precision, int in_mode, const float* in0, const float
   if (!grads) return NB200_ERR_ARG;
   for (int i = 0; i < 24; ++i)
     if (!grads[i]) return NB200_ERR_ARG;
-  if (precision == NB200_BF16X3) return NB200_ERR_UNSUPPORTED;
   if (M == 0) return NB200_OK;  // gradients are accumulated into: nothing to add
   if (!d_out || !saved || ((uintptr_t)d_out & 15) || ((uintptr_t)in0 & 7)) return NB200_ERR_ARG;
   if (precision == NB200_FP32) {
@@ -102,6 +105,8 @@ int nb200_mlp_backward(int precision, int in_mode, const float* in0, const float
                                 nb200::as_stream(stream));
   }
   if (!packed) return NB200_ERR_ARG;
+  if (precision == NB200_BF16X3)
+    return nb200::tc_backward_x3(M, packed, d_out, saved, grads, scratch, scratch_bytes, nb200::as_stream(stream));
   return nb200::tc_backward(in_mode, in0, in1, M, N, packed, d_out, saved, grads, scratch,
                             scratch_bytes, precision == NB200_BF16, nb200::as_stream(stream));
 }

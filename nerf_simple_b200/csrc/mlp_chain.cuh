@@ -76,20 +76,24 @@ constexpr bool kDevBuild = false;
 #endif
 struct SlabC { int src, kb, n, ksteps, both_a; };
 constexpr int kSchedFwd = 0, kSchedBwd = 1, kSchedFwd3 = 2, kSchedFwdFold = 3;   // Fold: layers 0..7, then color_fc.0 as layer 8
+constexpr int kSchedBwd3 = 4;   // bf16x3 delta chain: every kSchedBwd slab twice, hi (against delta_hi and delta_lo) then lo
 __host__ __device__ constexpr int sched_fwd_slabs(int l) { return l == 0 ? 1 : ((l == 5 || l == 9) ? 5 : 4); }
 __host__ __device__ constexpr SlabC sched_fwd_slab(int l, int s) {
   return l == 0 ? SlabC{1, 0, 256, 4, 0}
                 : (l == 9 ? (s < 4 ? SlabC{0, s, 128, 4, 0} : SlabC{1, 0, 128, 2, 0})
                           : (s < 4 ? SlabC{0, s, 256, 4, 0} : SlabC{1, 0, 256, 4, 0}));
 }
+template <int kSched> __host__ __device__ constexpr bool sched_is_bwd() { return kSched == kSchedBwd || kSched == kSchedBwd3; }
 template <int kSched> __host__ __device__ constexpr int sched_slabs(int l) {
-  return kSched == kSchedFwd ? sched_fwd_slabs(l)
+  return kSched == kSchedBwd3 ? 2 * (l == 0 ? 2 : 4)
+         : kSched == kSchedFwd ? sched_fwd_slabs(l)
                              : (kSched == kSchedFwdFold ? sched_fwd_slabs(l >= 8 ? 9 : l) : (kSched == kSchedBwd ? (l == 0 ? 2 : 4) : 2 * sched_fwd_slabs(l)));
 }
 template <int kSched> __host__ __device__ constexpr SlabC sched_slab(int l, int s) {
   if (kSched == kSchedFwd) return sched_fwd_slab(l, s);
   if (kSched == kSchedFwdFold) return sched_fwd_slab(l >= 8 ? 9 : l, s);
   if (kSched == kSchedBwd) return SlabC{0, s, 256, 4, 0};
+  if (kSched == kSchedBwd3) return SlabC{0, s >> 1, 256, 4, (s & 1) ? 0 : 1};
   SlabC c = sched_fwd_slab(l, s >> 1);   // bf16x3: every forward slab twice, hi (against A_hi and A_lo) then lo (A_hi only)
   c.both_a = (s & 1) ? 0 : 1;
   return c;
@@ -101,7 +105,7 @@ struct MmaRing { uint32_t stage, phase; };
 // one copy per layer and slot, was 100 KB of instructions and thrashed the instruction cache of the training kernels).
 // Class representatives: forward 0 | 1 (all plain 256x256 layers) | 5 (skip) | 9 (color_fc.0); delta chain 0 | 1.
 template <int kSched> __host__ __device__ constexpr int sched_class_rep(int l) {
-  return kSched == kSchedBwd ? (l == 0 ? 0 : 1) : ((l == 0 || l == 5 || l == 9) ? l : ((kSched == kSchedFwdFold && l == 8) ? 9 : 1));
+  return sched_is_bwd<kSched>() ? (l == 0 ? 0 : 1) : ((l == 0 || l == 5 || l == 9) ? l : ((kSched == kSchedFwdFold && l == 8) ? 9 : 1));
 }
 
 template <class Epi, int L, int S>
@@ -192,7 +196,7 @@ chain_kernel(const __grid_constant__ typename Epi::Params p) {
     for (int s = 0; s < 2; ++s) {
       mbar_init(bar + kB_Act + 8 * s, 16 * (3 - Epi::kSlots));   // one elected arrive per epilogue warp (8 or 16 warps x 2 CTAs)
       mbar_init(bar + kB_Acc + 8 * s, 1);
-      mbar_init(bar + kB_Written + 8 * s, 8);    // this CTA's 8 epilogue warps of the slot: "tile image complete"
+      mbar_init(bar + kB_Written + 8 * s, 8 * (3 - Epi::kSlots));   // this CTA's 8 (16) epilogue warps of the slot: "tile image complete"
       mbar_init(bar + kB_StoreFree + 8 * s, 1);  // the slot's store warp: "the bulk store has read the image"
     }
     fence_mbar_init();
@@ -225,7 +229,7 @@ chain_kernel(const __grid_constant__ typename Epi::Params p) {
     c.e_img = smem_base + kC_E + slot * kEBytes;
     c.t_lane = tmem_base + (((uint32_t)(warp & 3) * 32u) << 16) + (uint32_t)slot * 256u;
     c.b_img = smem_base + kC_Bias + (uint32_t)slot * 1024u;
-    c.gf = reinterpret_cast<const float*>(p.packed + (Epi::kSched == kSchedFwd3 ? c_layout.f32_off3 : c_layout.f32_off));
+    c.gf = reinterpret_cast<const float*>(p.packed + (Epi::kSched == kSchedFwd3 || Epi::kSched == kSchedBwd3 ? c_layout.f32_off3 : c_layout.f32_off));
     const uint32_t act_remote = mapa_shared(bar + kB_Act + 8 * slot, 0);  // leader's act_ready[slot]
     uint32_t acc_parity = 0, free_parity = 0;
     typename Epi::State st;
@@ -358,14 +362,15 @@ chain_kernel(const __grid_constant__ typename Epi::Params p) {
     }
   } else if (warp >= kCStoreWarp0) {
     // ============================ bulk-store issuer of one slot (training) ============================
-    if (Epi::kBulkStore && lane == 0) {
+    // (single-slot kernels: warp 18 stores, warp 19 idles; store_tile issues every image of the hand-off, e.g. hi and lo)
+    if (Epi::kBulkStore && lane == 0 && (Epi::kSlots == 2 || warp == kCStoreWarp0)) {
       const int slot = warp - kCStoreWarp0;
       TileCtx c;
       c.slot = slot;
       c.a_img = smem_base + kC_A + slot * kABytes;
       c.e_img = smem_base + kC_E + slot * kEBytes;
       uint32_t parity = 0;
-      for (int64_t k = slot; k < my_pt; k += 2) {
+      for (int64_t k = slot; k < my_pt; k += Epi::kSlots) {
         c.tile = 2 * (cid + k * C) + rank;
         if (Epi::kReverseTiles) c.tile = 2 * (PT - 1 - (cid + k * C)) + rank;
         for (int l = -1; l < Epi::kNumLayers; ++l) {
@@ -398,8 +403,8 @@ chain_kernel(const __grid_constant__ typename Epi::Params p) {
         const int rep = sched_class_rep<Epi::kSched>(l);
         if (rep == 0) issue_layer<Epi, 0>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
         else if (rep == 1) issue_layer<Epi, 1>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
-        else if (Epi::kSched != kSchedBwd && rep == 5) issue_layer<Epi, 5>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
-        else if (Epi::kSched != kSchedBwd) issue_layer<Epi, 9>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
+        else if (!sched_is_bwd<Epi::kSched>() && rep == 5) issue_layer<Epi, 5>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
+        else if (!sched_is_bwd<Epi::kSched>()) issue_layer<Epi, 9>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
       }
     }
 #ifdef NB200_DEV
@@ -862,10 +867,17 @@ __device__ __forceinline__ void encode_row3(const float* x, uint32_t img_hi, uin
   }
 }
 
+// Bit k / 8+k of a 16-column step's mask field is column 2k / 2k+1 (the layout of the bf16 chain's mask tensors).
+__device__ __forceinline__ uint32_t relu_bit(int col_in_step) { return 1u << ((col_in_step >> 1) + 8 * (col_in_step & 1)); }
+
+// kSave (training): the hi and lo images of every layer input leave through the store warp (saved layout: mlp_tc.cu,
+// kSavedTileBytes3), and the ReLU masks are formed from the fp32 values in the epilogue.  The outputs are the
+// inference kernel's, bit for bit.
+template <bool kSave>
 struct FwdEpi3 {
   using Params = FwdEpiParams;
   static constexpr bool kHasDbg = false;
-  static constexpr bool kBulkStore = false;
+  static constexpr bool kBulkStore = kSave;
   static constexpr int kSched = kSchedFwd3;
   static constexpr bool kStageBias = true;
   static constexpr int kSlots = 1;
@@ -882,7 +894,20 @@ struct FwdEpi3 {
   __device__ static void init_slot(const TileCtx&) {}
   __device__ static void prefetch(const Params&, State&, const TileCtx&, int) {}
   __device__ static void after_publish(const Params&, State&, const TileCtx&, int) {}
-  __device__ static void store_tile(const Params&, const TileCtx&, int) {}
+  // the store warp: layer l's hand-off (l = -1: posx; 0..8: h0..h7, g; 9: c1; posd rides on h5) as hi and lo images
+  __device__ static void store_tile(const Params& p, const TileCtx& c, int l) {
+    if (!kSave) return;
+    const int64_t T = p.num_tiles;
+    uint8_t* lo = p.saved + kSavedDataTileBytes * (size_t)T;
+    auto put = [&](int t, uint32_t img, uint32_t img_lo) {
+      const size_t off = saved_tensor_off(t, T) + (size_t)c.tile * saved_tile_bytes(t);
+      tma_bulk_s2g(p.saved + off, img, (uint32_t)saved_tile_bytes(t));
+      tma_bulk_s2g(lo + off, img_lo, (uint32_t)saved_tile_bytes(t));
+    };
+    if (l == -1) put(10, c.e_img, c.e_img + kEBytes);
+    else put(l, c.a_img, c.a_img + kABytes);
+    if (l == 5) put(11, c.e_img, c.e_img + kEBytes);   // posd, encoded in front of h5's epilogue
+  }
 
   __device__ static void encode(const float* x, const TileCtx& c, bool dirs) {
     const uint32_t hi = c.e_img, lo = c.e_img + kEBytes;
@@ -914,6 +939,7 @@ struct FwdEpi3 {
     if (ml < 9) {
       const int cbase = c.part * 64;
       const float* ws = c.gf + kF32WSig;   // (read-only global loads at warp-uniform addresses; this mode is not bound by them)
+      uint32_t mbits[2] = {0u, 0u};        // kSave: ReLU mask words of this thread's 64 columns (two 16-column steps each)
 #pragma unroll 1
       for (int q = 0; q < 4; ++q) {
         const int col0 = cbase + q * 16;
@@ -938,6 +964,12 @@ struct FwdEpi3 {
             st.sigma = fmaf(x[3], s0.w, st.sigma); st.sigma = fmaf(x[4], s1.x, st.sigma); st.sigma = fmaf(x[5], s1.y, st.sigma);
             st.sigma = fmaf(x[6], s1.z, st.sigma); st.sigma = fmaf(x[7], s1.w, st.sigma);
           }
+          if (kSave && ml != 8) {
+            uint32_t f = 0u;
+#pragma unroll
+            for (int e = 0; e < 8; ++e) f |= x[e] > 0.f ? relu_bit(8 * j + e) : 0u;
+            if (q & 2) mbits[1] |= f << (16 * (q & 1)); else mbits[0] |= f << (16 * (q & 1));
+          }
           uint32_t h[4], l[4];
 #pragma unroll
           for (int e = 0; e < 4; ++e) split_hi_lo(x[2 * e], x[2 * e + 1], h[e], l[e]);
@@ -946,6 +978,9 @@ struct FwdEpi3 {
           st_shared_v4(a_lo + o, l[0], l[1], l[2], l[3]);
         }
       }
+      if (kSave && ml != 8)   // 8 of the 16 bytes of the (row, column half) entry of mask tensor ml
+        *reinterpret_cast<uint2*>(p.saved + mask_tensor_off3(ml, p.num_tiles) + (size_t)c.tile * 4096 +
+                                  ((size_t)((c.part >> 1) * 128) + c.r) * 16 + (size_t)(c.part & 1) * 8) = make_uint2(mbits[0], mbits[1]);
     } else {
       // color_fc.0 epilogue (128 columns, 32 per thread, ReLU) + color_fc.2 (128 -> 3) in fp32 on CUDA cores; the four
       // threads of a row meet through the (now free) encoding buffer
@@ -955,10 +990,12 @@ struct FwdEpi3 {
       tmem_ld_wait();
       const float4* w4 = reinterpret_cast<const float4*>(c.gf + kF32WC1 + col0);   // color_fc.2's weight, rows 128 floats apart
       float rgb[3] = {0.f, 0.f, 0.f};
+      uint32_t mword = 0u;   // kSave: ReLU mask word of this thread's 32 columns of c1
 #pragma unroll
       for (int q = 0; q < 2; ++q) {
         float4 bq[4];
         load_bias16(c, col0 + 16 * q, bq);
+        uint32_t h[4], lw[4];
 #pragma unroll
         for (int g = 0; g < 4; ++g) {   // 4 columns at a time
           const float b[4] = {bq[g].x, bq[g].y, bq[g].z, bq[g].w};
@@ -971,8 +1008,22 @@ struct FwdEpi3 {
             rgb[k] = fmaf(x[0], wv.x, rgb[k]); rgb[k] = fmaf(x[1], wv.y, rgb[k]);
             rgb[k] = fmaf(x[2], wv.z, rgb[k]); rgb[k] = fmaf(x[3], wv.w, rgb[k]);
           }
+          if (kSave) {   // c1 hi / lo images -> K-block part/2 of A[0] / A[1] (free after color_fc.0's MMAs), 8 columns per chunk
+#pragma unroll
+            for (int e = 0; e < 4; ++e) mword |= x[e] > 0.f ? relu_bit(4 * g + e) << (16 * q) : 0u;
+            split_hi_lo(x[0], x[1], h[2 * (g & 1)], lw[2 * (g & 1)]);
+            split_hi_lo(x[2], x[3], h[2 * (g & 1) + 1], lw[2 * (g & 1) + 1]);
+            if (g & 1) {
+              const uint32_t o = sw_off(c, (uint32_t)(c.part >> 1), (uint32_t)((c.part & 1) * 4 + 2 * q + (g >> 1)));
+              st_shared_v4(c.a_img + o, h[0], h[1], h[2], h[3]);
+              st_shared_v4(c.a_img + kABytes + o, lw[0], lw[1], lw[2], lw[3]);
+            }
+          }
         }
       }
+      if (kSave)   // 4 of the 8 bytes of the (row, column half) entry of mask tensor 8
+        *reinterpret_cast<uint32_t*>(p.saved + mask_tensor_off3(8, p.num_tiles) + (size_t)c.tile * 2048 +
+                                     ((size_t)((c.part >> 1) * 128) + c.r) * 8 + (size_t)(c.part & 1) * 4) = mword;
       const uint32_t xaddr = c.e_img + ((uint32_t)c.part * 128u + c.r) * 16u;
       if (c.part != 0) st_shared_v4(xaddr, __float_as_uint(rgb[0]), __float_as_uint(rgb[1]), __float_as_uint(rgb[2]), __float_as_uint(st.sigma));
       asm volatile("bar.sync 1, 512;" ::: "memory");
@@ -1133,5 +1184,126 @@ struct DgradEpi {
     if (bl == 1) layer_t<false, false>(st, c);
     else if (bl == 2) layer_t<true, true>(st, c);
     else layer_t<true, false>(st, c);
+  }
+};
+
+// ================================================================ backward (dgrad), NB200_BF16X3
+// The delta chain in error-compensated bf16, on FwdEpi3's skeleton: one tile per CTA, 16 epilogue warps at 64 accumulator
+// columns each, delta_hi in A[0] and delta_lo in A[1].  Slabs come from the bwd3 table (hi then lo per K-block), so
+// delta_in = delta_hi W_hi + delta_lo W_hi + delta_hi W_lo in fp32 in TMEM; every delta is formed in fp32 (the
+// colour head, the sigma-head term, the ReLU mask of the forward's fp32 values) and split into hi / lo once.  The
+// store warp writes both images of every delta to the scratch (hi tensors, then lo tensors, in the bf16 layout).
+struct DgradEpi3 {
+  using Params = BwdParams;
+  static constexpr bool kHasDbg = false;
+  static constexpr bool kBulkStore = true;
+  static constexpr int kSched = kSchedBwd3;
+  static constexpr bool kStageBias = false;
+  static constexpr int kSlots = 1;
+  static constexpr int kNumLayers = 9;   // bl = 1..9
+  static constexpr bool kReverseTiles = true;
+  struct State { float4 g; uint2 mask; };
+  __device__ static const SlabDesc* slabs() { return c_layout.bwd3; }
+  __device__ static constexpr int bias_row(int l) { return l; }
+  __device__ static void after_publish(const Params&, State&, const TileCtx&, int) {}
+  // E[0] holds w_sigma (floats 0..255) and color_fc.2's weight (256..639) for the whole kernel
+  __device__ static void init_slot(const TileCtx& c) {
+    for (uint32_t i = threadIdx.x; i < 640u; i += 512u)
+      asm volatile("st.shared.f32 [%0], %1;" ::"r"(c.e_img + i * 4u), "f"(__ldg(c.gf + (i < 256u ? kF32WSig + (int)i : kF32WC1 + (int)(i - 256u)))) : "memory");
+    asm volatile("bar.sync 1, 512;" ::: "memory");
+  }
+  __device__ static __forceinline__ float4 head_ld4(const TileCtx& c, uint32_t i) {
+    float4 v;
+    asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(c.e_img + i * 4u));
+    return v;
+  }
+  // this thread's 8 bytes (64 columns) of the (row, column half) entry of a mask tensor
+  __device__ static void prefetch(const Params& p, State& st, const TileCtx& c, int l) {
+    const int bl = l + 1;   // bl=2 -> h7, ..., bl=9 -> h0; bl=1 yields delta_g (no activation)
+    if (bl >= 2)
+      st.mask = __ldg(reinterpret_cast<const uint2*>(p.saved + mask_tensor_off3(9 - bl, p.num_tiles) + (size_t)c.tile * 4096 +
+                                                     ((size_t)((c.part >> 1) * 128) + c.r) * 16 + (size_t)(c.part & 1) * 8));
+  }
+
+  __device__ static void begin_tile(const Params& p, State& st, const TileCtx& c) {
+    const int64_t T = p.num_tiles;
+    const int64_t m_raw = c.tile * kTileM + c.r;
+    st.g = make_float4(0.f, 0.f, 0.f, 0.f);  // rows past M carry zero gradient
+    if (m_raw < p.M) st.g = __ldg(reinterpret_cast<const float4*>(p.d_out) + m_raw);
+    // delta_c1 = (d_rgb @ Wc1) * (c1 > 0) in fp32: this thread's 32 of the 128 columns
+    const uint32_t cbits = __ldg(reinterpret_cast<const uint32_t*>(p.saved + mask_tensor_off3(8, T) + (size_t)c.tile * 2048 +
+                                                                   ((size_t)((c.part >> 1) * 128) + c.r) * 8 + (size_t)(c.part & 1) * 4));
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const uint32_t col = (uint32_t)(c.part * 32 + j * 8);
+      const uint32_t field = (cbits >> (16 * (j >> 1))) & 0xFFFFu;
+      const int k0 = 4 * (j & 1);
+      float x[8];
+      const float4 a0 = head_ld4(c, 256u + col), a1 = head_ld4(c, 256u + col + 4u);
+      x[0] = st.g.x * a0.x; x[1] = st.g.x * a0.y; x[2] = st.g.x * a0.z; x[3] = st.g.x * a0.w;
+      x[4] = st.g.x * a1.x; x[5] = st.g.x * a1.y; x[6] = st.g.x * a1.z; x[7] = st.g.x * a1.w;
+      const float4 b0 = head_ld4(c, 384u + col), b1 = head_ld4(c, 384u + col + 4u);
+      x[0] = fmaf(st.g.y, b0.x, x[0]); x[1] = fmaf(st.g.y, b0.y, x[1]); x[2] = fmaf(st.g.y, b0.z, x[2]); x[3] = fmaf(st.g.y, b0.w, x[3]);
+      x[4] = fmaf(st.g.y, b1.x, x[4]); x[5] = fmaf(st.g.y, b1.y, x[5]); x[6] = fmaf(st.g.y, b1.z, x[6]); x[7] = fmaf(st.g.y, b1.w, x[7]);
+      const float4 c0 = head_ld4(c, 512u + col), c1 = head_ld4(c, 512u + col + 4u);
+      x[0] = fmaf(st.g.z, c0.x, x[0]); x[1] = fmaf(st.g.z, c0.y, x[1]); x[2] = fmaf(st.g.z, c0.z, x[2]); x[3] = fmaf(st.g.z, c0.w, x[3]);
+      x[4] = fmaf(st.g.z, c1.x, x[4]); x[5] = fmaf(st.g.z, c1.y, x[5]); x[6] = fmaf(st.g.z, c1.z, x[6]); x[7] = fmaf(st.g.z, c1.w, x[7]);
+      uint32_t h[4], l[4];
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        split_hi_lo(x[2 * e], x[2 * e + 1], h[e], l[e]);
+        const uint32_t m = pair_mask_word(field, k0 + e);
+        h[e] &= m; l[e] &= m;
+      }
+      const uint32_t o = sw_off(c, (uint32_t)(c.part >> 1), (uint32_t)((c.part & 1) * 4 + j));
+      st_shared_v4(c.a_img + o, h[0], h[1], h[2], h[3]);
+      st_shared_v4(c.a_img + kABytes + o, l[0], l[1], l[2], l[3]);
+    }
+  }
+
+  // the store warp: delta tile images (hi from A[0], lo from A[1]) -> scratch, read back by wgrad
+  __device__ static void store_tile(const Params& p, const TileCtx& c, int l) {
+    const int64_t T = p.num_tiles;
+    const uint64_t pol = l2_policy_evict_first();
+    const uint32_t bytes = l == -1 ? 32768u : 65536u;
+    const size_t off = delta_tensor_off(l + 1, T) + (size_t)c.tile * bytes;   // l = -1: delta_c1 (tensor 0)
+    tma_bulk_s2g_hint(p.dscr + off, c.a_img, bytes, pol);
+    tma_bulk_s2g_hint(p.dscr + kDeltaTileBytes * (size_t)T + off, c.a_img + kABytes, bytes, pol);
+  }
+
+  __device__ static void layer(const Params&, State& st, const TileCtx& c, int l) {
+    const int bl = l + 1;
+    const int cbase = c.part * 64;
+#pragma unroll 1
+    for (int q = 0; q < 4; ++q) {
+      const int col0 = cbase + q * 16;
+      uint32_t a[16];
+      tmem_ld16(c.t_lane + col0, a);
+      tmem_ld_wait();
+      const uint32_t field = ((q & 2) ? st.mask.y : st.mask.x) >> (16 * (q & 1)) & 0xFFFFu;
+#pragma unroll
+      for (int j = 0; j < 2; ++j) {
+        float x[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) x[e] = __uint_as_float(a[8 * j + e]);
+        if (bl == 2) {   // + d_sigma * w_sigma (the sigma head reads h7)
+          const float4 s0 = head_ld4(c, (uint32_t)(col0 + 8 * j)), s1 = head_ld4(c, (uint32_t)(col0 + 8 * j + 4));
+          x[0] = fmaf(st.g.w, s0.x, x[0]); x[1] = fmaf(st.g.w, s0.y, x[1]); x[2] = fmaf(st.g.w, s0.z, x[2]); x[3] = fmaf(st.g.w, s0.w, x[3]);
+          x[4] = fmaf(st.g.w, s1.x, x[4]); x[5] = fmaf(st.g.w, s1.y, x[5]); x[6] = fmaf(st.g.w, s1.z, x[6]); x[7] = fmaf(st.g.w, s1.w, x[7]);
+        }
+        uint32_t h[4], lo[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          split_hi_lo(x[2 * e], x[2 * e + 1], h[e], lo[e]);
+          if (bl >= 2) {   // bl=1 yields delta_g: layers_2 has no activation
+            const uint32_t m = pair_mask_word(field, 4 * j + e);
+            h[e] &= m; lo[e] &= m;
+          }
+        }
+        const uint32_t o = sw_off(c, (uint32_t)c.part, (uint32_t)(2 * q + j));
+        st_shared_v4(c.a_img + o, h[0], h[1], h[2], h[3]);
+        st_shared_v4(c.a_img + kABytes + o, lo[0], lo[1], lo[2], lo[3]);
+      }
+    }
   }
 };

@@ -12,6 +12,7 @@
 #include <string.h>
 
 #include <mutex>
+#include <type_traits>
 #include <utility>
 
 #include "common.cuh"
@@ -74,12 +75,14 @@ struct PackedLayout {
   SlabDesc fold[8];
   uint32_t f32_off;  // fp32 section: bias[11][256] | wsig[256] | bsig(+pad 4) | wc1[3][128] | bc1[3](+pad) | fold tail
   uint32_t total_bytes;
-  // NB200_BF16X3 (error-compensated bf16, forward only): its own packed buffer = per K-block a hi slab bf16(W) and a lo
-  // slab bf16(W - bf16(W)), then the same fp32 tail
+  // NB200_BF16X3 (error-compensated bf16): its own packed buffer = per K-block a hi slab bf16(W) and a lo slab
+  // bf16(W - bf16(W)), then the same fp32 tail, then the delta chain's transposed slabs in the same hi / lo pairs
   int num_fwd3;
   SlabDesc fwd3[2 * kMaxSlabs];
   uint32_t f32_off3;
   uint32_t total_bytes3;
+  int num_bwd3;
+  SlabDesc bwd3[2 * kMaxSlabs];   // (behind every older field: the bf16 kernels' constant-bank offsets do not move)
 };
 constexpr int kF32Bias = 0, kF32WSig = 2816, kF32BSig = 3072, kF32WC1 = 3076, kF32BC1 = 3460,
               kF32Floats = 3520;
@@ -94,7 +97,7 @@ static bool h_layout_built = false;
 // Everything CUDA caches per device (constant-bank copies, function attributes, the architecture check) is keyed
 // by the current device, so one process can drive several GPUs; the tables are guarded by one mutex.
 constexpr int kMaxDevices = 64;
-struct DeviceState { bool layout_uploaded, attr_fwd, attr_render, attr_bwd, attr_x3; int arch; };
+struct DeviceState { bool layout_uploaded, attr_fwd, attr_render, attr_bwd, attr_x3, attr_bwd3; int arch; };
 static DeviceState g_dev[kMaxDevices];
 static std::mutex g_mu;
 static int current_device(int* dev) {
@@ -196,7 +199,20 @@ static void build_layout() {
   }
   h_layout.num_fwd3 = x.s;
   h_layout.f32_off3 = x.off;
-  h_layout.total_bytes3 = x.off + kF32Floats * (uint32_t)sizeof(float);
+  // bf16x3 delta chain: every transposed slab of `bwd` twice (hi: consumed with delta_hi and delta_lo; lo: with
+  // delta_hi), behind the fp32 tail, so that the forward slabs and the tail keep their offsets
+  LayoutBuilder y;
+  y.arr = h_layout.bwd3; y.off = x.off + kF32Floats * (uint32_t)sizeof(float); y.s = 0;
+  for (int i = 0; i < h_layout.num_bwd; ++i) {
+    const SlabDesc& d = h_layout.bwd[i];
+    for (int lo = 0; lo < 2; ++lo) {
+      y.add(d.ml, d.layer, 1, d.n, d.wcol0, d.kvalid, d.ldw, d.src, d.kb, d.ksteps, lo, lo ? 0 : 1);
+      h_layout.bwd3[y.s - 1].first = (uint8_t)(d.first && lo == 0);
+      h_layout.bwd3[y.s - 1].last = (uint8_t)(d.last && lo == 1);
+    }
+  }
+  h_layout.num_bwd3 = y.s;
+  h_layout.total_bytes3 = y.off;
 }
 
 // The MMA warps walk a compile-time schedule (mlp_chain.cuh: sched_slab), the weight producers and the packer this
@@ -235,7 +251,7 @@ __global__ void __launch_bounds__(256) pack_slabs_kernel(ParamPtrs P, uint8_t* _
   const int slab = (int)blockIdx.x / kPackSplit, part = (int)blockIdx.x % kPackSplit;
   const bool is_bwd = !kX3 && slab >= c_layout.num_fwd;
   const bool is_fold = !kX3 && slab >= c_layout.num_fwd + c_layout.num_bwd;
-  const SlabDesc d = kX3 ? c_layout.fwd3[slab]
+  const SlabDesc d = kX3 ? (slab < c_layout.num_fwd3 ? c_layout.fwd3[slab] : c_layout.bwd3[slab - c_layout.num_fwd3])
                          : (is_fold ? c_layout.fold[slab - c_layout.num_fwd - c_layout.num_bwd]
                                     : (is_bwd ? c_layout.bwd[slab - c_layout.num_fwd] : c_layout.fwd[slab]));
   // the folded weight was written to the packed buffer's fp32 tail by fold_weights_kernel (same stream, before this kernel)
@@ -403,6 +419,12 @@ __host__ __device__ __forceinline__ size_t saved_tensor_off(int t, int64_t num_t
 __host__ __device__ __forceinline__ size_t saved_tile_bytes(int t) {
   return t < 9 ? 65536 : (t == 9 ? 32768 : 16384);
 }
+// bf16x3 training: the data tensors above once for the hi images bf16(x) and once for the lo images bf16(x - hi) (lo
+// tensor t at kSavedDataTileBytes * T + saved_tensor_off(t, T)), then the same mask tensors, formed from the fp32 values
+constexpr size_t kSavedTileBytes3 = 2 * kSavedDataTileBytes + kMaskTileBytes;
+__host__ __device__ __forceinline__ size_t mask_tensor_off3(int t, int64_t num_tiles) {
+  return (2 * kSavedDataTileBytes + (size_t)t * 4096) * (size_t)num_tiles;
+}
 
 // Encode 3 coordinates with L levels into the bf16 operand row `r` of a SWIZZLE_128B image:
 // cols [x0,x1,x2, per coordinate: sin(2^i x), cos(2^i x) ...], zero padded to NCH*8 columns.
@@ -461,7 +483,8 @@ static bool check_schedules() {
          schedule_matches<kSchedBwd>(h_layout.bwd, h_layout.num_bwd, 9) &&
          schedule_matches<kSchedFwdFold>(h_layout.fwdf, h_layout.num_fwdf, kNumFoldLayers) &&
          schedule_matches<kSchedBwd>(h_layout.bwdf, h_layout.num_bwdf, 8) &&
-         schedule_matches<kSchedFwd3>(h_layout.fwd3, h_layout.num_fwd3, kNumMmaLayers);
+         schedule_matches<kSchedFwd3>(h_layout.fwd3, h_layout.num_fwd3, kNumMmaLayers) &&
+         schedule_matches<kSchedBwd3>(h_layout.bwd3, h_layout.num_bwd3, 9);
 }
 
 // ------------------------------------------------------------------------------ host API
@@ -485,6 +508,11 @@ constexpr size_t kPadC0 = 0, kPadSkip = kPadC0 + 128 * kPadPitchWide, kPadL00 = 
                  kPadFloats = kPadFoldS + 128;
 size_t tc_scratch_bytes(int64_t M, int train) {
   return train ? (size_t)train_tiles(M) * kDeltaTileBytes + kPadFloats * sizeof(float) : 0;
+}
+// bf16x3: saved = hi data | lo data | masks; scratch = hi deltas | lo deltas | pad images
+size_t tc_saved_bytes_x3(int64_t M) { return (size_t)train_tiles(M) * kSavedTileBytes3; }
+size_t tc_scratch_bytes_x3(int64_t M, int train) {
+  return train ? (size_t)train_tiles(M) * 2 * kDeltaTileBytes + kPadFloats * sizeof(float) : 0;
 }
 
 // grad[r, c] += pad[r, c] for the three padded images (one thread per padded float4 group)
@@ -534,7 +562,7 @@ int tc_pack_weights(const float* const* P, void* packed, int x3, cudaStream_t s)
   NB_TRY_RC(ensure_layout());
   ParamPtrs pp;
   for (int i = 0; i < 24; ++i) pp.p[i] = P[i];
-  const int nslabs = x3 ? h_layout.num_fwd3 : h_layout.num_fwd + h_layout.num_bwd + h_layout.num_fold;
+  const int nslabs = x3 ? h_layout.num_fwd3 + h_layout.num_bwd3 : h_layout.num_fwd + h_layout.num_bwd + h_layout.num_fold;
   if (!x3) {
     fold_weights_kernel<<<kFoldWBlocks, 256, 0, s>>>(pp, reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(packed) + h_layout.f32_off));
     NB_LAUNCH_CHECK("fold_weights_kernel");
@@ -591,7 +619,8 @@ static int get_tmaps(const void* packed, TmapPair* out, int x3 = 0) {   // retur
   static TmapPair cache[8];
   static int used = 0, next = 0;
   // keyed by the image's row count too: torch's allocator hands a freed bf16 buffer's address to a bf16x3 buffer
-  const uint32_t rows = (x3 ? h_layout.f32_off3 : h_layout.f32_off) / 128;
+  // (the bf16x3 map spans the whole buffer: its delta-chain slabs lie behind the fp32 tail)
+  const uint32_t rows = (x3 ? h_layout.total_bytes3 : h_layout.f32_off) / 128;
   for (int i = 0; i < used; ++i)
     if (cache[i].packed == packed && cache[i].dev == dev && cache[i].rows == rows) { *out = cache[i]; return NB200_OK; }
   static EncodeTiledFn encode = nullptr;
@@ -690,17 +719,26 @@ int tc_forward(int in_mode, const float* in0, const float* in1, int64_t M, int N
   return NB200_OK;
 }
 
+// one tile in flight per CTA: one pair-tile per cluster and round
+static int chain_grid_x3(int64_t T) {
+  const int64_t PT = (T + 1) / 2, maxc = sm_count() / 2;
+  return (int)(2 * (PT < maxc ? PT : maxc));
+}
+
 // NB200_BF16X3: error-compensated bf16 on the same chain skeleton (one tile in flight per CTA, three MMA passes per
 // K-block: A_hi W_hi + A_lo W_hi + A_hi W_lo, fp32 accumulation in TMEM): fp32-class accuracy on the tensor cores.
+// With `saved` (training) the same kernel also stores the hi and lo image of every layer input and the ReLU masks
+// (kSavedTileBytes3 per tile of train_tiles(M)); its outputs are the inference kernel's, bit for bit.
 int tc_forward_x3(int in_mode, const float* in0, const float* in1, int64_t M, int N, const void* packed, float* out,
-                  cudaStream_t s) {
+                  void* saved, cudaStream_t s) {
   NB_TRY_RC(check_arch());
   NB_TRY_RC(ensure_layout());
   NB_TRY_RC(ensure_attr(&DeviceState::attr_x3, []() -> int {
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<FwdEpi3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCSmemLaunch));
+    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<FwdEpi3<false>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCSmemLaunch));
+    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<FwdEpi3<true>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCSmemLaunch));
     return NB200_OK;
   }));
-  const int64_t T = ceil_div64(M, kTileM);
+  const int64_t T = saved ? train_tiles(M) : ceil_div64(M, kTileM);
   FwdEpiParams p;
   memset(&p, 0, sizeof(p));
   TmapPair tm;
@@ -710,10 +748,11 @@ int tc_forward_x3(int in_mode, const float* in0, const float* in1, int64_t M, in
   p.nshift = (N > 0 && (N & (N - 1)) == 0) ? __builtin_ctz((unsigned)N) : -1;
   p.packed = reinterpret_cast<const uint8_t*>(packed);
   p.out = out;
+  p.saved = reinterpret_cast<uint8_t*>(saved);
   p.num_tiles = T;
-  const int64_t PT = (T + 1) / 2, maxc = sm_count() / 2;
-  const int grid = (int)(2 * (PT < maxc ? PT : maxc));
-  chain_kernel<FwdEpi3><<<grid, kCThreads, kCSmemLaunch, s>>>(p);
+  const int grid = chain_grid_x3(T);
+  if (saved) chain_kernel<FwdEpi3<true>><<<grid, kCThreads, kCSmemLaunch, s>>>(p);
+  else chain_kernel<FwdEpi3<false>><<<grid, kCThreads, kCSmemLaunch, s>>>(p);
   NB_LAUNCH_CHECK("chain_kernel<FwdEpi3>");
   return NB200_OK;
 }
@@ -752,13 +791,58 @@ int tc_render(const float* rays, const float* poses, int H, int W, float f, int6
   return NB200_OK;
 }
 
+// One wgrad item: dW (+)= (delta tensor dt of `ds`)^T (saved tensor st of `sv`), rows of the layer's weight from col0.
+static void wgrad_item(WItem& w, const uint8_t* ds, const uint8_t* sv, int64_t T, float* pad, float* const* G, int dt, int st,
+                       int layer, int ldw, int col0, int ncols, int nrows, bool bias) {
+  w.a_ptr = ds + delta_tensor_off(dt, T);
+  w.a_tile_bytes = dt == 0 ? 32768u : 65536u;
+  w.a_chunks = dt == 0 ? 2 : 4;
+  w.b_ptr = sv + saved_tensor_off(st, T);
+  w.b_tile_bytes = (uint32_t)saved_tile_bytes(st);
+  w.b_chunks = st >= 10 ? 1 : 4;
+  w.n_mma = st >= 10 ? 64 : 256;
+  w.dW = G[2 * layer]; w.db = bias ? G[2 * layer + 1] : nullptr;
+  w.ldw = ldw; w.col0 = col0; w.ncols = ncols; w.nrows = nrows;
+  if (ldw & 3) {  // unaligned rows: flush the whole (zero-padded) accumulator into the padded image
+    w.dW = pad + (layer == L_C0 ? kPadC0 : (layer == L_SKIP ? kPadSkip : kPadL00));
+    w.ldw = layer == L0_0 ? kPadPitchX : kPadPitchWide;
+    w.ncols = w.n_mma;
+  }
+  w.cost = (w.a_chunks + w.b_chunks) * 16;
+  w.head = 0; w.x_ptr = nullptr; w.x_tile_bytes = 0; w.x_chunks = 0; w.hW = nullptr; w.hb = nullptr;
+}
+// the sigma / colour head gradients ride on the item that stages their input (h7 / an extra c1 slab)
+static void wgrad_head(WItem& w, const uint8_t* sv, int64_t T, float* const* G, int which, int st, int layer) {
+  w.head = which; w.hW = G[2 * layer]; w.hb = G[2 * layer + 1];
+  if (which == 2) {
+    w.x_ptr = sv + saved_tensor_off(st, T); w.x_tile_bytes = (uint32_t)saved_tile_bytes(st); w.x_chunks = 2;
+    w.cost += w.x_chunks * 16;
+  }
+}
+// Relative time per tile of each item kind, MEASURED per CTA on B200 (global-timer trace of the mixed
+// kernel; bytes alone mis-predict it because small stages are latency-bound in the ring and the head
+// items add CUDA-core work before a stage is released): plain 256x256 item = 100.
+static void wgrad_costs(WItem* items, int n) {
+  for (int i = 0; i < n; ++i) {
+    WItem& w = items[i];
+    const int chunks = w.a_chunks + w.b_chunks + w.x_chunks;
+    int c = chunks == 8 ? 100 : (chunks == 6 ? 85 : (w.db ? 85 : 77));
+#ifndef NB_WG_HEAD6_COST
+#define NB_WG_HEAD6_COST 130   // same-box A/B of the train step: 90 -> 1.085 ms, 106 -> 1.041, 124 -> 1.020, 140 -> 1.021
+#endif
+    if (w.head == 1) c = chunks == 8 ? 124 : NB_WG_HEAD6_COST;   // (the 6-chunk carrier of the folded chain)
+    if (w.head == 2) c = 83;
+    w.cost = c;
+  }
+}
+
 int tc_backward(int, const float*, const float*, int64_t M, int, const void* packed, const float* d_out,
                 const void* saved, float* const* G, void* scratch, size_t scratch_bytes, int fold, cudaStream_t s) {
   NB_TRY_RC(check_arch());
   NB_TRY_RC(ensure_layout());
   if (!scratch || scratch_bytes < tc_scratch_bytes(M, 1)) return NB200_ERR_WORKSPACE;
   NB_TRY_RC(ensure_attr(&DeviceState::attr_bwd, []() -> int {
-    NB_CUDA_CHECK(cudaFuncSetAttribute(mlp_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgSmemLaunch));
+    NB_CUDA_CHECK(cudaFuncSetAttribute(mlp_wgrad_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgSmemLaunch));
     NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<DgradEpi<false>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCSmemLaunch));
     NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<DgradEpi<true>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCSmemLaunch));
     return NB200_OK;
@@ -787,33 +871,9 @@ int tc_backward(int, const float*, const float*, int64_t M, int, const void* pac
   wp.T = T; wp.M = M; wp.d_out = d_out;
   int n = 0;
   auto item = [&](int dt, int st, int layer, int ldw, int col0, int ncols, int nrows, bool bias) {
-    WItem& w = wp.items[n++];
-    w.a_ptr = ds + delta_tensor_off(dt, T);
-    w.a_tile_bytes = dt == 0 ? 32768u : 65536u;
-    w.a_chunks = dt == 0 ? 2 : 4;
-    w.b_ptr = sv + saved_tensor_off(st, T);
-    w.b_tile_bytes = (uint32_t)saved_tile_bytes(st);
-    w.b_chunks = st >= 10 ? 1 : 4;
-    w.n_mma = st >= 10 ? 64 : 256;
-    w.dW = G[2 * layer]; w.db = bias ? G[2 * layer + 1] : nullptr;
-    w.ldw = ldw; w.col0 = col0; w.ncols = ncols; w.nrows = nrows;
-    if (ldw & 3) {  // unaligned rows: flush the whole (zero-padded) accumulator into the padded image
-      w.dW = pad + (layer == L_C0 ? kPadC0 : (layer == L_SKIP ? kPadSkip : kPadL00));
-      w.ldw = layer == L0_0 ? kPadPitchX : kPadPitchWide;
-      w.ncols = w.n_mma;
-    }
-    w.cost = (w.a_chunks + w.b_chunks) * 16;
-    w.head = 0; w.x_ptr = nullptr; w.x_tile_bytes = 0; w.x_chunks = 0; w.hW = nullptr; w.hb = nullptr;
+    wgrad_item(wp.items[n++], ds, sv, T, pad, G, dt, st, layer, ldw, col0, ncols, nrows, bias);
   };
-  // the sigma / colour head gradients ride on the item that stages their input (h7 / an extra c1 slab)
-  auto head = [&](int which, int st, int layer) {
-    WItem& w = wp.items[n - 1];
-    w.head = which; w.hW = G[2 * layer]; w.hb = G[2 * layer + 1];
-    if (which == 2) {
-      w.x_ptr = sv + saved_tensor_off(st, T); w.x_tile_bytes = (uint32_t)saved_tile_bytes(st); w.x_chunks = 2;
-      w.cost += w.x_chunks * 16;
-    }
-  };
+  auto head = [&](int which, int st, int layer) { wgrad_head(wp.items[n - 1], sv, T, G, which, st, layer); };
   if (fold) {
     item(0, 7, L_C0, kHidden + kPosD, 0, kHidden, kHidden / 2, true);      // Gm = delta_c1^T h7 -> pad image of color_fc.0
     wp.items[n - 1].db = pad + kPadFoldS;                                   //   column sums of delta_c1 (un-folded below)
@@ -836,25 +896,12 @@ int tc_backward(int, const float*, const float*, int64_t M, int, const void* pac
   item(7, 1, L0_2, kHidden, 0, kHidden, kHidden, true);
   item(8, 0, L0_1, kHidden, 0, kHidden, kHidden, true);
   item(9, 10, L0_0, kPosX, 0, kPosX, kHidden, true);                        // layers_0.0 <- posx
-  // Relative time per tile of each item kind, MEASURED per CTA on B200 (global-timer trace of the mixed
-  // kernel; bytes alone mis-predict it because small stages are latency-bound in the ring and the head
-  // items add CUDA-core work before a stage is released): plain 256x256 item = 100.
-  for (int i = 0; i < n; ++i) {
-    WItem& w = wp.items[i];
-    const int chunks = w.a_chunks + w.b_chunks + w.x_chunks;
-    int c = chunks == 8 ? 100 : (chunks == 6 ? 85 : (w.db ? 85 : 77));
-#ifndef NB_WG_HEAD6_COST
-#define NB_WG_HEAD6_COST 130   // same-box A/B of the train step: 90 -> 1.085 ms, 106 -> 1.041, 124 -> 1.020, 140 -> 1.021
-#endif
-    if (w.head == 1) c = chunks == 8 ? 124 : NB_WG_HEAD6_COST;   // (the 6-chunk carrier of the folded chain)
-    if (w.head == 2) c = 83;
-    w.cost = c;
-  }
+  wgrad_costs(wp.items, n);
 #ifdef NB200_DEV   // developer probe: time one item alone (leaves the other gradients at zero -- never in the shipped library)
   { const char* e = getenv("NB200_WG_ONLY"); if (e) { const int k = atoi(e); if (k >= 0 && k < n) { wp.items[0] = wp.items[k]; n = 1; } } }
 #endif
   wp.num_items = n;
-  mlp_wgrad_tc_kernel<<<sm_count(), kWgThreads, kWgSmemLaunch, s>>>(wp);
+  mlp_wgrad_tc_kernel<false><<<sm_count(), kWgThreads, kWgSmemLaunch, s>>>(wp);
   NB_LAUNCH_CHECK("mlp_wgrad_tc_kernel");
   unpad_add_kernel<<<((int)kPadFoldS + 255) / 256, 256, 0, s>>>(pad, G[2 * L_C0], G[2 * L_SKIP], G[2 * L0_0], fold);
   NB_LAUNCH_CHECK("unpad_add_kernel");
@@ -864,6 +911,77 @@ int tc_backward(int, const float*, const float*, int64_t M, int, const void* pac
         G[2 * L_2], G[2 * L_2 + 1]);
     NB_LAUNCH_CHECK("fold_grads_kernel");
   }
+  return NB200_OK;
+}
+
+// NB200_BF16X3 backward: the delta chain in error-compensated bf16 (chain_kernel<DgradEpi3>, hi / lo deltas), then wgrad
+// with every (delta, input) pair of the layer-by-layer chain as three items, dW = d_hi^T a_hi + d_lo^T a_hi + d_hi^T a_lo.
+// The bias sums ride on the two items that stage a_hi (sum d_hi + sum d_lo); of the two carriers of each head (h7 / c1,
+// hi and lo) only the hi one adds the head-bias sums.
+int tc_backward_x3(int64_t M, const void* packed, const float* d_out, const void* saved, float* const* G, void* scratch,
+                   size_t scratch_bytes, cudaStream_t s) {
+  NB_TRY_RC(check_arch());
+  NB_TRY_RC(ensure_layout());
+  if (!scratch || scratch_bytes < tc_scratch_bytes_x3(M, 1)) return NB200_ERR_WORKSPACE;
+  NB_TRY_RC(ensure_attr(&DeviceState::attr_bwd3, []() -> int {
+    NB_CUDA_CHECK(cudaFuncSetAttribute(mlp_wgrad_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgSmemLaunch));
+    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<DgradEpi3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCSmemLaunch));
+    return NB200_OK;
+  }));
+  const int64_t T = train_tiles(M);
+  const uint8_t* sv_hi = reinterpret_cast<const uint8_t*>(saved);
+  const uint8_t* sv_lo = sv_hi + kSavedDataTileBytes * (size_t)T;
+  uint8_t* ds_hi = reinterpret_cast<uint8_t*>(scratch);
+  uint8_t* ds_lo = ds_hi + kDeltaTileBytes * (size_t)T;
+  float* pad = reinterpret_cast<float*>(ds_lo + kDeltaTileBytes * (size_t)T);
+  NB_CUDA_CHECK(cudaMemsetAsync(pad, 0, kPadFloats * sizeof(float), s));
+  // 1. delta chain
+  BwdParams bp;
+  bp.dbg = 0;
+  bp.M = M; bp.num_tiles = T; bp.packed = reinterpret_cast<const uint8_t*>(packed); bp.saved = sv_hi;
+  bp.d_out = d_out; bp.dscr = ds_hi;
+  {
+    TmapPair tm;
+    NB_TRY_RC(get_tmaps(packed, &tm, 1));
+    bp.tmap128 = tm.m128; bp.tmap64 = tm.m64;
+    chain_kernel<DgradEpi3><<<chain_grid_x3(T), kCThreads, kCSmemLaunch, s>>>(bp);
+    NB_LAUNCH_CHECK("chain_kernel<DgradEpi3>");
+  }
+  // 2. weight gradients
+  WgradParams3 wp;
+  memset(&wp, 0, sizeof(wp));
+  wp.T = T; wp.M = M; wp.d_out = d_out;
+  int n = 0;
+  // `head`: the sigma (1) / colour (2) head rides on the items that stage h7 / c1, hi with the head bias, lo without
+  auto item3 = [&](int dt, int st, int layer, int ldw, int col0, int ncols, int nrows, bool bias, int head = 0, int hst = 0, int hlayer = 0) {
+    wgrad_item(wp.items[n++], ds_hi, sv_hi, T, pad, G, dt, st, layer, ldw, col0, ncols, nrows, bias);
+    if (head) wgrad_head(wp.items[n - 1], sv_hi, T, G, head, hst, hlayer);
+    wgrad_item(wp.items[n++], ds_lo, sv_hi, T, pad, G, dt, st, layer, ldw, col0, ncols, nrows, bias);
+    wgrad_item(wp.items[n++], ds_hi, sv_lo, T, pad, G, dt, st, layer, ldw, col0, ncols, nrows, false);
+    if (head) {
+      wgrad_head(wp.items[n - 1], sv_lo, T, G, head, hst, hlayer);
+      wp.items[n - 1].hb = nullptr;
+    }
+  };
+  item3(0, 8, L_C0, kHidden + kPosD, 0, kHidden, kHidden / 2, true);                     // color_fc.0 <- g
+  item3(0, 11, L_C0, kHidden + kPosD, kHidden, kPosD, kHidden / 2, false, 2, 9, L_C1);  // color_fc.0 <- posd; color_fc.2 <- c1
+  item3(1, 7, L_2, kHidden, 0, kHidden, kHidden, true, 1, 7, L_SIGMA);                   // layers_2 <- h7; sigma_fc <- h7
+  item3(2, 6, L1_1, kHidden, 0, kHidden, kHidden, true);
+  item3(3, 5, L1_0, kHidden, 0, kHidden, kHidden, true);
+  item3(4, 4, L_SKIP, kHidden + kPosX, 0, kHidden, kHidden, true);
+  item3(4, 10, L_SKIP, kHidden + kPosX, kHidden, kPosX, kHidden, false);
+  item3(5, 3, L0_4, kHidden, 0, kHidden, kHidden, true);
+  item3(6, 2, L0_3, kHidden, 0, kHidden, kHidden, true);
+  item3(7, 1, L0_2, kHidden, 0, kHidden, kHidden, true);
+  item3(8, 0, L0_1, kHidden, 0, kHidden, kHidden, true);
+  item3(9, 10, L0_0, kPosX, 0, kPosX, kHidden, true);
+  // the bf16 chain's measured per-kind costs; the three items of a pair stage the same bytes (not separately measured)
+  wgrad_costs(wp.items, n);
+  wp.num_items = n;
+  mlp_wgrad_tc_kernel<true><<<sm_count(), kWgThreads, kWgSmemLaunch, s>>>(wp);
+  NB_LAUNCH_CHECK("mlp_wgrad_tc_kernel<bf16x3>");
+  unpad_add_kernel<<<((int)kPadFoldS + 255) / 256, 256, 0, s>>>(pad, G[2 * L_C0], G[2 * L_SKIP], G[2 * L0_0], 0);
+  NB_LAUNCH_CHECK("unpad_add_kernel");
   return NB200_OK;
 }
 

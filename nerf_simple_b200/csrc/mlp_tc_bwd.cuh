@@ -71,13 +71,17 @@ struct WItem {
   float* hb;              // gradient of the head bias
 };
 constexpr int kMaxWItems = 12;
-struct WgradParams {
-  WItem items[kMaxWItems];
+constexpr int kMaxWItems3 = 3 * kMaxWItems;   // bf16x3: three items per (delta, input) pair
+template <int kItems>
+struct WgradParamsT {
+  WItem items[kItems];
   int num_items;
   int64_t T;
   int64_t M;
   const float* d_out;     // [M,4] cotangent of (r,g,b,sigma): the head "deltas"
 };
+using WgradParams = WgradParamsT<kMaxWItems>;
+using WgradParams3 = WgradParamsT<kMaxWItems3>;
 
 // A stage holds kWgRows sample rows of up to 4 A chunks and 4 B chunks (64 features x kWgRows x 2 B each).
 // (An extra L2 prefetch ahead of the ring was measured: 548 -> 742 us, so there is none.)
@@ -98,7 +102,8 @@ constexpr int kWgThreads = 192;  // warp 0 producer, warp 1 MMA, warps 2-5 bias 
 struct WSeg { int item; int64_t t0, t1; };
 
 // Position x in the global cost sequence -> (item, tile).
-__device__ __forceinline__ void wg_locate(const WgradParams& p, int64_t x, int& item, int64_t& tile) {
+template <class P>
+__device__ __forceinline__ void wg_locate(const P& p, int64_t x, int& item, int64_t& tile) {
   int64_t cum = 0;
   for (int i = 0; i < p.num_items; ++i) {
     const int64_t span = (int64_t)p.items[i].cost * p.T;
@@ -108,7 +113,11 @@ __device__ __forceinline__ void wg_locate(const WgradParams& p, int64_t x, int& 
   item = p.num_items; tile = 0;
 }
 
-__global__ void __launch_bounds__(kWgThreads, 1) mlp_wgrad_tc_kernel(const __grid_constant__ WgradParams p) {
+// kX3 (bf16x3): the parameter block has room for three items per pair, and an item whose head-bias pointer is null adds
+// the head-weight gradient only (the two carriers of h7 / c1, hi and lo, must add db_sigma / db_c1 once).
+template <bool kX3>
+__global__ void __launch_bounds__(kWgThreads, 1)
+mlp_wgrad_tc_kernel(const __grid_constant__ std::conditional_t<kX3, WgradParams3, WgradParams> p) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t bar_base = smem_base + kWgSmemBar;
@@ -298,7 +307,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) mlp_wgrad_tc_kernel(const __gri
         const int n = cw * 64 + 2 * lane;
         atomicAdd(w.hW + n, hacc[0] + hacc[2]);          // even + odd row partial sums
         atomicAdd(w.hW + n + 1, hacc[1] + hacc[3]);
-        if (cw == 0) {
+        if (cw == 0 && (!kX3 || w.hb)) {
           const float tot = warp_sum_f(hbias.w);
           if (lane == 0) atomicAdd(w.hb, tot);
         }
@@ -309,7 +318,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) mlp_wgrad_tc_kernel(const __gri
           atomicAdd(w.hW + k * 128 + n, hacc[2 * k]);
           atomicAdd(w.hW + k * 128 + n + 1, hacc[2 * k + 1]);
         }
-        if (cw == 2) {
+        if (cw == 2 && (!kX3 || w.hb)) {
           const float tr = warp_sum_f(hbias.x), tg = warp_sum_f(hbias.y), tbl = warp_sum_f(hbias.z);
           if (lane == 0) { atomicAdd(w.hb, tr); atomicAdd(w.hb + 1, tg); atomicAdd(w.hb + 2, tbl); }
         }

@@ -134,7 +134,11 @@ def mlp_apply(net, in_mode, in0, in1=None, N=1, precision=None):
         in1 = _f32c(in1, "ts")
     need_grad = torch.is_grad_enabled() and any(p.requires_grad for p in params)
     if need_grad and precision == _lib.BF16X3:
-        precision = _lib.FP32      # bf16x3 is a forward mode: gradients in fp32-class accuracy come from the fp32 kernels
+        # Autograd accepts any cotangent.  With random cotangents on all five render outputs (tests/test_gpu_parity.py)
+        # the ReLU masks that the 16-bit (hi + lo) weights of the bf16x3 forward flip move some gradients by 5e-3 of the
+        # tensor max, over the suite's 3e-3 fp32-class bound, so autograd keeps the fp32 kernels.  Training steps
+        # (Trainer(precision="bf16x3"), the C ABI) run the bf16x3 tensor-core backward and meet the fp32 bounds there.
+        precision = _lib.FP32
     packed = net._packed.get(params, precision)
     cap = config._state["max_samples_per_call"]
     M = in0.shape[0] if in_mode == _lib.IN_POINTS else in0.shape[0] * N

@@ -133,7 +133,9 @@ class Trainer:
                  tn=2.0, tf=6.0, seed=1, precision="bf16", world_size=1, use_graph=True, rank=None, group=None):
         self.net, self.N, self.B = net, int(N), int(batch_size)
         self.tn, self.tf = float(tn), float(tf)
-        self.precision = {"fp32": _lib.FP32, "bf16": _lib.BF16, "bf16_layerwise": _lib.BF16_LAYERWISE}[precision]
+        self.precision = {"fp32": _lib.FP32, "bf16": _lib.BF16, "bf16_layerwise": _lib.BF16_LAYERWISE, "bf16x3": _lib.BF16X3}[precision]
+        # the tensor-core modes: packed weight images refreshed every step, the step captured in one CUDA graph
+        self._tc = self.precision in _lib.BF16_MODES or self.precision == _lib.BF16X3
         self.world_size, self.group = int(world_size), group
         self.rank = 0
         if self.world_size > 1:
@@ -194,13 +196,13 @@ class Trainer:
         self._param_ptrs = _lib.ptr_array(self.params)
         self._grad_ptrs = _lib.ptr_array(self.grads)
         self._packed_buf = (torch.empty(lib.nb200_packed_weights_bytes(self.precision), dtype=torch.uint8, device=self.device)
-                            if self.precision in _lib.BF16_MODES else None)
-        self.use_graph = bool(use_graph) and self.precision in _lib.BF16_MODES and self.N % 4 == 0 and self.N <= 1024
+                            if self._tc else None)
+        self.use_graph = bool(use_graph) and self._tc and self.N % 4 == 0 and self.N <= 1024
         # why the step is NOT one CUDA-graph replay, when it is not (the eager path computes the same numbers, with
         # ~14 launches of host overhead per step): readable by the caller instead of a silent fallback
         self.graph_off_reason = (None if self.use_graph else
                                  "use_graph=False" if not use_graph else
-                                 "precision is not bf16 (the fp32 step is ~65 launches, not captured)" if self.precision not in _lib.BF16_MODES else
+                                 "precision is fp32 (the SIMT step is ~65 launches, not captured)" if not self._tc else
                                  f"N={self.N}: the device-resident sampler state needs N % 4 == 0 and N <= 1024")
         if use_graph and not self.use_graph:
             import warnings
@@ -262,7 +264,7 @@ class Trainer:
                        "nb200_stratified_ts")
         pa = self._param_ptrs
         packed = self._packed_buf
-        if self.precision in _lib.BF16_MODES:   # the optimizer changed the fp32 masters: refresh the bf16 operand images
+        if self._tc:   # the optimizer changed the fp32 masters: refresh the bf16 (hi / lo) operand images
             _lib.check(lib.nb200_pack_weights(self.precision, pa, _lib.ptr(packed), st), "nb200_pack_weights")
         if time_parts:
             ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
@@ -382,8 +384,9 @@ class Trainer:
         self._offset += (self.B * self.N + 3) // 4
         self.lr *= self.lr_decay
         self._bump_versions()
-        # select, ts, pack x2, fwd, comp fwd, mse, comp bwd, bwd kernels, unpad, adam, state (+ memsets)
-        self.launches += ((16 if self.precision == _lib.BF16 else 14) if self.precision in _lib.BF16_MODES else 65) - (0 if select else 1) - (0 if ts is None else 1)
+        # select, ts, pack x2, fwd, comp fwd, mse, comp bwd, bwd kernels, unpad, adam, state (+ memsets); the folded bf16
+        # chain adds the fold / un-fold kernels, bf16_layerwise and bf16x3 have none
+        self.launches += ((16 if self.precision == _lib.BF16 else 14) if self._tc else 65) - (0 if select else 1) - (0 if ts is None else 1)
         self.last_loss = self._loss
         return float(self._loss) if sync_loss else self._loss.clone()
 
