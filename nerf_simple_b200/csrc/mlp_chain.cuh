@@ -67,52 +67,72 @@ __device__ __forceinline__ void slot_barrier(int slot) {  // the 256 epilogue th
 // and the accumulate flags are immediates, and the only runtime state is the ring position.  (Walking the
 // constant-bank SlabDesc table instead cost a chain of dependent indexed LDC + R2UR + LDCU per slab, ~700 cycles of
 // MMA-warp time for the 512 cycles of tensor work it issued: the issue warp, not the weights or the epilogue, was
-// the bottleneck of every chain kernel.)  The producer still walks the table (it is never late); check_schedules()
-// verifies on the host that table and compile-time schedule agree.
+// the bottleneck of every chain kernel.)  The schedule is read from kLayout at compile time, the table whose
+// constant-bank copy the producer walks (it is never late), so both see the same slabs in the same order.
 #ifdef NB200_DEV
 constexpr bool kDevBuild = true;    // cycle counters of the MMA / epilogue / producer warps (NB200_DBG=8), never in the shipped library
 #else
 constexpr bool kDevBuild = false;
 #endif
-struct SlabC { int src, kb, n, ksteps, both_a; };
-constexpr int kSchedFwd = 0, kSchedBwd = 1, kSchedFwd3 = 2, kSchedFwdFold = 3;   // Fold: layers 0..7, then color_fc.0 as layer 8
-constexpr int kSchedBwd3 = 4;   // bf16x3 delta chain: every kSchedBwd slab twice, hi (against delta_hi and delta_lo) then lo
-__host__ __device__ constexpr int sched_fwd_slabs(int l) { return l == 0 ? 1 : ((l == 5 || l == 9) ? 5 : 4); }
-__host__ __device__ constexpr SlabC sched_fwd_slab(int l, int s) {
-  return l == 0 ? SlabC{1, 0, 256, 4, 0}
-                : (l == 9 ? (s < 4 ? SlabC{0, s, 128, 4, 0} : SlabC{1, 0, 128, 2, 0})
-                          : (s < 4 ? SlabC{0, s, 256, 4, 0} : SlabC{1, 0, 256, 4, 0}));
+// The slab tables of PackedLayout; each epilogue names the one it walks (Epi::kTab).
+enum SlabTab { kTabFwd, kTabFwdFold, kTabBwd, kTabBwdFold, kTabFwd3, kTabBwd3 };
+template <int kTab, class Layout> __host__ __device__ constexpr auto& slab_table(Layout& lay) {
+  if constexpr (kTab == kTabFwd) return lay.fwd;
+  else if constexpr (kTab == kTabFwdFold) return lay.fwdf;
+  else if constexpr (kTab == kTabBwd) return lay.bwd;
+  else if constexpr (kTab == kTabBwdFold) return lay.bwdf;
+  else if constexpr (kTab == kTabFwd3) return lay.fwd3;
+  else return lay.bwd3;
 }
-template <int kSched> __host__ __device__ constexpr bool sched_is_bwd() { return kSched == kSchedBwd || kSched == kSchedBwd3; }
-template <int kSched> __host__ __device__ constexpr int sched_slabs(int l) {
-  return kSched == kSchedBwd3 ? 2 * (l == 0 ? 2 : 4)
-         : kSched == kSchedFwd ? sched_fwd_slabs(l)
-                             : (kSched == kSchedFwdFold ? sched_fwd_slabs(l >= 8 ? 9 : l) : (kSched == kSchedBwd ? (l == 0 ? 2 : 4) : 2 * sched_fwd_slabs(l)));
+template <int kTab> __host__ __device__ constexpr bool sched_is_bwd() { return kTab == kTabBwd || kTab == kTabBwdFold || kTab == kTabBwd3; }
+// loop layer l = the l-th run of slabs closed by a `last` flag (the producer walks the table the same way)
+template <int kTab> __host__ __device__ constexpr int sched_first(int l) {
+  int i = 0;
+  for (int k = 0; k < l; ++k, ++i)
+    while (!slab_table<kTab>(kLayout)[i].last) ++i;
+  return i;
 }
-template <int kSched> __host__ __device__ constexpr SlabC sched_slab(int l, int s) {
-  if (kSched == kSchedFwd) return sched_fwd_slab(l, s);
-  if (kSched == kSchedFwdFold) return sched_fwd_slab(l >= 8 ? 9 : l, s);
-  if (kSched == kSchedBwd) return SlabC{0, s, 256, 4, 0};
-  if (kSched == kSchedBwd3) return SlabC{0, s >> 1, 256, 4, (s & 1) ? 0 : 1};
-  SlabC c = sched_fwd_slab(l, s >> 1);   // bf16x3: every forward slab twice, hi (against A_hi and A_lo) then lo (A_hi only)
-  c.both_a = (s & 1) ? 0 : 1;
-  return c;
+template <int kTab> __host__ __device__ constexpr int sched_slabs(int l) {
+  int i = sched_first<kTab>(l);
+  while (!slab_table<kTab>(kLayout)[i].last) ++i;
+  return i - sched_first<kTab>(l) + 1;
+}
+template <int kTab> __host__ __device__ constexpr SlabDesc sched_slab(int l, int s) {
+  return slab_table<kTab>(kLayout)[sched_first<kTab>(l) + s];
 }
 
 struct MmaRing { uint32_t stage, phase; };
 
 // Layers with the same slab list share one unrolled copy of the issue code (kept small: the fully unrolled version,
 // one copy per layer and slot, was 100 KB of instructions and thrashed the instruction cache of the training kernels).
-// Class representatives: forward 0 | 1 (all plain 256x256 layers) | 5 (skip) | 9 (color_fc.0); delta chain 0 | 1.
-template <int kSched> __host__ __device__ constexpr int sched_class_rep(int l) {
-  return sched_is_bwd<kSched>() ? (l == 0 ? 0 : 1) : ((l == 0 || l == 5 || l == 9) ? l : ((kSched == kSchedFwdFold && l == 8) ? 9 : 1));
+// Class representatives (loop indices): forward 0 | 1 (all plain 256x256 layers) | 5 (skip) | the last (color_fc.0);
+// delta chain 0 | 1.
+template <class Epi> __host__ __device__ constexpr int sched_class_rep(int l) {
+  return sched_is_bwd<Epi::kTab>() ? (l == 0 ? 0 : 1) : ((l == 0 || l == 5 || l == Epi::kNumLayers - 1) ? l : 1);
+}
+// The table holds Epi::kNumLayers layers, and each has the slab list (as far as the issue code reads it) of its class
+// representative.
+template <class Epi> constexpr bool sched_classes_hold() {
+  int layers = 0;
+  for (const SlabDesc& d : slab_table<Epi::kTab>(kLayout)) layers += d.last;
+  if (layers != Epi::kNumLayers) return false;
+  for (int l = 0; l < Epi::kNumLayers; ++l) {
+    const int rep = sched_class_rep<Epi>(l);
+    if (sched_slabs<Epi::kTab>(l) != sched_slabs<Epi::kTab>(rep)) return false;
+    for (int s = 0; s < sched_slabs<Epi::kTab>(l); ++s) {
+      const SlabDesc a = sched_slab<Epi::kTab>(l, s), b = sched_slab<Epi::kTab>(rep, s);
+      if (a.src != b.src || a.kb != b.kb || a.n != b.n || a.ksteps != b.ksteps || (a.flags & kSlabBothA) != (b.flags & kSlabBothA))
+        return false;
+    }
+  }
+  return true;
 }
 
 template <class Epi, int L, int S>
 __device__ __forceinline__ void issue_slab(uint32_t smem_base, uint32_t bar, uint32_t tmem_base, uint64_t desc_hi, uint32_t slot,
                                            bool replay, bool release, MmaRing& r) {
-  constexpr SlabC sc = sched_slab<Epi::kSched>(L, S);
-  constexpr int NS = sched_slabs<Epi::kSched>(L);
+  constexpr SlabDesc sc = sched_slab<Epi::kTab>(L, S);
+  constexpr int NS = sched_slabs<Epi::kTab>(L);
   if (!replay) {
     mbar_wait(bar + kB_WFull + 8 * r.stage, r.phase, 400);
     tc_fence_after();
@@ -129,7 +149,7 @@ __device__ __forceinline__ void issue_slab(uint32_t smem_base, uint32_t bar, uin
       umma_bf16_2cta(d_tmem, adesc + 4, bdesc + 4, idesc, 1u);
       umma_bf16_2cta(d_tmem, adesc + 6, bdesc + 6, idesc, 1u);
     }
-    if (sc.both_a) {   // bf16x3: the same B slab against the residual image A_lo (the other slot's buffer)
+    if (sc.flags & kSlabBothA) {   // bf16x3: the same B slab against the residual image A_lo (the other slot's buffer)
       const uint64_t alo = adesc + ((sc.src ? kEBytes : kABytes) >> 4);
       umma_bf16_2cta(d_tmem, alo, bdesc, idesc, 1u);
       umma_bf16_2cta(d_tmem, alo + 2, bdesc + 2, idesc, 1u);
@@ -153,7 +173,7 @@ __device__ __forceinline__ void issue_slabs(std::integer_sequence<int, S...>, ui
 template <class Epi, int L>
 __device__ __forceinline__ void issue_layer(uint32_t smem_base, uint32_t bar, uint32_t tmem_base, uint64_t desc_hi, int nslots, int l,
                                             MmaRing& r, uint32_t (&act_parity)[2], long long& t_act) {
-  constexpr int NS = sched_slabs<Epi::kSched>(L);
+  constexpr int NS = sched_slabs<Epi::kTab>(L);
   using Seq = std::make_integer_sequence<int, NS>;
   const bool shared = (nslots == 2 && NS <= kCStages);   // do both slots consume one copy of the layer's slabs?
   const MmaRing r0 = r;
@@ -177,6 +197,7 @@ __device__ __forceinline__ void issue_layer(uint32_t smem_base, uint32_t bar, ui
 template <class Epi>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kCThreads, 1)
 chain_kernel(const __grid_constant__ typename Epi::Params p) {
+  static_assert(sched_classes_hold<Epi>(), "a layer's slab list differs from its class representative's, or the table's layer count from the epilogue's");
   extern __shared__ __align__(1024) uint8_t chain_smem[];
   const uint32_t smem_base = smem_u32(chain_smem);
   if (smem_base & 1023u) {   // the SWIZZLE_128B images need it, and there is no slack left to round up
@@ -213,7 +234,7 @@ chain_kernel(const __grid_constant__ typename Epi::Params p) {
   const int64_t PT = (p.num_tiles + 1) / 2;
   const int64_t C = num_clusters_x(), cid = cluster_id_x();
   const int64_t my_pt = (cid < PT) ? (PT - cid + C - 1) / C : 0;
-  const SlabDesc* slabs = Epi::slabs();
+  const SlabDesc* slabs = slab_table<Epi::kTab>(c_layout);
 
   if (warp < 16) {
     // ============================ prologue + epilogue of one slot ============================
@@ -229,7 +250,7 @@ chain_kernel(const __grid_constant__ typename Epi::Params p) {
     c.e_img = smem_base + kC_E + slot * kEBytes;
     c.t_lane = tmem_base + (((uint32_t)(warp & 3) * 32u) << 16) + (uint32_t)slot * 256u;
     c.b_img = smem_base + kC_Bias + (uint32_t)slot * 1024u;
-    c.gf = reinterpret_cast<const float*>(p.packed + (Epi::kSched == kSchedFwd3 || Epi::kSched == kSchedBwd3 ? c_layout.f32_off3 : c_layout.f32_off));
+    c.gf = reinterpret_cast<const float*>(p.packed + (Epi::kTab == kTabFwd3 || Epi::kTab == kTabBwd3 ? c_layout.f32_off3 : c_layout.f32_off));
     const uint32_t act_remote = mapa_shared(bar + kB_Act + 8 * slot, 0);  // leader's act_ready[slot]
     uint32_t acc_parity = 0, free_parity = 0;
     typename Epi::State st;
@@ -400,11 +421,11 @@ chain_kernel(const __grid_constant__ typename Epi::Params p) {
       const int nslots = (Epi::kSlots == 2 && my_pt - 2 * pr >= 2) ? 2 : 1;
 #pragma unroll 1
       for (int l = 0; l < Epi::kNumLayers; ++l) {
-        const int rep = sched_class_rep<Epi::kSched>(l);
+        const int rep = sched_class_rep<Epi>(l);
         if (rep == 0) issue_layer<Epi, 0>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
         else if (rep == 1) issue_layer<Epi, 1>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
-        else if (!sched_is_bwd<Epi::kSched>() && rep == 5) issue_layer<Epi, 5>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
-        else if (!sched_is_bwd<Epi::kSched>()) issue_layer<Epi, 9>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
+        else if (!sched_is_bwd<Epi::kTab>() && rep == 5) issue_layer<Epi, 5>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
+        else if (!sched_is_bwd<Epi::kTab>()) issue_layer<Epi, Epi::kNumLayers - 1>(smem_base, bar, tmem_base, desc_hi, nslots, l, ring, act_parity, t_act);
       }
     }
 #ifdef NB200_DEV
@@ -663,7 +684,7 @@ struct FwdEpi {
   using Params = FwdEpiParams;
   static constexpr bool kHasDbg = true;
   static constexpr bool kBulkStore = kSave;  // training: finished tile images leave through TMA bulk stores
-  static constexpr int kSched = kFold ? kSchedFwdFold : kSchedFwd;
+  static constexpr int kTab = kFold ? kTabFwdFold : kTabFwd;
   static constexpr bool kStageBias = true;
   static constexpr int kSlots = 2;
   static constexpr int kNumLayers = kFold ? kNumFoldLayers : kNumMmaLayers;
@@ -677,7 +698,6 @@ struct FwdEpi {
     int64_t m_raw;
     bool row_valid;
   };
-  __device__ static const SlabDesc* slabs() { return kFold ? c_layout.fwdf : c_layout.fwd; }
   __device__ static void init_slot(const TileCtx&) {}
 
   __device__ static void prefetch(const Params&, State&, const TileCtx&, int) {}
@@ -878,7 +898,7 @@ struct FwdEpi3 {
   using Params = FwdEpiParams;
   static constexpr bool kHasDbg = false;
   static constexpr bool kBulkStore = kSave;
-  static constexpr int kSched = kSchedFwd3;
+  static constexpr int kTab = kTabFwd3;
   static constexpr bool kStageBias = true;
   static constexpr int kSlots = 1;
   static constexpr int kNumLayers = kNumMmaLayers;
@@ -889,7 +909,6 @@ struct FwdEpi3 {
     int64_t m_raw;
     bool row_valid;
   };
-  __device__ static const SlabDesc* slabs() { return c_layout.fwd3; }
   __device__ static constexpr int bias_row(int l) { return l; }
   __device__ static void init_slot(const TileCtx&) {}
   __device__ static void prefetch(const Params&, State&, const TileCtx&, int) {}
@@ -1055,14 +1074,13 @@ struct DgradEpi {
   using Params = BwdParams;
   static constexpr bool kHasDbg = false;
   static constexpr bool kBulkStore = true;
-  static constexpr int kSched = kSchedBwd;
+  static constexpr int kTab = kFold ? kTabBwdFold : kTabBwd;
   static constexpr bool kStageBias = false;
   static constexpr int kSlots = 2;
   static constexpr int kNumLayers = kFold ? 8 : 9;  // bl = 1..9 (folded: 2..9)
   static constexpr int kBl0 = kFold ? 2 : 1;        // bl of loop index 0
   static constexpr bool kReverseTiles = true;
   struct State { float4 g; uint4 mask; };
-  __device__ static const SlabDesc* slabs() { return kFold ? c_layout.bwdf : c_layout.bwd; }
   __device__ static constexpr int bias_row(int l) { return l; }
   __device__ static void after_publish(const Params&, State&, const TileCtx&, int) {}
   // The delta chain has no use for the encoding buffers: E[slot] holds w_sigma (floats 0..255) and color_fc.2's weight
@@ -1197,13 +1215,12 @@ struct DgradEpi3 {
   using Params = BwdParams;
   static constexpr bool kHasDbg = false;
   static constexpr bool kBulkStore = true;
-  static constexpr int kSched = kSchedBwd3;
+  static constexpr int kTab = kTabBwd3;
   static constexpr bool kStageBias = false;
   static constexpr int kSlots = 1;
   static constexpr int kNumLayers = 9;   // bl = 1..9
   static constexpr bool kReverseTiles = true;
   struct State { float4 g; uint2 mask; };
-  __device__ static const SlabDesc* slabs() { return c_layout.bwd3; }
   __device__ static constexpr int bias_row(int l) { return l; }
   __device__ static void after_publish(const Params&, State&, const TileCtx&, int) {}
   // E[0] holds w_sigma (floats 0..255) and color_fc.2's weight (256..639) for the whole kernel

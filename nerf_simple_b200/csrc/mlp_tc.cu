@@ -90,21 +90,6 @@ constexpr int kF32Bias = 0, kF32WSig = 2816, kF32BSig = 3072, kF32WC1 = 3076, kF
 constexpr int kF32Wf = kF32Floats, kF32WgT = kF32Wf + 128 * 256, kF32Wc0g = kF32WgT + 256 * 256, kF32Bg = kF32Wc0g + 128 * 256,
               kF32FloatsFold = kF32Bg + 256;
 
-__constant__ __align__(16) PackedLayout c_layout;
-static PackedLayout h_layout;
-static bool h_layout_built = false;
-
-// Everything CUDA caches per device (constant-bank copies, function attributes, the architecture check) is keyed
-// by the current device, so one process can drive several GPUs; the tables are guarded by one mutex.
-constexpr int kMaxDevices = 64;
-struct DeviceState { bool layout_uploaded, attr_fwd, attr_render, attr_bwd, attr_x3, attr_bwd3; int arch; };
-static DeviceState g_dev[kMaxDevices];
-static std::mutex g_mu;
-static int current_device(int* dev) {
-  NB_CUDA_CHECK(cudaGetDevice(dev));
-  return (*dev >= 0 && *dev < kMaxDevices) ? NB200_OK : NB200_ERR_UNSUPPORTED;
-}
-
 __host__ __device__ constexpr int mma_layer_of(int ml) {
   return ml <= 4 ? L0_0 + ml : (ml == 5 ? L_SKIP : (ml <= 7 ? L1_0 + (ml - 6) : (ml == 8 ? L_2 : L_C0)));
 }
@@ -113,8 +98,8 @@ struct LayoutBuilder {
   SlabDesc* arr;
   uint32_t off;
   int s;
-  void add(int ml, int layer, int transposed, int n, int wcol0, int kvalid, int ldw, int src, int kb, int ksteps, int lo = 0,
-           int amode = 0) {
+  constexpr void add(int ml, int layer, int transposed, int n, int wcol0, int kvalid, int ldw, int src, int kb, int ksteps,
+                     int lo = 0, int amode = 0) {
     SlabDesc& d = arr[s++];
     d.off = off; d.bytes = (uint32_t)n * 128u; d.n = (uint16_t)n; d.wcol0 = (uint16_t)wcol0;
     d.kvalid = (uint16_t)kvalid; d.ldw = (uint16_t)ldw; d.ml = (uint8_t)ml; d.layer = (uint8_t)layer;
@@ -130,10 +115,9 @@ __host__ __device__ constexpr int bwd_layer_of(int bl) {
   return bl == 1 ? L_C0 : (bl == 2 ? L_2 : (bl == 3 ? L1_1 : (bl == 4 ? L1_0 : (bl == 5 ? L_SKIP : L0_4 - (bl - 6)))));
 }
 
-static void build_layout() {
-  memset(&h_layout, 0, sizeof(h_layout));
-  LayoutBuilder b;
-  b.arr = h_layout.fwd; b.off = 0; b.s = 0;
+constexpr PackedLayout make_layout() {
+  PackedLayout lay{};
+  LayoutBuilder b{lay.fwd, 0, 0};
   for (int ml = 0; ml < kNumMmaLayers; ++ml) {
     const int first = b.s, ly = mma_layer_of(ml);
     if (ml == 0) {
@@ -147,98 +131,84 @@ static void build_layout() {
     } else {
       for (int kb = 0; kb < 4; ++kb) b.add(ml, ly, 0, 256, kb * 64, 64, kHidden, 0, kb, 4);
     }
-    h_layout.fwd[first].first = 1;
-    h_layout.fwd[b.s - 1].last = 1;
+    lay.fwd[first].first = 1;
+    lay.fwd[b.s - 1].last = 1;
   }
-  h_layout.num_fwd = b.s;
+  lay.num_fwd = b.s;
   // dgrad slabs: n = 256 input features (rows of the image), k-blocks over the output features
-  LayoutBuilder t;
-  t.arr = h_layout.bwd; t.off = b.off; t.s = 0;
+  LayoutBuilder t{lay.bwd, b.off, 0};
   for (int bl = 1; bl <= 9; ++bl) {
     const int first = t.s, ly = bwd_layer_of(bl);
     const int ldw = (ly == L_C0) ? kHidden + kPosD : (ly == L_SKIP ? kHidden + kPosX : kHidden);
     const int nkb = (bl == 1) ? 2 : 4;  // color_fc.0 has 128 outputs
     for (int kb = 0; kb < nkb; ++kb) t.add(bl, ly, 1, 256, kb * 64, 64, ldw, 0, kb, 4);
-    h_layout.bwd[first].first = 1;
-    h_layout.bwd[t.s - 1].last = 1;
+    lay.bwd[first].first = 1;
+    lay.bwd[t.s - 1].last = 1;
   }
-  h_layout.num_bwd = t.s;
+  lay.num_bwd = t.s;
   // the slabs of the folded weight: forward image (n = c1 feature, k = h7 feature), then transposed for the delta chain
-  LayoutBuilder f;
-  f.arr = h_layout.fold; f.off = t.off; f.s = 0;
+  LayoutBuilder f{lay.fold, t.off, 0};
   for (int kb = 0; kb < 4; ++kb) f.add(9, kLayerFold, 0, 128, kb * 64, 64, kHidden, 0, kb, 4);
   for (int kb = 0; kb < 2; ++kb) f.add(2, kLayerFold, 1, 256, kb * 64, 64, kHidden, 0, kb, 4);
-  h_layout.num_fold = f.s;
+  lay.num_fold = f.s;
   {
     int n = 0;
-    for (int i = 0; i < h_layout.num_fwd; ++i)
-      if (h_layout.fwd[i].ml < 8) h_layout.fwdf[n++] = h_layout.fwd[i];
-    for (int kb = 0; kb < 4; ++kb) h_layout.fwdf[n++] = h_layout.fold[kb];
-    h_layout.fwdf[n - 4].first = 1;
-    h_layout.fwdf[n++] = h_layout.fwd[h_layout.num_fwd - 1];   // color_fc.0 <- posd (last slab of the layer)
-    h_layout.num_fwdf = n;
+    for (int i = 0; i < lay.num_fwd; ++i)
+      if (lay.fwd[i].ml < 8) lay.fwdf[n++] = lay.fwd[i];
+    for (int kb = 0; kb < 4; ++kb) lay.fwdf[n++] = lay.fold[kb];
+    lay.fwdf[n - 4].first = 1;
+    lay.fwdf[n++] = lay.fwd[lay.num_fwd - 1];   // color_fc.0 <- posd (last slab of the layer)
+    lay.num_fwdf = n;
     n = 0;
-    for (int kb = 0; kb < 2; ++kb) h_layout.bwdf[n++] = h_layout.fold[4 + kb];
-    h_layout.bwdf[0].first = 1; h_layout.bwdf[1].last = 1;
-    for (int i = 0; i < h_layout.num_bwd; ++i)
-      if (h_layout.bwd[i].ml >= 3) h_layout.bwdf[n++] = h_layout.bwd[i];
-    h_layout.num_bwdf = n;
+    for (int kb = 0; kb < 2; ++kb) lay.bwdf[n++] = lay.fold[4 + kb];
+    lay.bwdf[0].first = 1; lay.bwdf[1].last = 1;
+    for (int i = 0; i < lay.num_bwd; ++i)
+      if (lay.bwd[i].ml >= 3) lay.bwdf[n++] = lay.bwd[i];
+    lay.num_bwdf = n;
   }
-  h_layout.f32_off = f.off;
-  h_layout.total_bytes = f.off + kF32FloatsFold * (uint32_t)sizeof(float);
+  lay.f32_off = f.off;
+  lay.total_bytes = f.off + kF32FloatsFold * (uint32_t)sizeof(float);
   // bf16x3: every forward slab twice (hi: consumed with A_hi and A_lo; lo: with A_hi), in consumption order
-  LayoutBuilder x;
-  x.arr = h_layout.fwd3; x.off = 0; x.s = 0;
-  for (int i = 0; i < h_layout.num_fwd; ++i) {
-    const SlabDesc& f = h_layout.fwd[i];
+  LayoutBuilder x{lay.fwd3, 0, 0};
+  for (int i = 0; i < lay.num_fwd; ++i) {
+    const SlabDesc& f = lay.fwd[i];
     for (int lo = 0; lo < 2; ++lo) {
       x.add(f.ml, f.layer, 0, f.n, f.wcol0, f.kvalid, f.ldw, f.src, f.kb, f.ksteps, lo, lo ? 0 : 1);
-      h_layout.fwd3[x.s - 1].first = (uint8_t)(f.first && lo == 0);
-      h_layout.fwd3[x.s - 1].last = (uint8_t)(f.last && lo == 1);
+      lay.fwd3[x.s - 1].first = (uint8_t)(f.first && lo == 0);
+      lay.fwd3[x.s - 1].last = (uint8_t)(f.last && lo == 1);
     }
   }
-  h_layout.num_fwd3 = x.s;
-  h_layout.f32_off3 = x.off;
+  lay.num_fwd3 = x.s;
+  lay.f32_off3 = x.off;
   // bf16x3 delta chain: every transposed slab of `bwd` twice (hi: consumed with delta_hi and delta_lo; lo: with
   // delta_hi), behind the fp32 tail, so that the forward slabs and the tail keep their offsets
-  LayoutBuilder y;
-  y.arr = h_layout.bwd3; y.off = x.off + kF32Floats * (uint32_t)sizeof(float); y.s = 0;
-  for (int i = 0; i < h_layout.num_bwd; ++i) {
-    const SlabDesc& d = h_layout.bwd[i];
+  LayoutBuilder y{lay.bwd3, x.off + kF32Floats * (uint32_t)sizeof(float), 0};
+  for (int i = 0; i < lay.num_bwd; ++i) {
+    const SlabDesc& d = lay.bwd[i];
     for (int lo = 0; lo < 2; ++lo) {
       y.add(d.ml, d.layer, 1, d.n, d.wcol0, d.kvalid, d.ldw, d.src, d.kb, d.ksteps, lo, lo ? 0 : 1);
-      h_layout.bwd3[y.s - 1].first = (uint8_t)(d.first && lo == 0);
-      h_layout.bwd3[y.s - 1].last = (uint8_t)(d.last && lo == 1);
+      lay.bwd3[y.s - 1].first = (uint8_t)(d.first && lo == 0);
+      lay.bwd3[y.s - 1].last = (uint8_t)(d.last && lo == 1);
     }
   }
-  h_layout.num_bwd3 = y.s;
-  h_layout.total_bytes3 = y.off;
+  lay.num_bwd3 = y.s;
+  lay.total_bytes3 = y.off;
+  return lay;
 }
 
-// The MMA warps walk a compile-time schedule (mlp_chain.cuh: sched_slab), the weight producers and the packer this
-// table: they must describe the same slabs in the same order.
-template <int kSched>
-static bool schedule_matches(const SlabDesc* tab, int num, int layers);
-static bool check_schedules();
+// The one description of the packed image.  The weight producers and the packer walk its constant-bank copy; the MMA
+// warp's compile-time schedule (mlp_chain.cuh: sched_slab) is read from it while compiling.
+constexpr PackedLayout kLayout = make_layout();
+__constant__ __align__(16) PackedLayout c_layout = kLayout;
 
-static void ensure_host_layout() {   // caller holds g_mu
-  if (h_layout_built) return;
-  build_layout();
-  if (!check_schedules()) {
-    fprintf(stderr, "nb200: packed-weight table and compile-time MMA schedule disagree\n");
-    abort();
-  }
-  h_layout_built = true;
-}
-static int ensure_layout() {
-  int dev = 0;
-  NB_TRY_RC(current_device(&dev));
-  std::lock_guard<std::mutex> lock(g_mu);
-  ensure_host_layout();
-  if (g_dev[dev].layout_uploaded) return NB200_OK;
-  NB_CUDA_CHECK(cudaMemcpyToSymbol(c_layout, &h_layout, sizeof(PackedLayout)));   // this device's constant bank
-  g_dev[dev].layout_uploaded = true;
-  return NB200_OK;
+// Everything CUDA caches per device (function attributes, the architecture check) is keyed by the current device, so
+// one process can drive several GPUs; the caches are guarded by one mutex.
+constexpr int kMaxDevices = 64;
+static int g_arch[kMaxDevices];
+static std::mutex g_mu;
+static int current_device(int* dev) {
+  NB_CUDA_CHECK(cudaGetDevice(dev));
+  return (*dev >= 0 && *dev < kMaxDevices) ? NB200_OK : NB200_ERR_UNSUPPORTED;
 }
 
 struct ParamPtrs { const float* p[24]; };
@@ -462,42 +432,18 @@ __device__ __forceinline__ void encode_row(const float* x, uint32_t img_base, ui
 #include "mlp_tc_bwd.cuh"
 #include "mlp_chain.cuh"
 
-template <int kSched>
-static bool schedule_matches(const SlabDesc* tab, int num, int layers) {
-  int i = 0;
-  for (int l = 0; l < layers; ++l) {
-    const int ns = sched_slabs<kSched>(l);
-    for (int k = 0; k < ns; ++k, ++i) {
-      if (i >= num) return false;
-      const SlabC c = sched_slab<kSched>(l, k);
-      const SlabDesc& d = tab[i];
-      if (d.src != c.src || d.kb != c.kb || d.n != c.n || d.ksteps != c.ksteps || ((d.flags & kSlabBothA) != 0) != (c.both_a != 0) ||
-          (d.first != 0) != (k == 0) || (d.last != 0) != (k == ns - 1) || d.bytes != (uint32_t)c.n * 128u)
-        return false;
-    }
-  }
-  return i == num;
-}
-static bool check_schedules() {
-  return schedule_matches<kSchedFwd>(h_layout.fwd, h_layout.num_fwd, kNumMmaLayers) &&
-         schedule_matches<kSchedBwd>(h_layout.bwd, h_layout.num_bwd, 9) &&
-         schedule_matches<kSchedFwdFold>(h_layout.fwdf, h_layout.num_fwdf, kNumFoldLayers) &&
-         schedule_matches<kSchedBwd>(h_layout.bwdf, h_layout.num_bwdf, 8) &&
-         schedule_matches<kSchedFwd3>(h_layout.fwd3, h_layout.num_fwd3, kNumMmaLayers) &&
-         schedule_matches<kSchedBwd3>(h_layout.bwd3, h_layout.num_bwd3, 9);
-}
-
 // ------------------------------------------------------------------------------ host API
-size_t tc_packed_bytes(int x3) {
-  std::lock_guard<std::mutex> lock(g_mu);
-  ensure_host_layout();  // layout is host-computable without a device
-  return x3 ? h_layout.total_bytes3 : h_layout.total_bytes;
-}
+// `precision` selects the tensor-core mode: NB200_BF16 (layers_2 folded into color_fc.0), NB200_BF16_LAYERWISE or
+// NB200_BF16X3.  The two bf16 modes share the packed image and the saved / scratch layouts.
+size_t tc_packed_bytes(int precision) { return precision == NB200_BF16X3 ? kLayout.total_bytes3 : kLayout.total_bytes; }
 // Training tensors are laid out for an EVEN number of 128-sample tiles: the chain kernels work on pair-tiles
 // (one tile per CTA of a cluster), so with an odd tile count the second CTA of the last pair still writes a
 // (zero-gradient) tile image, which must not alias tile 0 of the next tensor.
 static int64_t train_tiles(int64_t M) { return (ceil_div64(M, kTileM) + 1) & ~(int64_t)1; }
-size_t tc_saved_bytes(int64_t M) { return (size_t)train_tiles(M) * kSavedTileBytes; }
+// bf16x3: saved = hi data | lo data | masks; scratch = hi deltas | lo deltas | pad images
+size_t tc_saved_bytes(int precision, int64_t M) {
+  return (size_t)train_tiles(M) * (precision == NB200_BF16X3 ? kSavedTileBytes3 : kSavedTileBytes);
+}
 // padded staging of the three weight gradients whose rows are not 16-byte multiples (283, 319, 63
 // columns): wgrad flushes into [rows x 320] / [rows x 64] images with vector reductions, and
 // unpad_add_kernel folds them into the real gradients (the scalar-atomic flush of those three layers
@@ -506,13 +452,9 @@ constexpr int kPadPitchWide = 320, kPadPitchX = 64;
 constexpr size_t kPadC0 = 0, kPadSkip = kPadC0 + 128 * kPadPitchWide, kPadL00 = kPadSkip + 256 * kPadPitchWide,
                  kPadFoldS = kPadL00 + 256 * kPadPitchX,   // folded chain: column sums of delta_c1 (128 floats)
                  kPadFloats = kPadFoldS + 128;
-size_t tc_scratch_bytes(int64_t M, int train) {
-  return train ? (size_t)train_tiles(M) * kDeltaTileBytes + kPadFloats * sizeof(float) : 0;
-}
-// bf16x3: saved = hi data | lo data | masks; scratch = hi deltas | lo deltas | pad images
-size_t tc_saved_bytes_x3(int64_t M) { return (size_t)train_tiles(M) * kSavedTileBytes3; }
-size_t tc_scratch_bytes_x3(int64_t M, int train) {
-  return train ? (size_t)train_tiles(M) * 2 * kDeltaTileBytes + kPadFloats * sizeof(float) : 0;
+size_t tc_scratch_bytes(int precision, int64_t M, int train) {
+  const size_t delta_sets = precision == NB200_BF16X3 ? 2 : 1;
+  return train ? (size_t)train_tiles(M) * delta_sets * kDeltaTileBytes + kPadFloats * sizeof(float) : 0;
 }
 
 // grad[r, c] += pad[r, c] for the three padded images (one thread per padded float4 group)
@@ -558,20 +500,20 @@ __global__ void __launch_bounds__(256) fold_grads_kernel(const float* __restrict
   }
 }
 
-int tc_pack_weights(const float* const* P, void* packed, int x3, cudaStream_t s) {
-  NB_TRY_RC(ensure_layout());
+int tc_pack_weights(const float* const* P, void* packed, int precision, cudaStream_t s) {
+  const bool x3 = precision == NB200_BF16X3;
   ParamPtrs pp;
   for (int i = 0; i < 24; ++i) pp.p[i] = P[i];
-  const int nslabs = x3 ? h_layout.num_fwd3 + h_layout.num_bwd3 : h_layout.num_fwd + h_layout.num_bwd + h_layout.num_fold;
+  const int nslabs = x3 ? kLayout.num_fwd3 + kLayout.num_bwd3 : kLayout.num_fwd + kLayout.num_bwd + kLayout.num_fold;
   if (!x3) {
-    fold_weights_kernel<<<kFoldWBlocks, 256, 0, s>>>(pp, reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(packed) + h_layout.f32_off));
+    fold_weights_kernel<<<kFoldWBlocks, 256, 0, s>>>(pp, reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(packed) + kLayout.f32_off));
     NB_LAUNCH_CHECK("fold_weights_kernel");
   }
   if (x3) pack_slabs_kernel<true><<<nslabs * kPackSplit, 256, 0, s>>>(pp, reinterpret_cast<uint8_t*>(packed));
   else pack_slabs_kernel<false><<<nslabs * kPackSplit, 256, 0, s>>>(pp, reinterpret_cast<uint8_t*>(packed));
   NB_LAUNCH_CHECK("pack_slabs_kernel");
   pack_f32_kernel<<<(kF32Floats + 255) / 256, 256, 0, s>>>(
-      pp, reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(packed) + (x3 ? h_layout.f32_off3 : h_layout.f32_off)));
+      pp, reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(packed) + (x3 ? kLayout.f32_off3 : kLayout.f32_off)));
   NB_LAUNCH_CHECK("pack_f32_kernel");
   return NB200_OK;
 }
@@ -582,21 +524,21 @@ static int check_arch() {
   int arch;
   {
     std::lock_guard<std::mutex> lock(g_mu);
-    if (g_dev[dev].arch == 0) g_dev[dev].arch = nb200_device_arch();
-    arch = g_dev[dev].arch;
+    if (g_arch[dev] == 0) g_arch[dev] = nb200_device_arch();
+    arch = g_arch[dev];
   }
   if (arch < 0) return NB200_ERR_CUDA;
   return (arch / 10 == 10) ? NB200_OK : NB200_ERR_ARCH;
 }
-// cudaFuncSetAttribute is per device: `which` selects the flag of the current device's DeviceState
-template <class F>
-static int ensure_attr(bool DeviceState::*which, F&& set) {
+// cudaFuncSetAttribute is per device: `done` holds one kernel's flag per device
+template <class Kernel>
+static int set_smem_once(bool (&done)[kMaxDevices], Kernel* kernel, uint32_t bytes) {
   int dev = 0;
   NB_TRY_RC(current_device(&dev));
   std::lock_guard<std::mutex> lock(g_mu);
-  if (g_dev[dev].*which) return NB200_OK;
-  NB_TRY_RC(set());
-  g_dev[dev].*which = true;
+  if (done[dev]) return NB200_OK;
+  NB_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+  done[dev] = true;
   return NB200_OK;
 }
 
@@ -612,7 +554,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 struct TmapPair { const void* packed; int dev; uint32_t rows; CUtensorMap m128, m64; };
-static int get_tmaps(const void* packed, TmapPair* out, int x3 = 0) {   // returns a COPY: the cache entry may be recycled by another thread
+static int get_tmaps(const void* packed, TmapPair* out, bool x3) {   // returns a COPY: the cache entry may be recycled by another thread
   int dev = 0;
   NB_TRY_RC(current_device(&dev));
   std::lock_guard<std::mutex> lock(g_mu);
@@ -620,7 +562,7 @@ static int get_tmaps(const void* packed, TmapPair* out, int x3 = 0) {   // retur
   static int used = 0, next = 0;
   // keyed by the image's row count too: torch's allocator hands a freed bf16 buffer's address to a bf16x3 buffer
   // (the bf16x3 map spans the whole buffer: its delta-chain slabs lie behind the fp32 tail)
-  const uint32_t rows = (x3 ? h_layout.total_bytes3 : h_layout.f32_off) / 128;
+  const uint32_t rows = (x3 ? kLayout.total_bytes3 : kLayout.f32_off) / 128;
   for (int i = 0; i < used; ++i)
     if (cache[i].packed == packed && cache[i].dev == dev && cache[i].rows == rows) { *out = cache[i]; return NB200_OK; }
   static EncodeTiledFn encode = nullptr;
@@ -655,38 +597,51 @@ static int get_tmaps(const void* packed, TmapPair* out, int x3 = 0) {   // retur
   return NB200_OK;
 }
 
-static int chain_grid(int64_t T) {
+// A cluster works on `slots` pair-tiles at a time (one per in-flight tile of each CTA); with two, two pair-tiles per
+// cluster keep the ping-pong busy.
+static int chain_grid(int64_t T, int slots) {
   const int64_t PT = (T + 1) / 2;         // 256-row pair-tiles
-  const int64_t want = (PT + 1) / 2;      // two pair-tiles per cluster keep the ping-pong busy
+  const int64_t want = (PT + slots - 1) / slots;
   const int64_t maxc = sm_count() / 2;
   const int64_t clusters = want < maxc ? (want > 0 ? want : 1) : maxc;
   return (int)(2 * clusters);
 }
 
-int tc_forward(int in_mode, const float* in0, const float* in1, int64_t M, int N, const void* packed,
-               float* out, void* saved, void*, size_t, int fold, cudaStream_t s) {
-  NB_TRY_RC(check_arch());
-  NB_TRY_RC(ensure_layout());
-  NB_TRY_RC(ensure_attr(&DeviceState::attr_fwd, []() -> int {
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<FwdEpi<false>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)kCSmemLaunch));
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<FwdEpi<true>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)kCSmemLaunch));
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<FwdEpi<false, false, true>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)kCSmemLaunch));
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<FwdEpi<true, false, true>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)kCSmemLaunch));
-    return NB200_OK;
-  }));
-  const int64_t T = saved ? train_tiles(M) : ceil_div64(M, kTileM);
-  FwdEpiParams p;
+template <class Epi>
+static int launch_chain(const typename Epi::Params& p, cudaStream_t s) {
+  static bool smem_set[kMaxDevices];
+  NB_TRY_RC(set_smem_once(smem_set, chain_kernel<Epi>, kCSmemLaunch));
+  chain_kernel<Epi><<<chain_grid(p.num_tiles, Epi::kSlots), kCThreads, kCSmemLaunch, s>>>(p);
+  NB_LAUNCH_CHECK("chain_kernel");
+  return NB200_OK;
+}
+
+// What every forward chain launch shares: the weight tensor maps, the input and the tile count.
+static int fwd_params(FwdEpiParams& p, int precision, int in_mode, const float* in0, const float* in1, int64_t M, int N,
+                      int64_t T, const void* packed) {
+  memset(&p, 0, sizeof(p));
   TmapPair tm;
-  NB_TRY_RC(get_tmaps(packed, &tm));
+  NB_TRY_RC(get_tmaps(packed, &tm, precision == NB200_BF16X3));
   p.tmap128 = tm.m128; p.tmap64 = tm.m64;
-  p.dbg = 0;
-  p.dbg_counters = nullptr;
-#ifdef NB200_DEV   // developer probe (synchronises, allocates, prints): never in the shipped library
-  { const char* e = getenv("NB200_DBG"); p.dbg = e ? atoi(e) : 0; }
+  p.in_mode = in_mode; p.in0 = in0; p.in1 = in1; p.M = M; p.N = N;
+  p.nshift = (N > 0 && (N & (N - 1)) == 0) ? __builtin_ctz((unsigned)N) : -1;
+  p.packed = reinterpret_cast<const uint8_t*>(packed);
+  p.num_tiles = T;
+  return NB200_OK;
+}
+
+// NB200_BF16X3 runs error-compensated bf16 on the same chain skeleton (one tile in flight per CTA, three MMA passes per
+// K-block: A_hi W_hi + A_lo W_hi + A_hi W_lo, fp32 accumulation in TMEM): fp32-class accuracy on the tensor cores.
+// With `saved` (training) its kernel also stores the hi and lo image of every layer input and the ReLU masks
+// (kSavedTileBytes3 per tile of train_tiles(M)); its outputs are the inference kernel's, bit for bit.
+int tc_forward(int precision, int in_mode, const float* in0, const float* in1, int64_t M, int N, const void* packed,
+               float* out, void* saved, cudaStream_t s) {
+  NB_TRY_RC(check_arch());
+  FwdEpiParams p;
+  NB_TRY_RC(fwd_params(p, precision, in_mode, in0, in1, M, N, saved ? train_tiles(M) : ceil_div64(M, kTileM), packed));
+  p.out = out; p.saved = reinterpret_cast<uint8_t*>(saved);
+#ifdef NB200_DEV   // developer probe of the bf16 chains (synchronises, allocates, prints): never in the shipped library
+  if (precision != NB200_BF16X3) { const char* e = getenv("NB200_DBG"); p.dbg = e ? atoi(e) : 0; }
   if (p.dbg & 8) {
     static unsigned long long* ctr = nullptr;
     if (!ctr) { cudaMalloc(&ctr, 512); cudaMemset(ctr, 0, 512); }
@@ -701,94 +656,25 @@ int tc_forward(int in_mode, const float* in0, const float* in1, int64_t M, int N
     p.dbg_counters = ctr;
   }
 #endif
-  p.in_mode = in_mode; p.in0 = in0; p.in1 = in1; p.M = M; p.N = N;
-  p.nshift = (N > 0 && (N & (N - 1)) == 0) ? __builtin_ctz((unsigned)N) : -1;
-  p.packed = reinterpret_cast<const uint8_t*>(packed);
-  p.out = out; p.saved = reinterpret_cast<uint8_t*>(saved);
-  p.num_tiles = T;
-  const int grid = chain_grid(T);
-  if (saved && fold)
-    chain_kernel<FwdEpi<true, false, true>><<<grid, kCThreads, kCSmemLaunch, s>>>(p);
-  else if (saved)
-    chain_kernel<FwdEpi<true>><<<grid, kCThreads, kCSmemLaunch, s>>>(p);
-  else if (fold)
-    chain_kernel<FwdEpi<false, false, true>><<<grid, kCThreads, kCSmemLaunch, s>>>(p);
-  else
-    chain_kernel<FwdEpi<false>><<<grid, kCThreads, kCSmemLaunch, s>>>(p);
-  NB_LAUNCH_CHECK("chain_kernel<FwdEpi>");
-  return NB200_OK;
-}
-
-// one tile in flight per CTA: one pair-tile per cluster and round
-static int chain_grid_x3(int64_t T) {
-  const int64_t PT = (T + 1) / 2, maxc = sm_count() / 2;
-  return (int)(2 * (PT < maxc ? PT : maxc));
-}
-
-// NB200_BF16X3: error-compensated bf16 on the same chain skeleton (one tile in flight per CTA, three MMA passes per
-// K-block: A_hi W_hi + A_lo W_hi + A_hi W_lo, fp32 accumulation in TMEM): fp32-class accuracy on the tensor cores.
-// With `saved` (training) the same kernel also stores the hi and lo image of every layer input and the ReLU masks
-// (kSavedTileBytes3 per tile of train_tiles(M)); its outputs are the inference kernel's, bit for bit.
-int tc_forward_x3(int in_mode, const float* in0, const float* in1, int64_t M, int N, const void* packed, float* out,
-                  void* saved, cudaStream_t s) {
-  NB_TRY_RC(check_arch());
-  NB_TRY_RC(ensure_layout());
-  NB_TRY_RC(ensure_attr(&DeviceState::attr_x3, []() -> int {
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<FwdEpi3<false>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCSmemLaunch));
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<FwdEpi3<true>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCSmemLaunch));
-    return NB200_OK;
-  }));
-  const int64_t T = saved ? train_tiles(M) : ceil_div64(M, kTileM);
-  FwdEpiParams p;
-  memset(&p, 0, sizeof(p));
-  TmapPair tm;
-  NB_TRY_RC(get_tmaps(packed, &tm, 1));
-  p.tmap128 = tm.m128; p.tmap64 = tm.m64;
-  p.in_mode = in_mode; p.in0 = in0; p.in1 = in1; p.M = M; p.N = N;
-  p.nshift = (N > 0 && (N & (N - 1)) == 0) ? __builtin_ctz((unsigned)N) : -1;
-  p.packed = reinterpret_cast<const uint8_t*>(packed);
-  p.out = out;
-  p.saved = reinterpret_cast<uint8_t*>(saved);
-  p.num_tiles = T;
-  const int grid = chain_grid_x3(T);
-  if (saved) chain_kernel<FwdEpi3<true>><<<grid, kCThreads, kCSmemLaunch, s>>>(p);
-  else chain_kernel<FwdEpi3<false>><<<grid, kCThreads, kCSmemLaunch, s>>>(p);
-  NB_LAUNCH_CHECK("chain_kernel<FwdEpi3>");
-  return NB200_OK;
+  if (precision == NB200_BF16_LAYERWISE) return !saved ? launch_chain<FwdEpi<false>>(p, s) : launch_chain<FwdEpi<true>>(p, s);
+  if (precision == NB200_BF16) return !saved ? launch_chain<FwdEpi<false, false, true>>(p, s) : launch_chain<FwdEpi<true, false, true>>(p, s);
+  return !saved ? launch_chain<FwdEpi3<false>>(p, s) : launch_chain<FwdEpi3<true>>(p, s);
 }
 
 // Fused render: sampler -> posenc + MLP -> compositing in ONE kernel; per-sample (r,g,b,sigma) and the
 // sample depths never reach HBM.  rays == nullptr: rays are generated from (poses, H, W, f, ray_begin).
 // ts == nullptr: Philox sample depths (same stream as nb200_stratified_ts with the same seed/offset).
-int tc_render(const float* rays, const float* poses, int H, int W, float f, int64_t ray_begin, const float* ts, uint64_t seed,
-              uint64_t offset, int64_t B, int N, float tn, float tf, const void* packed, float* rgb, float* disp, float* acc,
-              int fold, cudaStream_t s) {
+int tc_render(int precision, const float* rays, const float* poses, int H, int W, float f, int64_t ray_begin, const float* ts,
+              uint64_t seed, uint64_t offset, int64_t B, int N, float tn, float tf, const void* packed, float* rgb, float* disp,
+              float* acc, cudaStream_t s) {
   NB_TRY_RC(check_arch());
-  NB_TRY_RC(ensure_layout());
-  NB_TRY_RC(ensure_attr(&DeviceState::attr_render, []() -> int {
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<FwdEpi<false, true>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)kCSmemLaunch));
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<FwdEpi<false, true, true>>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)kCSmemLaunch));
-    return NB200_OK;
-  }));
-  const int64_t M = B * N, T = ceil_div64(M, kTileM);
+  const int64_t M = B * N;
   FwdEpiParams p;
-  memset(&p, 0, sizeof(p));
-  TmapPair tm;
-  NB_TRY_RC(get_tmaps(packed, &tm));
-  p.tmap128 = tm.m128; p.tmap64 = tm.m64;
-  p.in_mode = rays ? NB200_IN_RAYS : kInCamera; p.in0 = rays; p.in1 = ts; p.M = M; p.N = N;
-  p.nshift = (N > 0 && (N & (N - 1)) == 0) ? __builtin_ctz((unsigned)N) : -1;
-  p.packed = reinterpret_cast<const uint8_t*>(packed);
-  p.num_tiles = T;
+  NB_TRY_RC(fwd_params(p, precision, rays ? NB200_IN_RAYS : kInCamera, rays, ts, M, N, ceil_div64(M, kTileM), packed));
   p.rgb = rgb; p.disp = disp; p.acc = acc; p.B = B;
   p.sampler = ts ? 0 : 1; p.seed = seed; p.offset = offset; p.tn = tn; p.tf = tf;
   p.poses = poses; p.H = H; p.W = W; p.f = f; p.ray_begin = ray_begin;
-  if (fold) chain_kernel<FwdEpi<false, true, true>><<<chain_grid(T), kCThreads, kCSmemLaunch, s>>>(p);
-  else chain_kernel<FwdEpi<false, true>><<<chain_grid(T), kCThreads, kCSmemLaunch, s>>>(p);
-  NB_LAUNCH_CHECK("chain_kernel<FwdEpi<render>>");
-  return NB200_OK;
+  return precision == NB200_BF16_LAYERWISE ? launch_chain<FwdEpi<false, true>>(p, s) : launch_chain<FwdEpi<false, true, true>>(p, s);
 }
 
 // One wgrad item: dW (+)= (delta tensor dt of `ds`)^T (saved tensor st of `sv`), rows of the layer's weight from col0.
@@ -811,11 +697,12 @@ static void wgrad_item(WItem& w, const uint8_t* ds, const uint8_t* sv, int64_t T
   w.cost = (w.a_chunks + w.b_chunks) * 16;
   w.head = 0; w.x_ptr = nullptr; w.x_tile_bytes = 0; w.x_chunks = 0; w.hW = nullptr; w.hb = nullptr;
 }
-// the sigma / colour head gradients ride on the item that stages their input (h7 / an extra c1 slab)
-static void wgrad_head(WItem& w, const uint8_t* sv, int64_t T, float* const* G, int which, int st, int layer) {
+// the sigma (1) / colour (2) head gradients ride on the item that stages their input (h7 / an extra c1 slab)
+static void wgrad_head(WItem& w, const uint8_t* sv, int64_t T, float* const* G, int which) {
+  const int layer = which == 1 ? L_SIGMA : L_C1;
   w.head = which; w.hW = G[2 * layer]; w.hb = G[2 * layer + 1];
   if (which == 2) {
-    w.x_ptr = sv + saved_tensor_off(st, T); w.x_tile_bytes = (uint32_t)saved_tile_bytes(st); w.x_chunks = 2;
+    w.x_ptr = sv + saved_tensor_off(9, T); w.x_tile_bytes = (uint32_t)saved_tile_bytes(9); w.x_chunks = 2;
     w.cost += w.x_chunks * 16;
   }
 }
@@ -836,152 +723,94 @@ static void wgrad_costs(WItem* items, int n) {
   }
 }
 
-int tc_backward(int, const float*, const float*, int64_t M, int, const void* packed, const float* d_out,
-                const void* saved, float* const* G, void* scratch, size_t scratch_bytes, int fold, cudaStream_t s) {
+template <bool kX3>
+static int launch_wgrad(const WItem* items, int n, int64_t T, int64_t M, const float* d_out, cudaStream_t s) {
+  std::conditional_t<kX3, WgradParams3, WgradParams> p;
+  memset(&p, 0, sizeof(p));
+  memcpy(p.items, items, (size_t)n * sizeof(WItem));
+  p.num_items = n; p.T = T; p.M = M; p.d_out = d_out;
+  static bool smem_set[kMaxDevices];
+  NB_TRY_RC(set_smem_once(smem_set, mlp_wgrad_tc_kernel<kX3>, kWgSmemLaunch));
+  mlp_wgrad_tc_kernel<kX3><<<sm_count(), kWgThreads, kWgSmemLaunch, s>>>(p);
+  NB_LAUNCH_CHECK("mlp_wgrad_tc_kernel");
+  return NB200_OK;
+}
+
+// The (delta tensor, input tensor) pairs of the layer-by-layer chain, in the order wgrad splits and sums them.  `head`:
+// the sigma (1) / colour (2) head gradients ride on that item.
+struct WPair { int dt, st, layer, ldw, col0, ncols, nrows; bool bias; int head; };
+constexpr WPair kWPairs[] = {
+    {0, 8, L_C0, kHidden + kPosD, 0, kHidden, kHidden / 2, true, 0},         // color_fc.0 <- g
+    {0, 11, L_C0, kHidden + kPosD, kHidden, kPosD, kHidden / 2, false, 2},   // color_fc.0 <- posd; color_fc.2 <- c1
+    {1, 7, L_2, kHidden, 0, kHidden, kHidden, true, 1},                      // layers_2   <- h7;   sigma_fc   <- h7
+    {2, 6, L1_1, kHidden, 0, kHidden, kHidden, true, 0},                     // layers_1.2 <- h6
+    {3, 5, L1_0, kHidden, 0, kHidden, kHidden, true, 0},                     // layers_1.0 <- h5
+    {4, 4, L_SKIP, kHidden + kPosX, 0, kHidden, kHidden, true, 0},           // skip       <- h4
+    {4, 10, L_SKIP, kHidden + kPosX, kHidden, kPosX, kHidden, false, 0},     // skip       <- posx
+    {5, 3, L0_4, kHidden, 0, kHidden, kHidden, true, 0},                     // layers_0.8 <- h3
+    {6, 2, L0_3, kHidden, 0, kHidden, kHidden, true, 0},
+    {7, 1, L0_2, kHidden, 0, kHidden, kHidden, true, 0},
+    {8, 0, L0_1, kHidden, 0, kHidden, kHidden, true, 0},
+    {9, 10, L0_0, kPosX, 0, kPosX, kHidden, true, 0},                        // layers_0.0 <- posx
+};
+static_assert(sizeof(kWPairs) / sizeof(WPair) == kMaxWItems, "one wgrad item per pair");
+
+// Backward: the delta chain (chain_kernel<DgradEpi> / <DgradEpi3>), then wgrad over the pairs above.
+// NB200_BF16: Gm = delta_c1^T h7 (pad image of color_fc.0, with the column sums of delta_c1 as its "bias") replaces
+// color_fc.0 <- g and layers_2 <- h7 and carries the sigma head; fold_grads_kernel un-folds it.
+// NB200_BF16X3: hi / lo deltas, and every pair as three items, dW = d_hi^T a_hi + d_lo^T a_hi + d_hi^T a_lo.  The bias
+// sums ride on the two items that stage a_hi (sum d_hi + sum d_lo); of the two carriers of each head (hi and lo) only
+// the hi one adds the head-bias sums.
+int tc_backward(int precision, int64_t M, const void* packed, const float* d_out, const void* saved, float* const* G,
+                void* scratch, size_t scratch_bytes, cudaStream_t s) {
   NB_TRY_RC(check_arch());
-  NB_TRY_RC(ensure_layout());
-  if (!scratch || scratch_bytes < tc_scratch_bytes(M, 1)) return NB200_ERR_WORKSPACE;
-  NB_TRY_RC(ensure_attr(&DeviceState::attr_bwd, []() -> int {
-    NB_CUDA_CHECK(cudaFuncSetAttribute(mlp_wgrad_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgSmemLaunch));
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<DgradEpi<false>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCSmemLaunch));
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<DgradEpi<true>>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCSmemLaunch));
-    return NB200_OK;
-  }));
+  if (!scratch || scratch_bytes < tc_scratch_bytes(precision, M, 1)) return NB200_ERR_WORKSPACE;
+  const bool x3 = precision == NB200_BF16X3, fold = precision == NB200_BF16;
   const int64_t T = train_tiles(M);
   const uint8_t* sv = reinterpret_cast<const uint8_t*>(saved);
   uint8_t* ds = reinterpret_cast<uint8_t*>(scratch);
-  float* pad = reinterpret_cast<float*>(ds + (size_t)T * kDeltaTileBytes);
+  const uint8_t* sv_lo = sv + kSavedDataTileBytes * (size_t)T;   // bf16x3 only
+  const uint8_t* ds_lo = ds + kDeltaTileBytes * (size_t)T;       // bf16x3 only
+  float* pad = reinterpret_cast<float*>(ds + (x3 ? 2 : 1) * kDeltaTileBytes * (size_t)T);
   NB_CUDA_CHECK(cudaMemsetAsync(pad, 0, kPadFloats * sizeof(float), s));
-  // 1. fused delta chain
+  // 1. delta chain
   BwdParams bp;
-  bp.dbg = 0;
+  memset(&bp, 0, sizeof(bp));
+  TmapPair tm;
+  NB_TRY_RC(get_tmaps(packed, &tm, x3));
+  bp.tmap128 = tm.m128; bp.tmap64 = tm.m64;
   bp.M = M; bp.num_tiles = T; bp.packed = reinterpret_cast<const uint8_t*>(packed); bp.saved = sv;
   bp.d_out = d_out; bp.dscr = ds;
-  {
-    TmapPair tm;
-    NB_TRY_RC(get_tmaps(packed, &tm));
-    bp.tmap128 = tm.m128; bp.tmap64 = tm.m64;
-    if (fold) chain_kernel<DgradEpi<true>><<<chain_grid(T), kCThreads, kCSmemLaunch, s>>>(bp);
-    else chain_kernel<DgradEpi<false>><<<chain_grid(T), kCThreads, kCSmemLaunch, s>>>(bp);
-    NB_LAUNCH_CHECK("chain_kernel<DgradEpi>");
-  }
-  // 2. weight gradients: (delta tensor, input tensor) pairs
-  WgradParams wp;
-  memset(&wp, 0, sizeof(wp));
-  wp.T = T; wp.M = M; wp.d_out = d_out;
+  NB_TRY_RC(x3 ? launch_chain<DgradEpi3>(bp, s) : (fold ? launch_chain<DgradEpi<true>>(bp, s) : launch_chain<DgradEpi<false>>(bp, s)));
+  // 2. weight gradients
+  WItem items[kMaxWItems3];
   int n = 0;
-  auto item = [&](int dt, int st, int layer, int ldw, int col0, int ncols, int nrows, bool bias) {
-    wgrad_item(wp.items[n++], ds, sv, T, pad, G, dt, st, layer, ldw, col0, ncols, nrows, bias);
-  };
-  auto head = [&](int which, int st, int layer) { wgrad_head(wp.items[n - 1], sv, T, G, which, st, layer); };
-  if (fold) {
-    item(0, 7, L_C0, kHidden + kPosD, 0, kHidden, kHidden / 2, true);      // Gm = delta_c1^T h7 -> pad image of color_fc.0
-    wp.items[n - 1].db = pad + kPadFoldS;                                   //   column sums of delta_c1 (un-folded below)
-    head(1, 7, L_SIGMA);                                                    // sigma_fc   <- h7 (CUDA cores)
-    item(0, 11, L_C0, kHidden + kPosD, kHidden, kPosD, kHidden / 2, false);  // color_fc.0 <- posd
-    head(2, 9, L_C1);                                                       // color_fc.2 <- c1 (CUDA cores)
-  } else {
-    item(0, 8, L_C0, kHidden + kPosD, 0, kHidden, kHidden / 2, true);        // color_fc.0 <- g
-    item(0, 11, L_C0, kHidden + kPosD, kHidden, kPosD, kHidden / 2, false);  // color_fc.0 <- posd
-    head(2, 9, L_C1);                                                         // color_fc.2 <- c1 (CUDA cores)
-    item(1, 7, L_2, kHidden, 0, kHidden, kHidden, true);                      // layers_2   <- h7
-    head(1, 7, L_SIGMA);                                                      // sigma_fc   <- h7 (CUDA cores)
+  for (const WPair& q : kWPairs) {
+    if (fold && q.layer == L_2) continue;
+    const bool gm = fold && q.st == 8;   // color_fc.0 <- g becomes Gm = delta_c1^T h7
+    const int st = gm ? 7 : q.st, head = gm ? 1 : q.head;
+    for (int k = 0; k < (x3 ? 3 : 1); ++k) {   // bf16x3: d_hi^T a_hi, d_lo^T a_hi, d_hi^T a_lo
+      WItem& w = items[n++];
+      wgrad_item(w, k == 1 ? ds_lo : ds, k == 2 ? sv_lo : sv, T, pad, G, q.dt, st, q.layer, q.ldw, q.col0, q.ncols, q.nrows,
+                 q.bias && k < 2);
+      if (gm) w.db = pad + kPadFoldS;   // column sums of delta_c1 (un-folded below)
+      if (head && k != 1) wgrad_head(w, k == 2 ? sv_lo : sv, T, G, head);
+      if (head && k == 2) w.hb = nullptr;
+    }
   }
-  item(2, 6, L1_1, kHidden, 0, kHidden, kHidden, true);                     // layers_1.2 <- h6
-  item(3, 5, L1_0, kHidden, 0, kHidden, kHidden, true);                     // layers_1.0 <- h5
-  item(4, 4, L_SKIP, kHidden + kPosX, 0, kHidden, kHidden, true);           // skip       <- h4
-  item(4, 10, L_SKIP, kHidden + kPosX, kHidden, kPosX, kHidden, false);     // skip       <- posx
-  item(5, 3, L0_4, kHidden, 0, kHidden, kHidden, true);                     // layers_0.8 <- h3
-  item(6, 2, L0_3, kHidden, 0, kHidden, kHidden, true);
-  item(7, 1, L0_2, kHidden, 0, kHidden, kHidden, true);
-  item(8, 0, L0_1, kHidden, 0, kHidden, kHidden, true);
-  item(9, 10, L0_0, kPosX, 0, kPosX, kHidden, true);                        // layers_0.0 <- posx
-  wgrad_costs(wp.items, n);
+  wgrad_costs(items, n);   // the bf16 chain's measured per-kind costs; the three items of a bf16x3 pair were not timed apart
 #ifdef NB200_DEV   // developer probe: time one item alone (leaves the other gradients at zero -- never in the shipped library)
-  { const char* e = getenv("NB200_WG_ONLY"); if (e) { const int k = atoi(e); if (k >= 0 && k < n) { wp.items[0] = wp.items[k]; n = 1; } } }
+  if (!x3) { const char* e = getenv("NB200_WG_ONLY"); if (e) { const int k = atoi(e); if (k >= 0 && k < n) { items[0] = items[k]; n = 1; } } }
 #endif
-  wp.num_items = n;
-  mlp_wgrad_tc_kernel<false><<<sm_count(), kWgThreads, kWgSmemLaunch, s>>>(wp);
-  NB_LAUNCH_CHECK("mlp_wgrad_tc_kernel");
+  NB_TRY_RC(x3 ? launch_wgrad<true>(items, n, T, M, d_out, s) : launch_wgrad<false>(items, n, T, M, d_out, s));
   unpad_add_kernel<<<((int)kPadFoldS + 255) / 256, 256, 0, s>>>(pad, G[2 * L_C0], G[2 * L_SKIP], G[2 * L0_0], fold);
   NB_LAUNCH_CHECK("unpad_add_kernel");
   if (fold) {
     fold_grads_kernel<<<kFoldGBlocks, 256, 0, s>>>(
-        pad, reinterpret_cast<const float*>(reinterpret_cast<const uint8_t*>(packed) + h_layout.f32_off), G[2 * L_C0], G[2 * L_C0 + 1],
+        pad, reinterpret_cast<const float*>(reinterpret_cast<const uint8_t*>(packed) + kLayout.f32_off), G[2 * L_C0], G[2 * L_C0 + 1],
         G[2 * L_2], G[2 * L_2 + 1]);
     NB_LAUNCH_CHECK("fold_grads_kernel");
   }
-  return NB200_OK;
-}
-
-// NB200_BF16X3 backward: the delta chain in error-compensated bf16 (chain_kernel<DgradEpi3>, hi / lo deltas), then wgrad
-// with every (delta, input) pair of the layer-by-layer chain as three items, dW = d_hi^T a_hi + d_lo^T a_hi + d_hi^T a_lo.
-// The bias sums ride on the two items that stage a_hi (sum d_hi + sum d_lo); of the two carriers of each head (h7 / c1,
-// hi and lo) only the hi one adds the head-bias sums.
-int tc_backward_x3(int64_t M, const void* packed, const float* d_out, const void* saved, float* const* G, void* scratch,
-                   size_t scratch_bytes, cudaStream_t s) {
-  NB_TRY_RC(check_arch());
-  NB_TRY_RC(ensure_layout());
-  if (!scratch || scratch_bytes < tc_scratch_bytes_x3(M, 1)) return NB200_ERR_WORKSPACE;
-  NB_TRY_RC(ensure_attr(&DeviceState::attr_bwd3, []() -> int {
-    NB_CUDA_CHECK(cudaFuncSetAttribute(mlp_wgrad_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kWgSmemLaunch));
-    NB_CUDA_CHECK(cudaFuncSetAttribute(chain_kernel<DgradEpi3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kCSmemLaunch));
-    return NB200_OK;
-  }));
-  const int64_t T = train_tiles(M);
-  const uint8_t* sv_hi = reinterpret_cast<const uint8_t*>(saved);
-  const uint8_t* sv_lo = sv_hi + kSavedDataTileBytes * (size_t)T;
-  uint8_t* ds_hi = reinterpret_cast<uint8_t*>(scratch);
-  uint8_t* ds_lo = ds_hi + kDeltaTileBytes * (size_t)T;
-  float* pad = reinterpret_cast<float*>(ds_lo + kDeltaTileBytes * (size_t)T);
-  NB_CUDA_CHECK(cudaMemsetAsync(pad, 0, kPadFloats * sizeof(float), s));
-  // 1. delta chain
-  BwdParams bp;
-  bp.dbg = 0;
-  bp.M = M; bp.num_tiles = T; bp.packed = reinterpret_cast<const uint8_t*>(packed); bp.saved = sv_hi;
-  bp.d_out = d_out; bp.dscr = ds_hi;
-  {
-    TmapPair tm;
-    NB_TRY_RC(get_tmaps(packed, &tm, 1));
-    bp.tmap128 = tm.m128; bp.tmap64 = tm.m64;
-    chain_kernel<DgradEpi3><<<chain_grid_x3(T), kCThreads, kCSmemLaunch, s>>>(bp);
-    NB_LAUNCH_CHECK("chain_kernel<DgradEpi3>");
-  }
-  // 2. weight gradients
-  WgradParams3 wp;
-  memset(&wp, 0, sizeof(wp));
-  wp.T = T; wp.M = M; wp.d_out = d_out;
-  int n = 0;
-  // `head`: the sigma (1) / colour (2) head rides on the items that stage h7 / c1, hi with the head bias, lo without
-  auto item3 = [&](int dt, int st, int layer, int ldw, int col0, int ncols, int nrows, bool bias, int head = 0, int hst = 0, int hlayer = 0) {
-    wgrad_item(wp.items[n++], ds_hi, sv_hi, T, pad, G, dt, st, layer, ldw, col0, ncols, nrows, bias);
-    if (head) wgrad_head(wp.items[n - 1], sv_hi, T, G, head, hst, hlayer);
-    wgrad_item(wp.items[n++], ds_lo, sv_hi, T, pad, G, dt, st, layer, ldw, col0, ncols, nrows, bias);
-    wgrad_item(wp.items[n++], ds_hi, sv_lo, T, pad, G, dt, st, layer, ldw, col0, ncols, nrows, false);
-    if (head) {
-      wgrad_head(wp.items[n - 1], sv_lo, T, G, head, hst, hlayer);
-      wp.items[n - 1].hb = nullptr;
-    }
-  };
-  item3(0, 8, L_C0, kHidden + kPosD, 0, kHidden, kHidden / 2, true);                     // color_fc.0 <- g
-  item3(0, 11, L_C0, kHidden + kPosD, kHidden, kPosD, kHidden / 2, false, 2, 9, L_C1);  // color_fc.0 <- posd; color_fc.2 <- c1
-  item3(1, 7, L_2, kHidden, 0, kHidden, kHidden, true, 1, 7, L_SIGMA);                   // layers_2 <- h7; sigma_fc <- h7
-  item3(2, 6, L1_1, kHidden, 0, kHidden, kHidden, true);
-  item3(3, 5, L1_0, kHidden, 0, kHidden, kHidden, true);
-  item3(4, 4, L_SKIP, kHidden + kPosX, 0, kHidden, kHidden, true);
-  item3(4, 10, L_SKIP, kHidden + kPosX, kHidden, kPosX, kHidden, false);
-  item3(5, 3, L0_4, kHidden, 0, kHidden, kHidden, true);
-  item3(6, 2, L0_3, kHidden, 0, kHidden, kHidden, true);
-  item3(7, 1, L0_2, kHidden, 0, kHidden, kHidden, true);
-  item3(8, 0, L0_1, kHidden, 0, kHidden, kHidden, true);
-  item3(9, 10, L0_0, kPosX, 0, kPosX, kHidden, true);
-  // the bf16 chain's measured per-kind costs; the three items of a pair stage the same bytes (not separately measured)
-  wgrad_costs(wp.items, n);
-  wp.num_items = n;
-  mlp_wgrad_tc_kernel<true><<<sm_count(), kWgThreads, kWgSmemLaunch, s>>>(wp);
-  NB_LAUNCH_CHECK("mlp_wgrad_tc_kernel<bf16x3>");
-  unpad_add_kernel<<<((int)kPadFoldS + 255) / 256, 256, 0, s>>>(pad, G[2 * L_C0], G[2 * L_SKIP], G[2 * L0_0], 0);
-  NB_LAUNCH_CHECK("unpad_add_kernel");
   return NB200_OK;
 }
 

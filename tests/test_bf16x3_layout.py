@@ -1,7 +1,7 @@
 """Buffer sizes of the bf16x3 training path, computed from shapes (no GPU needed: the queries are host-only).
 
-Loading the library also builds the packed-weight tables and checks them against the compile-time MMA schedules of
-every chain kernel (the bf16x3 delta chain's included); a mismatch aborts the process."""
+The packed image's size is read from the compile-time packed layout, the table from which the chain kernels' MMA
+schedules are also derived."""
 
 KB = 1024
 TILE_DATA = 9 * 64 * KB + 32 * KB + 16 * KB + 16 * KB     # h0..h7, g | c1 | posx | posd per 128-sample tile (bf16 images)
