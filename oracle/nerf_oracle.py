@@ -222,10 +222,12 @@ def volume_render_backward(nerf_outs, ts, dirs, d_rgb, d_disp=None, d_alpha=None
                            d_w=None, dtype=np.float32):
     """Analytic gradient of volume_render w.r.t. nerf_outs [B,N,4] (what autograd computes
     through utils/rendering.py:60-83; ts/dirs carry no grad).  The exclusive-cumprod backward is
-    reverse_cumsum(grad*T)/factor, PyTorch's formula for zero-free inputs (factors are >= 1e-10)."""
+    reverse_cumsum(grad*T)/factor, PyTorch's formula for zero-free inputs (factors are >= 1e-10).
+    Without d_disp the disparity is not part of the graph, so a transparent ray (acc = 0) gets no NaN from it."""
     o = nerf_outs.astype(dtype); ts = ts.astype(dtype); dirs = dirs.astype(dtype)
     B, N = ts.shape
     z = lambda a, shp: np.zeros(shp, dtype) if a is None else a.astype(dtype)
+    use_disp = d_disp is not None
     d_rgb = z(d_rgb, (B, 3)); d_disp = z(d_disp, (B,)); d_alpha = z(d_alpha, (B, N))
     d_acc = z(d_acc, (B,)); d_w = z(d_w, (B, N))
     deltas = ts[:, 1:] - ts[:, :-1]
@@ -244,8 +246,8 @@ def volume_render_backward(nerf_outs, ts, dirs, d_rgb, d_disp=None, d_alpha=None
         m = np.maximum(dtype(1e-10), q)
         d_m = -d_disp / (m * m)
         d_q = np.where(q > 1e-10, d_m, 0)
-        d_depth = d_q / acc
-        d_acc_t = d_acc - d_q * depth / (acc * acc)
+        d_depth = d_q / acc if use_disp else np.zeros_like(acc)
+        d_acc_t = d_acc - d_q * depth / (acc * acc) if use_disp else d_acc
         gw = (d_w + np.einsum("bnc,bc->bn", o[..., :3], d_rgb) + d_depth[:, None] * ts
               + d_acc_t[:, None])                      # total d(loss)/d(w_i)
         gwT = gw * w                                   # = d_T_i * T_i with d_T_i = gw_i*alpha_i
