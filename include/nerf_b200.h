@@ -215,6 +215,14 @@ int nb200_stratified_ts_state(uint64_t seed, const void* state, int64_t B, int N
                               nb200_stream_t stream);   /* Philox mode, N % 4 == 0 */
 int nb200_adam_step_state(float* param, const float* grad, float* exp_avg, float* exp_avg_sq, int64_t n,
                           const void* state, float beta1, float beta2, float eps, nb200_stream_t stream);
+/* Graph-replayable form of nb200_sample_pdf_merge, Philox mode (mode 2): the stream position is the train state's
+ * sampler position (the `sample_offset` nb200_stratified_ts_state reads), read on the device.  Output is identical to
+ * nb200_sample_pdf_merge(ts, weights, NULL, 2, seed, <state's sample_offset>, B, Nc, Nf, z_all).  Same limits:
+ * 3 <= Nc <= 128, Nc + Nf <= 384.  The fine draws use their own Philox counter tag, so sharing the position with the
+ * stratified sampler reuses no random number; a step that calls both advances sample_offset by
+ * max(ceil(B*Nc/4), ceil(B*Nf/4)). */
+int nb200_sample_pdf_merge_state(const float* ts, const float* weights, uint64_t seed, const void* state,
+                                 int64_t B, int Nc, int Nf, float* z_all, nb200_stream_t stream);
 
 /* Data-parallel training (new functionality, SURVEY 8e; the reference is single-GPU): the gradient all-reduce FUSED
  * into the Adam update over NVLink peer memory.  Replaces an NCCL all-reduce of the flat gradient followed by

@@ -57,6 +57,7 @@ SYMBOLS = {
     "nb200_adam_allreduce_p2p": (_i, [_p, _p, _p, _i, _i, _p, _p, _i64, _p, _f, _f, _f, _p]),
     "nb200_frame_to_u8": (_i, [_p, _i64, _i, _p, _p]),
     "nb200_sample_pdf_merge": (_i, [_p, _p, _p, _i, _u64, _u64, _i64, _i, _i, _p, _p]),
+    "nb200_sample_pdf_merge_state": (_i, [_p, _p, _u64, _p, _i64, _i, _i, _p, _p]),
 }
 
 _lib = None

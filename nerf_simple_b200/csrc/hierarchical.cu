@@ -8,6 +8,7 @@
 // search; the merge is a rank count (coarse depths are sorted, fine ones need not be).
 // HBM traffic: 8 B/coarse sample read (+4 B/fine sample of u) and 4 B per merged sample written.
 #include "common.cuh"
+#include "stream_common.cuh"
 
 namespace nb200 {
 
@@ -15,6 +16,9 @@ constexpr int kHsWarps = 4;
 constexpr int kHsMaxNc = 128, kHsMaxAll = 384;
 
 __device__ __forceinline__ uint32_t hs_mulhilo(uint32_t a, uint32_t b, uint32_t* hi) { *hi = __umulhi(a, b); return a * b; }
+// The fine stream's counter tag c2 = "HSP1" keeps it disjoint from philox4x32_10 (c2 = 0), the stratified sampler's
+// generator: in a training step both read the same train-state position (sample_offset) with keys derived from one
+// seed, and the tag is what makes their draws independent.
 __device__ __forceinline__ uint4 hs_philox(uint64_t ctr, uint64_t seed) {
   uint32_t c0 = (uint32_t)ctr, c1 = (uint32_t)(ctr >> 32), c2 = 0x48535031u /* stream tag "HSP1" */, c3 = 0u;
   uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
@@ -28,10 +32,12 @@ __device__ __forceinline__ uint4 hs_philox(uint64_t ctr, uint64_t seed) {
   return make_uint4(c0, c1, c2, c3);
 }
 
-// mode: 0 = u supplied by the caller, 1 = deterministic linspace(0,1,Nf), 2 = Philox
+// mode: 0 = u supplied by the caller, 1 = deterministic linspace(0,1,Nf), 2 = Philox at offset (+ *offset_dev when
+// non-null: the device-resident stream position of a CUDA-graph-replayed training step)
 __global__ void __launch_bounds__(kHsWarps * 32)
 sample_pdf_merge_kernel(const float* __restrict__ ts, const float* __restrict__ weights, const float* __restrict__ u_in,
-                        int mode, uint64_t seed, uint64_t offset, int64_t B, int Nc, int Nf, float* __restrict__ z_all) {
+                        int mode, uint64_t seed, uint64_t offset, int64_t B, int Nc, int Nf, float* __restrict__ z_all,
+                        const uint64_t* __restrict__ offset_dev) {
   __shared__ float s_cdf[kHsWarps][kHsMaxNc];
   __shared__ float s_bins[kHsWarps][kHsMaxNc];
   __shared__ float s_all[kHsWarps][kHsMaxAll];
@@ -42,6 +48,7 @@ sample_pdf_merge_kernel(const float* __restrict__ ts, const float* __restrict__ 
   const int nb = Nc - 1;   // bins / cdf entries
   const int nw = Nc - 2;   // interior weights
   const int NA = Nc + Nf;
+  if (offset_dev) offset += *offset_dev;
   for (int64_t ray = (int64_t)blockIdx.x * kHsWarps + warp; ray < B; ray += (int64_t)gridDim.x * kHsWarps) {
     const float* t = ts + ray * Nc;
     const float* w = weights + ray * Nc;
@@ -122,7 +129,22 @@ extern "C" int nb200_sample_pdf_merge(const float* ts, const float* weights, con
   const int64_t blocks = ceil_div64(B, kHsWarps);
   const int64_t cap = (int64_t)sm_count() * 16;
   sample_pdf_merge_kernel<<<(unsigned)(blocks < cap ? blocks : cap), kHsWarps * 32, 0, as_stream(stream)>>>(
-      ts, weights, u, mode, seed, offset, B, Nc, Nf, z_all);
+      ts, weights, u, mode, seed, offset, B, Nc, Nf, z_all, nullptr);
+  NB_LAUNCH_CHECK("sample_pdf_merge_kernel");
+  return NB200_OK;
+}
+
+extern "C" int nb200_sample_pdf_merge_state(const float* ts, const float* weights, uint64_t seed, const void* state,
+                                            int64_t B, int Nc, int Nf, float* z_all, nb200_stream_t stream) {
+  using namespace nb200;
+  if (!state || B < 0 || Nc < 3 || Nf < 1) return NB200_ERR_ARG;
+  if (Nc > kHsMaxNc || Nc + Nf > kHsMaxAll) return NB200_ERR_UNSUPPORTED;
+  if (B == 0) return NB200_OK;
+  if (!ts || !weights || !z_all) return NB200_ERR_ARG;
+  const int64_t blocks = ceil_div64(B, kHsWarps);
+  const int64_t cap = (int64_t)sm_count() * 16;
+  sample_pdf_merge_kernel<<<(unsigned)(blocks < cap ? blocks : cap), kHsWarps * 32, 0, as_stream(stream)>>>(
+      ts, weights, nullptr, 2, seed, 0, B, Nc, Nf, z_all, &reinterpret_cast<const TrainState*>(state)->sample_offset);
   NB_LAUNCH_CHECK("sample_pdf_merge_kernel");
   return NB200_OK;
 }

@@ -188,17 +188,7 @@ __global__ void __launch_bounds__(1024) mse_loss_grad_kernel(const float* __rest
 }
 
 // ------------------------------------------------------------------ device-resident step state
-// What changes from one training step to the next lives on the device, so that a whole step can be
-// captured once in a CUDA graph and replayed: Philox stream positions, Adam's step count, the lr.
-struct TrainState {
-  uint64_t select_offset;   // Philox counter of the ray selection
-  uint64_t sample_offset;   // Philox counter of the stratified sampler (quads)
-  int64_t step;             // optimizer steps taken so far
-  float lr;                 // current learning rate
-  float pad;
-};
-static_assert(sizeof(TrainState) == NB200_TRAIN_STATE_BYTES, "train state layout");
-
+// (TrainState: stream_common.cuh)
 __global__ void __launch_bounds__(256) adam_flat_state_kernel(float* __restrict__ p, const float* __restrict__ g,
                                                               float* __restrict__ m, float* __restrict__ v, int64_t n,
                                                               const TrainState* __restrict__ st, float beta1, float beta2, float eps) {

@@ -4,7 +4,22 @@
 #pragma once
 #include <stdint.h>
 
+#include "../../include/nerf_b200.h"
+
 namespace nb200 {
+
+// ------------------------------------------------------------------ device-resident step state
+// What changes from one training step to the next lives on the device, so that a whole step can be
+// captured once in a CUDA graph and replayed: Philox stream positions, Adam's step count, the lr.
+// Read by the *_state entry points of rays_sampler.cu and hierarchical.cu.
+struct TrainState {
+  uint64_t select_offset;   // Philox counter of the ray selection
+  uint64_t sample_offset;   // Philox counter of the stratified and the fine sampler (quads)
+  int64_t step;             // optimizer steps taken so far
+  float lr;                 // current learning rate
+  float pad;
+};
+static_assert(sizeof(TrainState) == NB200_TRAIN_STATE_BYTES, "train state layout");
 
 // ------------------------------------------------------------------------------- ray grid
 // World ray r of the table [P*H*W]: pose r / (H*W), pixel (h, w) = divmod(r % (H*W), W).

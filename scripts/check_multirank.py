@@ -4,6 +4,8 @@
   2. a data-parallel Trainer: ranks draw different rays, replicas start identical (broadcast) and stay identical,
      the all-reduced gradient is the mean of the per-rank gradients, the loss falls; checked in the launch mode
      given by NB200_P2P_ALLREDUCE (1: all-reduce fused into the Adam kernel over peer memory, one graph; 0: NCCL between two graphs).
+     --fine: the Trainer trains a coarse and a fine network (hierarchical sampling, 32 + 64 samples); both networks'
+     parameters live in the one flat buffer the checks compare.
 Prints one JSON line on rank 0 and exits non-zero on any failed check."""
 import json
 import os
@@ -19,6 +21,7 @@ from nerf_simple_b200.nets import Nerf                              # noqa: E402
 from nerf_simple_b200.trainer import Trainer                        # noqa: E402
 from nerf_simple_b200.xyz import poses_to_render                    # noqa: E402
 
+FINE = "--fine" in sys.argv[1:]
 rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
 torch.cuda.set_device(local)
 dev = torch.device("cuda", local)
@@ -28,7 +31,7 @@ net = Nerf().to(dev)
 poses = torch.stack(poses_to_render(4, -30, 3)).to(dev)
 H = W = 96
 n = H * W
-res = {}
+res = {"fine": FINE}
 # ---- 1. sharded frame == single-GPU frame (same weights everywhere first)
 for p in net.parameters():
     dist.broadcast(p.data, 0)
@@ -47,7 +50,8 @@ torch.manual_seed(100 + rank)
 net = Nerf().to(dev)                                 # different weights per rank again
 rays = ops.generate_rays(poses, H, W, 133.3)
 gt = torch.sigmoid(rays[:, 3:6] * 3)
-tr = Trainer(net, rays, gt, N=32, batch_size=1024, seed=1, world_size=world)      # same seed argument on every rank
+fine_kw = dict(net_fine=Nerf().to(dev), Nf=64) if FINE else {}                   # different fine weights per rank too
+tr = Trainer(net, rays, gt, N=32, batch_size=1024, seed=1, world_size=world, **fine_kw)      # same seed argument on every rank
 ref = tr.flat_param.clone()
 dist.broadcast(ref, 0)
 res["replicas_identical_after_init"] = bool(torch.equal(tr.flat_param, ref))
