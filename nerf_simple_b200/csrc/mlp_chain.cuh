@@ -58,8 +58,10 @@ __device__ __forceinline__ uint32_t sw_off(const TileCtx& c, uint32_t kb, uint32
   return kb * 16384u + c.rowoff + ((j << 4) ^ c.r7s);
 }
 
-__device__ __forceinline__ void slot_barrier(int slot) {  // the 256 epilogue threads of one slot
-  asm volatile("bar.sync %0, 256;" ::"r"(slot + 1) : "memory");
+// the epilogue threads of one slot: 256 when two slots are in flight (named barrier slot + 1), else all 512 (barrier 1)
+template <int kSlots> __device__ __forceinline__ void epi_barrier(int slot) {
+  if (kSlots == 2) asm volatile("bar.sync %0, 256;" ::"r"(slot + 1) : "memory");
+  else asm volatile("bar.sync 1, 512;" ::: "memory");
 }
 
 // ---------------------------------------------------------------- compile-time slab schedule
@@ -85,6 +87,15 @@ template <int kTab, class Layout> __host__ __device__ constexpr auto& slab_table
   else return lay.bwd3;
 }
 template <int kTab> __host__ __device__ constexpr bool sched_is_bwd() { return kTab == kTabBwd || kTab == kTabBwdFold || kTab == kTabBwd3; }
+// A chain's loop index l -> the layer it runs (SlabDesc::ml of its slabs, checked in sched_classes_hold).
+// Forward chains: the MMA layer ml 0..9, whose output is saved tensor ml and whose biases are row bias_row; the folded
+// chain has no layers_2, so its loop index 8 is ml 9, with the bias row formed at pack time.  l = -1 is the tile prologue.
+template <int kTab> __host__ __device__ constexpr int fwd_layer(int l) { return kTab == kTabFwdFold && l == 8 ? 9 : l; }
+template <int kTab> __host__ __device__ constexpr int bias_row(int l) { return kTab == kTabFwdFold && l == 8 ? kFoldBiasRow : l; }
+// Delta chains: the backward layer bl 1..9, whose output is delta tensor bl; the folded chain starts at bl 2 (delta_h7
+// from delta_c1 in one layer).
+template <int kTab> __host__ __device__ __forceinline__ constexpr int bwd_layer(int l) { return l + (kTab == kTabBwdFold ? 2 : 1); }
+template <int kTab> __host__ __device__ constexpr int chain_layer(int l) { return sched_is_bwd<kTab>() ? bwd_layer<kTab>(l) : fwd_layer<kTab>(l); }
 // loop layer l = the l-th run of slabs closed by a `last` flag (the producer walks the table the same way)
 template <int kTab> __host__ __device__ constexpr int sched_first(int l) {
   int i = 0;
@@ -110,13 +121,14 @@ struct MmaRing { uint32_t stage, phase; };
 template <class Epi> __host__ __device__ constexpr int sched_class_rep(int l) {
   return sched_is_bwd<Epi::kTab>() ? (l == 0 ? 0 : 1) : ((l == 0 || l == 5 || l == Epi::kNumLayers - 1) ? l : 1);
 }
-// The table holds Epi::kNumLayers layers, and each has the slab list (as far as the issue code reads it) of its class
-// representative.
+// The table holds Epi::kNumLayers layers, each of them the layer chain_layer names, and each has the slab list (as far
+// as the issue code reads it) of its class representative.
 template <class Epi> constexpr bool sched_classes_hold() {
   int layers = 0;
   for (const SlabDesc& d : slab_table<Epi::kTab>(kLayout)) layers += d.last;
   if (layers != Epi::kNumLayers) return false;
   for (int l = 0; l < Epi::kNumLayers; ++l) {
+    if (sched_slab<Epi::kTab>(l, 0).ml != chain_layer<Epi::kTab>(l)) return false;
     const int rep = sched_class_rep<Epi>(l);
     if (sched_slabs<Epi::kTab>(l) != sched_slabs<Epi::kTab>(rep)) return false;
     for (int s = 0; s < sched_slabs<Epi::kTab>(l); ++s) {
@@ -197,7 +209,7 @@ __device__ __forceinline__ void issue_layer(uint32_t smem_base, uint32_t bar, ui
 template <class Epi>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kCThreads, 1)
 chain_kernel(const __grid_constant__ typename Epi::Params p) {
-  static_assert(sched_classes_hold<Epi>(), "a layer's slab list differs from its class representative's, or the table's layer count from the epilogue's");
+  static_assert(sched_classes_hold<Epi>(), "a layer's slab list differs from its class representative's, a layer from chain_layer's, or the table's layer count from the epilogue's");
   extern __shared__ __align__(1024) uint8_t chain_smem[];
   const uint32_t smem_base = smem_u32(chain_smem);
   if (smem_base & 1023u) {   // the SWIZZLE_128B images need it, and there is no slack left to round up
@@ -274,12 +286,12 @@ chain_kernel(const __grid_constant__ typename Epi::Params p) {
     // packed buffer's fp32 tail in global memory: coalesced and L2-resident, where 256 DIFFERENT constant-bank
     // addresses per slot serialise in the constant cache (~1,000 cycles per staged row).
     const uint32_t bias_t = threadIdx.x & 255u;
-    auto fetch_bias = [&](int l) -> float { return Epi::kStageBias ? __ldg(c.gf + kF32Bias + Epi::bias_row(l) * 256 + (int)bias_t) : 0.f; };
+    auto fetch_bias = [&](int l) -> float { return Epi::kStageBias ? __ldg(c.gf + kF32Bias + bias_row<Epi::kTab>(l) * 256 + (int)bias_t) : 0.f; };
     auto stage_bias = [&](float v) {
       if (!Epi::kStageBias) return;
-      if (Epi::kSlots == 2) slot_barrier(slot); else asm volatile("bar.sync 1, 512;" ::: "memory");
+      epi_barrier<Epi::kSlots>(slot);
       if (Epi::kSlots == 2 || threadIdx.x < 256u) asm volatile("st.shared.f32 [%0], %1;" ::"r"(c.b_img + bias_t * 4u), "f"(v) : "memory");
-      if (Epi::kSlots == 2) slot_barrier(slot); else asm volatile("bar.sync 1, 512;" ::: "memory");
+      epi_barrier<Epi::kSlots>(slot);
     };
     // before overwriting A[slot] / E[slot]: the bulk store of the previous image must have read it
     auto reclaim = [&]() {
@@ -527,7 +539,7 @@ __device__ __forceinline__ void composite_staged_ray(const FwdEpiParams& p, uint
   const uint32_t row0 = (uint32_t)(ray_local * N + lane * S);
 #pragma unroll
   for (int j = 0; j < S; ++j) {
-    asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(o[j].x), "=f"(o[j].y), "=f"(o[j].z), "=f"(o[j].w) : "r"(stage_o + (row0 + j) * 16u));
+    o[j] = ld_shared_f4(stage_o + (row0 + j) * 16u);
     asm volatile("ld.shared.f32 %0, [%1];" : "=f"(t[j]) : "r"(stage_t + (row0 + j) * 4u));
   }
   float rd[6];
@@ -587,9 +599,7 @@ __host__ __device__ constexpr uint32_t tab_off(uint32_t i) {
   return (i >> 4) * 128u + (((4u + ((i >> 2) & 3u)) ^ ((i >> 4) & 7u)) << 4) + (i & 3u) * 4u;
 }
 __device__ __forceinline__ float4 tab_ld4(uint32_t e_img, uint32_t i) {   // i % 4 == 0, warp-uniform
-  float4 v;
-  asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(e_img + tab_off(i)));
-  return v;
+  return ld_shared_f4(e_img + tab_off(i));
 }
 
 // 16 accumulator columns + their (staged) biases -> [ReLU] -> two 16-byte chunks of the next layer's bf16 A operand.
@@ -644,7 +654,7 @@ __device__ __forceinline__ void epi_cols16(const TileCtx& c, const uint32_t (&a)
 __device__ __forceinline__ void load_bias16(const TileCtx& c, int col0, float4 (&bq)[4]) {
 #pragma unroll
   for (int i = 0; i < 4; ++i)
-    asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(bq[i].x), "=f"(bq[i].y), "=f"(bq[i].z), "=f"(bq[i].w) : "r"(c.b_img + (uint32_t)(col0 + 4 * i) * 4u));
+    bq[i] = ld_shared_f4(c.b_img + (uint32_t)(col0 + 4 * i) * 4u);
 }
 template <bool kRelu, bool kSigma, bool kSave, int kHalf>
 __device__ __forceinline__ void epi_hidden_h(const TileCtx& c, float& sigma) {
@@ -677,6 +687,57 @@ __device__ __forceinline__ void epi_hidden(const TileCtx& c, float& sigma) {
 #undef tmem_ld16
 #endif
 
+// This thread's entry of ReLU-mask tensor t (mask layout: mlp_tc.cu): 16 bytes per (row, column half) for h0..h7, 8
+// bytes for c1 (t = 8).
+__device__ __forceinline__ size_t mask_entry_off(int t, int64_t T, const TileCtx& c) {
+  const size_t e = t == 8 ? 8 : 16;
+  return mask_tensor_off(t, T) + (size_t)c.tile * (256 * e) + ((size_t)(c.half * 128) + c.r) * e;
+}
+// bf16x3: the same entries behind the hi and lo data tensors, each split between the two threads of its column half
+// (part >> 1); part & 1 takes the upper half of the entry.
+__device__ __forceinline__ size_t mask_entry_off3(int t, int64_t T, const TileCtx& c) {
+  const size_t e = t == 8 ? 8 : 16;
+  return mask_tensor_off3(t, T) + (size_t)c.tile * (256 * e) + ((size_t)((c.part >> 1) * 128) + c.r) * e + (size_t)(c.part & 1) * (e / 2);
+}
+
+// The saved tensors a forward hand-off carries (saved layout: mlp_tc.cu).  The tile prologue's hand-off (ml = -1) carries
+// posx from E, the hand-off of MMA layer ml its output from A (h0..h7, g, c1 = tensor ml).  posd (tensor 11, from E)
+// leaves with the first hand-off published after it was encoded, the one of MMA layer kPosdMl:
+//   FwdEpi  encodes posd behind h5's hand-off (after_publish, while the slot waits for its next accumulator): kPosdMl = 6;
+//   FwdEpi3 encodes posd in front of layer 5's epilogue:                                                     kPosdMl = 5.
+// kX3: every tensor as its hi image (A[0] / E[0]) and its lo image (A[1] / E[1], stored behind the hi data tensors).
+template <int kPosdMl, bool kX3>
+__device__ __forceinline__ void store_saved(const FwdEpiParams& p, const TileCtx& c, int ml) {
+  const int64_t T = p.num_tiles;
+  uint8_t* lo = p.saved + kSavedDataTileBytes * (size_t)T;
+  auto put = [&](int t, uint32_t img, uint32_t img_lo) {
+    const size_t off = saved_tensor_off(t, T) + (size_t)c.tile * saved_tile_bytes(t);
+    tma_bulk_s2g(p.saved + off, img, (uint32_t)saved_tile_bytes(t));
+    if (kX3) tma_bulk_s2g(lo + off, img_lo, (uint32_t)saved_tile_bytes(t));
+  };
+  if (ml == -1) put(10, c.e_img, c.e_img + kEBytes);       // posx
+  else if (ml < 9) put(ml, c.a_img, c.a_img + kABytes);    // h0..h7, g
+  else put(9, c.a_img, c.a_img + kABytes);                 // c1
+  if (ml == kPosdMl) put(11, c.e_img, c.e_img + kEBytes);  // posd
+}
+
+struct FwdState {
+  float v[6];       // the query (point and view direction)
+  float sigma;      // this thread's share of the sigma head
+  float t;          // sample depth (fused render)
+  int64_t m_raw;
+  bool row_valid;
+};
+// the tile prologue of both forward chains, up to the encoding: this thread's row and its query (rows past M re-read
+// row M - 1 and are not written)
+template <bool kRender>
+__device__ __forceinline__ void fwd_begin_row(const FwdEpiParams& p, FwdState& st, const TileCtx& c) {
+  st.m_raw = c.tile * kTileM + c.r;
+  st.row_valid = st.m_raw < p.M;
+  load_query_chain<kRender>(p, st.row_valid ? st.m_raw : p.M - 1, st.v, st.t);
+  st.sigma = 0.f;
+}
+
 // kFold: layers_2 folded into color_fc.0 (mlp_tc.cu, top): the chain has 9 layers, loop index 8 is MMA layer 9.
 template <bool kSave, bool kRender = false, bool kFold = false>
 struct FwdEpi {
@@ -689,15 +750,7 @@ struct FwdEpi {
   static constexpr int kSlots = 2;
   static constexpr int kNumLayers = kFold ? kNumFoldLayers : kNumMmaLayers;
   static constexpr bool kReverseTiles = false;
-  __device__ static constexpr int ml_of(int l) { return (kFold && l == 8) ? 9 : l; }                 // loop index -> MMA layer
-  __device__ static constexpr int bias_row(int l) { return (kFold && l == 8) ? kFoldBiasRow : l; }
-  struct State {
-    float v[6];
-    float sigma;
-    float t;          // sample depth (fused render)
-    int64_t m_raw;
-    bool row_valid;
-  };
+  using State = FwdState;
   __device__ static void init_slot(const TileCtx&) {}
 
   __device__ static void prefetch(const Params&, State&, const TileCtx&, int) {}
@@ -707,7 +760,7 @@ struct FwdEpi {
   // this slot would otherwise idle until their next accumulator is ready, so the ~130 extra instructions per thread
   // and layer stay off the critical path (inside the epilogue they cost the kernel 11 %).
   __device__ static void after_publish(const Params& p, State& st, const TileCtx& c, int l) {
-    const int ml = ml_of(l);
+    const int ml = fwd_layer<kTab>(l);
     if (ml == 5) {
       // posx has been consumed by the skip layer's MMAs: the encoding buffer now carries posd (27 -> 64) for color_fc.0,
       // plus the head-weight table in the free half of its rows.  Done here, behind the hand-off of h5, so that it
@@ -725,7 +778,7 @@ struct FwdEpi {
     if (!kSave || ml < 0 || ml == 8) return;
     const int64_t T = p.num_tiles;
     if (ml < 8) {
-      uint8_t* row = p.saved + mask_tensor_off(ml, T) + (size_t)c.tile * 4096 + ((size_t)(c.half * 128) + c.r) * 16;
+      uint8_t* row = p.saved + mask_entry_off(ml, T, c);
       uint32_t m[4];                         // unrolled: no spills, the 16 LDS.128 in flight together (-5 % on the kernel)
 #pragma unroll
       for (int q = 0; q < 4; ++q) {          // 32 columns = 4 chunks of 16 B = one mask word
@@ -742,7 +795,7 @@ struct FwdEpi {
       }
       *reinterpret_cast<uint4*>(row) = make_uint4(m[0], m[1], m[2], m[3]);
     } else {   // ml == 9: c1, 64 columns per thread = K-block `half` of the image
-      uint8_t* row = p.saved + mask_tensor_off(8, T) + (size_t)c.tile * 2048 + ((size_t)(c.half * 128) + c.r) * 8;
+      uint8_t* row = p.saved + mask_entry_off(8, T, c);
       uint32_t m[2];
 #pragma unroll
       for (int q = 0; q < 2; ++q) {
@@ -762,27 +815,17 @@ struct FwdEpi {
   }
 
   __device__ static void begin_tile(const Params& p, State& st, const TileCtx& c) {
-    st.m_raw = c.tile * kTileM + c.r;
-    st.row_valid = st.m_raw < p.M;
-    load_query_chain<kRender>(p, st.row_valid ? st.m_raw : p.M - 1, st.v, st.t);
-    st.sigma = 0.f;
+    fwd_begin_row<kRender>(p, st, c);
     // posx -> E[slot] (K = 64); each half of the slot's threads stores 4 of the 8 16-byte chunks
     if (c.half == 0) encode_row<kLp, 0, 4>(st.v, c.e_img, c.r, nullptr);
     else encode_row<kLp, 4, 8>(st.v, c.e_img, c.r, nullptr);
   }
 
-  // one thread per slot, after the slot barrier: tile images shared -> global (saved activations)
-  __device__ static void store_tile(const Params& p, const TileCtx& c, int l) {
-    const int64_t T = p.num_tiles;
-    const int ml = ml_of(l);
-    if (ml == -1) tma_bulk_s2g(p.saved + saved_tensor_off(10, T) + (size_t)c.tile * 16384, c.e_img, 16384);        // posx
-    else if (ml < 9) tma_bulk_s2g(p.saved + saved_tensor_off(ml, T) + (size_t)c.tile * 65536, c.a_img, 65536);    // h0..h7, g
-    else tma_bulk_s2g(p.saved + saved_tensor_off(9, T) + (size_t)c.tile * 32768, c.a_img, 32768);                  // c1
-    if (ml == 6) tma_bulk_s2g(p.saved + saved_tensor_off(11, T) + (size_t)c.tile * 16384, c.e_img, 16384);         // posd (encoded behind h5's hand-off)
-  }
+  // the store warp: the saved tensors of hand-off l
+  __device__ static void store_tile(const Params& p, const TileCtx& c, int l) { store_saved<6, false>(p, c, fwd_layer<kTab>(l)); }
 
   __device__ static void layer(const Params& p, State& st, const TileCtx& c, int l) {
-    const int ml = ml_of(l);
+    const int ml = fwd_layer<kTab>(l);
     if (ml < 9) {
       if (ml == 7) epi_hidden<true, true, kSave>(c, st.sigma);
       else if (ml == 8) epi_hidden<false, false, kSave>(c, st.sigma);  // layers_2: no act.
@@ -799,9 +842,9 @@ struct FwdEpi {
         tmem_ld_wait();
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
-          float x[8], b[8];
-          asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(b[0]), "=f"(b[1]), "=f"(b[2]), "=f"(b[3]) : "r"(c.b_img + (uint32_t)(col0 + 8 * j) * 4u));
-          asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(b[4]), "=f"(b[5]), "=f"(b[6]), "=f"(b[7]) : "r"(c.b_img + (uint32_t)(col0 + 8 * j + 4) * 4u));
+          const float4 b0 = ld_shared_f4(c.b_img + (uint32_t)(col0 + 8 * j) * 4u), b1 = ld_shared_f4(c.b_img + (uint32_t)(col0 + 8 * j + 4) * 4u);
+          const float b[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+          float x[8];
 #pragma unroll
           for (int e = 0; e < 8; ++e) x[e] = fmaxf(__uint_as_float(a[8 * j + e]) + b[e], 0.f);
 #pragma unroll
@@ -819,10 +862,9 @@ struct FwdEpi {
       }
       const uint32_t xaddr = c.e_img + c.r * 16u;
       if (c.half == 1) st_shared_v4(xaddr, __float_as_uint(rgb[0]), __float_as_uint(rgb[1]), __float_as_uint(rgb[2]), __float_as_uint(st.sigma));
-      slot_barrier(c.slot);
+      epi_barrier<kSlots>(c.slot);
       if (c.half == 0) {
-        float4 o;
-        asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(o.x), "=f"(o.y), "=f"(o.z), "=f"(o.w) : "r"(xaddr));
+        const float4 o = ld_shared_f4(xaddr);
         const float4 hb = tab_ld4(c.e_img, kTabBC1);   // color_fc.2's bias, sigma_fc's bias
         const float4 res = make_float4(rgb[0] + o.x + hb.x, rgb[1] + o.y + hb.y, rgb[2] + o.z + hb.z, st.sigma + o.w + hb.w);  // (r,g,b,sigma), utils/nets.py:43
         if (kRender) {
@@ -835,7 +877,7 @@ struct FwdEpi {
           reinterpret_cast<float4*>(p.out)[st.m_raw] = res;
         }
       }
-      slot_barrier(c.slot);  // E[slot] may be re-encoded for the next tile only after the exchange was read
+      epi_barrier<kSlots>(c.slot);  // E[slot] may be re-encoded for the next tile only after the exchange was read
       if (kRender) {
         const int wq = (int)(threadIdx.x >> 5) & 7, nr = kTileM / p.N;   // warp wq composites ray wq of the tile
         const int64_t ray = c.tile * nr + wq;
@@ -903,29 +945,13 @@ struct FwdEpi3 {
   static constexpr int kSlots = 1;
   static constexpr int kNumLayers = kNumMmaLayers;
   static constexpr bool kReverseTiles = false;
-  struct State {
-    float v[6];
-    float sigma;      // this thread's share (64 columns) of the sigma head
-    int64_t m_raw;
-    bool row_valid;
-  };
-  __device__ static constexpr int bias_row(int l) { return l; }
+  using State = FwdState;
   __device__ static void init_slot(const TileCtx&) {}
   __device__ static void prefetch(const Params&, State&, const TileCtx&, int) {}
   __device__ static void after_publish(const Params&, State&, const TileCtx&, int) {}
-  // the store warp: layer l's hand-off (l = -1: posx; 0..8: h0..h7, g; 9: c1; posd rides on h5) as hi and lo images
+  // the store warp: the saved tensors of hand-off l, hi and lo images
   __device__ static void store_tile(const Params& p, const TileCtx& c, int l) {
-    if (!kSave) return;
-    const int64_t T = p.num_tiles;
-    uint8_t* lo = p.saved + kSavedDataTileBytes * (size_t)T;
-    auto put = [&](int t, uint32_t img, uint32_t img_lo) {
-      const size_t off = saved_tensor_off(t, T) + (size_t)c.tile * saved_tile_bytes(t);
-      tma_bulk_s2g(p.saved + off, img, (uint32_t)saved_tile_bytes(t));
-      tma_bulk_s2g(lo + off, img_lo, (uint32_t)saved_tile_bytes(t));
-    };
-    if (l == -1) put(10, c.e_img, c.e_img + kEBytes);
-    else put(l, c.a_img, c.a_img + kABytes);
-    if (l == 5) put(11, c.e_img, c.e_img + kEBytes);   // posd, encoded in front of h5's epilogue
+    if (kSave) store_saved<5, true>(p, c, fwd_layer<kTab>(l));
   }
 
   __device__ static void encode(const float* x, const TileCtx& c, bool dirs) {
@@ -944,15 +970,12 @@ struct FwdEpi3 {
   }
 
   __device__ static void begin_tile(const Params& p, State& st, const TileCtx& c) {
-    st.m_raw = c.tile * kTileM + c.r;
-    st.row_valid = st.m_raw < p.M;
-    float t;
-    load_query_chain<false>(p, st.row_valid ? st.m_raw : p.M - 1, st.v, t);
-    st.sigma = 0.f;
+    fwd_begin_row<false>(p, st, c);
     encode(st.v, c, false);
   }
 
-  __device__ static void layer(const Params& p, State& st, const TileCtx& c, int ml) {
+  __device__ static void layer(const Params& p, State& st, const TileCtx& c, int l) {
+    const int ml = fwd_layer<kTab>(l);
     if (ml == 5) encode(st.v + 3, c, true);   // posx consumed by the skip layer: the encoding buffers now carry posd
     const uint32_t a_hi = c.a_img, a_lo = c.a_img + kABytes;
     if (ml < 9) {
@@ -997,9 +1020,7 @@ struct FwdEpi3 {
           st_shared_v4(a_lo + o, l[0], l[1], l[2], l[3]);
         }
       }
-      if (kSave && ml != 8)   // 8 of the 16 bytes of the (row, column half) entry of mask tensor ml
-        *reinterpret_cast<uint2*>(p.saved + mask_tensor_off3(ml, p.num_tiles) + (size_t)c.tile * 4096 +
-                                  ((size_t)((c.part >> 1) * 128) + c.r) * 16 + (size_t)(c.part & 1) * 8) = make_uint2(mbits[0], mbits[1]);
+      if (kSave && ml != 8) *reinterpret_cast<uint2*>(p.saved + mask_entry_off3(ml, p.num_tiles, c)) = make_uint2(mbits[0], mbits[1]);
     } else {
       // color_fc.0 epilogue (128 columns, 32 per thread, ReLU) + color_fc.2 (128 -> 3) in fp32 on CUDA cores; the four
       // threads of a row meet through the (now free) encoding buffer
@@ -1040,34 +1061,66 @@ struct FwdEpi3 {
           }
         }
       }
-      if (kSave)   // 4 of the 8 bytes of the (row, column half) entry of mask tensor 8
-        *reinterpret_cast<uint32_t*>(p.saved + mask_tensor_off3(8, p.num_tiles) + (size_t)c.tile * 2048 +
-                                     ((size_t)((c.part >> 1) * 128) + c.r) * 8 + (size_t)(c.part & 1) * 4) = mword;
+      if (kSave) *reinterpret_cast<uint32_t*>(p.saved + mask_entry_off3(8, p.num_tiles, c)) = mword;
       const uint32_t xaddr = c.e_img + ((uint32_t)c.part * 128u + c.r) * 16u;
       if (c.part != 0) st_shared_v4(xaddr, __float_as_uint(rgb[0]), __float_as_uint(rgb[1]), __float_as_uint(rgb[2]), __float_as_uint(st.sigma));
-      asm volatile("bar.sync 1, 512;" ::: "memory");
+      epi_barrier<kSlots>(c.slot);
       if (c.part == 0) {
         float4 acc = make_float4(rgb[0], rgb[1], rgb[2], st.sigma);
 #pragma unroll
         for (int q = 1; q < 4; ++q) {
-          float4 o;
-          asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(o.x), "=f"(o.y), "=f"(o.z), "=f"(o.w) : "r"(c.e_img + ((uint32_t)q * 128u + c.r) * 16u));
+          const float4 o = ld_shared_f4(c.e_img + ((uint32_t)q * 128u + c.r) * 16u);
           acc.x += o.x; acc.y += o.y; acc.z += o.z; acc.w += o.w;
         }
         if (st.row_valid)
           reinterpret_cast<float4*>(p.out)[st.m_raw] = make_float4(acc.x + __ldg(c.gf + kF32BC1), acc.y + __ldg(c.gf + kF32BC1 + 1), acc.z + __ldg(c.gf + kF32BC1 + 2),
                                                                    acc.w + __ldg(c.gf + kF32BSig));   // (r,g,b,sigma), utils/nets.py:43
       }
-      asm volatile("bar.sync 1, 512;" ::: "memory");   // the encoding buffers may be rewritten for the next tile
+      epi_barrier<kSlots>(c.slot);   // the encoding buffers may be rewritten for the next tile
     }
   }
 };
 
 // ======================================================================= backward (dgrad)
-#ifndef NB_DG_L2HINT
-#define NB_DG_L2HINT 2   // bit 1: delta stores evict_first (511 -> 501 us).  bit 0 (mask prefetch evict_last, -6 us more) is off:
-                          // the evict_last lines outlive the kernel and made the first render after training 2x slower
-#endif
+// The delta chains have no use for the encoding buffers: E[slot] holds w_sigma (floats 0..255) and color_fc.2's weight
+// Wc1 [3][128] (256..639) for the whole kernel, read with warp-uniform LDS.128 instead of constant-bank loads.  Staged
+// once per kernel by the slot's 512 / kSlots epilogue threads.
+template <int kSlots> __device__ __forceinline__ void stage_head_weights(const TileCtx& c) {
+  for (uint32_t i = kSlots == 2 ? threadIdx.x & 255u : threadIdx.x; i < 640u; i += 512u / kSlots)
+    asm volatile("st.shared.f32 [%0], %1;" ::"r"(c.e_img + i * 4u), "f"(__ldg(c.gf + (i < 256u ? kF32WSig + (int)i : kF32WC1 + (int)(i - 256u)))) : "memory");
+  epi_barrier<kSlots>(c.slot);
+}
+// delta_c1 of the 8 columns [col, col + 8) before its ReLU mask: d_rgb @ Wc1 (color_fc.2 backward, 3 -> 128)
+__device__ __forceinline__ void head_dc1(const float4& g, uint32_t e_img, uint32_t col, float (&x)[8]) {
+  const float4 a0 = ld_shared_f4(e_img + (256u + col) * 4u), a1 = ld_shared_f4(e_img + (256u + col + 4u) * 4u);
+  x[0] = g.x * a0.x; x[1] = g.x * a0.y; x[2] = g.x * a0.z; x[3] = g.x * a0.w;
+  x[4] = g.x * a1.x; x[5] = g.x * a1.y; x[6] = g.x * a1.z; x[7] = g.x * a1.w;
+  const float4 b0 = ld_shared_f4(e_img + (384u + col) * 4u), b1 = ld_shared_f4(e_img + (384u + col + 4u) * 4u);
+  x[0] = fmaf(g.y, b0.x, x[0]); x[1] = fmaf(g.y, b0.y, x[1]); x[2] = fmaf(g.y, b0.z, x[2]); x[3] = fmaf(g.y, b0.w, x[3]);
+  x[4] = fmaf(g.y, b1.x, x[4]); x[5] = fmaf(g.y, b1.y, x[5]); x[6] = fmaf(g.y, b1.z, x[6]); x[7] = fmaf(g.y, b1.w, x[7]);
+  const float4 c0 = ld_shared_f4(e_img + (512u + col) * 4u), c1 = ld_shared_f4(e_img + (512u + col + 4u) * 4u);
+  x[0] = fmaf(g.z, c0.x, x[0]); x[1] = fmaf(g.z, c0.y, x[1]); x[2] = fmaf(g.z, c0.z, x[2]); x[3] = fmaf(g.z, c0.w, x[3]);
+  x[4] = fmaf(g.z, c1.x, x[4]); x[5] = fmaf(g.z, c1.y, x[5]); x[6] = fmaf(g.z, c1.z, x[6]); x[7] = fmaf(g.z, c1.w, x[7]);
+}
+// + d_sigma * w_sigma[col .. col + 8) on the 8 deltas of h7's columns [col, col + 8) (the sigma head reads h7)
+__device__ __forceinline__ void add_sigma_term(float gsig, uint32_t e_img, int col, float (&x)[8]) {
+  const float4 s0 = ld_shared_f4(e_img + (uint32_t)col * 4u), s1 = ld_shared_f4(e_img + (uint32_t)(col + 4) * 4u);
+  x[0] = fmaf(gsig, s0.x, x[0]); x[1] = fmaf(gsig, s0.y, x[1]); x[2] = fmaf(gsig, s0.z, x[2]); x[3] = fmaf(gsig, s0.w, x[3]);
+  x[4] = fmaf(gsig, s1.x, x[4]); x[5] = fmaf(gsig, s1.y, x[5]); x[6] = fmaf(gsig, s1.z, x[6]); x[7] = fmaf(gsig, s1.w, x[7]);
+}
+// The store warp: the delta image of hand-off l -> delta tensor t = l < 0 ? 0 (delta_c1, the tile prologue) : bl, read back
+// by wgrad.  kX3: the hi image from A[0] and the lo image from A[1], behind the hi tensors.  The stores carry the
+// evict-first L2 policy (511 -> 501 us per delta chain); evict-last on the mask loads gained 6 us more but was dropped:
+// its lines outlive the kernel and made the first render after training 2x slower.
+template <bool kX3> __device__ __forceinline__ void store_delta(const BwdParams& p, const TileCtx& c, int t) {
+  const int64_t T = p.num_tiles;
+  const uint64_t pol = l2_policy_evict_first();
+  const uint32_t bytes = delta_tile_bytes(t);
+  const size_t off = delta_tensor_off(t, T) + (size_t)c.tile * bytes;
+  tma_bulk_s2g_hint(p.dscr + off, c.a_img, bytes, pol);
+  if (kX3) tma_bulk_s2g_hint(p.dscr + kDeltaTileBytes * (size_t)T + off, c.a_img + kABytes, bytes, pol);
+}
+
 // kFold: delta_h7 = delta_c1 Wf in ONE layer (mlp_tc.cu, top): 8 MMA layers, loop index l is bl = l + 2.
 template <bool kFold>
 struct DgradEpi {
@@ -1078,33 +1131,18 @@ struct DgradEpi {
   static constexpr bool kStageBias = false;
   static constexpr int kSlots = 2;
   static constexpr int kNumLayers = kFold ? 8 : 9;  // bl = 1..9 (folded: 2..9)
-  static constexpr int kBl0 = kFold ? 2 : 1;        // bl of loop index 0
   static constexpr bool kReverseTiles = true;
   struct State { float4 g; uint4 mask; };
-  __device__ static constexpr int bias_row(int l) { return l; }
   __device__ static void after_publish(const Params&, State&, const TileCtx&, int) {}
-  // The delta chain has no use for the encoding buffers: E[slot] holds w_sigma (floats 0..255) and color_fc.2's weight
-  // (256..639) for the whole kernel, read with warp-uniform LDS.128 instead of constant-bank loads.
-  __device__ static void init_slot(const TileCtx& c) {
-    for (uint32_t i = threadIdx.x & 255u; i < 640u; i += 256u)
-      asm volatile("st.shared.f32 [%0], %1;" ::"r"(c.e_img + i * 4u), "f"(__ldg(c.gf + (i < 256u ? kF32WSig + (int)i : kF32WC1 + (int)(i - 256u)))) : "memory");
-    slot_barrier(c.slot);
-  }
-  __device__ static __forceinline__ float4 head_ld4(const TileCtx& c, uint32_t i) {   // i % 4 == 0, warp-uniform
-    float4 v;
-    asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(c.e_img + i * 4u));
-    return v;
-  }
+  __device__ static void init_slot(const TileCtx& c) { stage_head_weights<kSlots>(c); }
 
   // The ReLU mask of layer l is this thread's 16-byte row of the bit-mask tensor the forward pass wrote (one bit per
   // element instead of the 64 KB bf16 activation tile): ONE load per thread and layer, issued before the accumulator
   // wait, so its latency is off the epilogue's critical path (the per-thread loads of the activation tile used to
   // account for 25 % of the kernel's stall samples, and for 1.1 GB of DRAM reads per step).
   __device__ static void prefetch(const Params& p, State& st, const TileCtx& c, int l) {
-    const int bl = l + kBl0;    // masks with h_{9-bl}: bl=2 -> h7, ..., bl=9 -> h0; bl=1 yields delta_g (no activation)
-    if (bl >= 2)
-      st.mask = __ldg(reinterpret_cast<const uint4*>(p.saved + mask_tensor_off(9 - bl, p.num_tiles) + (size_t)c.tile * 4096 +
-                                                     ((size_t)(c.half * 128) + c.r) * 16));
+    const int bl = bwd_layer<kTab>(l);   // masks with h_{9-bl}: bl=2 -> h7, ..., bl=9 -> h0; bl=1 yields delta_g (no activation)
+    if (bl >= 2) st.mask = __ldg(reinterpret_cast<const uint4*>(p.saved + mask_entry_off(9 - bl, p.num_tiles, c)));
   }
 
   __device__ static void begin_tile(const Params& p, State& st, const TileCtx& c) {
@@ -1113,8 +1151,7 @@ struct DgradEpi {
     st.g = make_float4(0.f, 0.f, 0.f, 0.f);  // rows past M carry zero gradient
     if (m_raw < p.M) st.g = __ldg(reinterpret_cast<const float4*>(p.d_out) + m_raw);
     // delta_c1 = (d_rgb @ Wc1) * (c1 > 0)   (color_fc.2 backward, 3 -> 128, CUDA cores)
-    const uint2 cbits = __ldg(reinterpret_cast<const uint2*>(p.saved + mask_tensor_off(8, T) + (size_t)c.tile * 2048 +
-                                                             ((size_t)(c.half * 128) + c.r) * 8));
+    const uint2 cbits = __ldg(reinterpret_cast<const uint2*>(p.saved + mask_entry_off(8, T, c)));
     const uint32_t kb = (uint32_t)c.half;  // 128 columns: each half of the slot's threads takes 64
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
@@ -1122,37 +1159,15 @@ struct DgradEpi {
       // 8 columns = pairs 4*(j&1) .. +3 of the 16-column step j/2; steps 0,1 in cbits.x, 2,3 in cbits.y
       const uint32_t field = ((j < 4 ? cbits.x : cbits.y) >> (16 * ((j >> 1) & 1))) & 0xFFFFu;
       const int k0 = 4 * (j & 1);
-      const uint32_t col = (uint32_t)(c.half * 64 + j * 8);
       float x[8];
-      {
-        const float4 a0 = head_ld4(c, 256u + col), a1 = head_ld4(c, 256u + col + 4u);
-        x[0] = st.g.x * a0.x; x[1] = st.g.x * a0.y; x[2] = st.g.x * a0.z; x[3] = st.g.x * a0.w;
-        x[4] = st.g.x * a1.x; x[5] = st.g.x * a1.y; x[6] = st.g.x * a1.z; x[7] = st.g.x * a1.w;
-        const float4 b0 = head_ld4(c, 384u + col), b1 = head_ld4(c, 384u + col + 4u);
-        x[0] = fmaf(st.g.y, b0.x, x[0]); x[1] = fmaf(st.g.y, b0.y, x[1]); x[2] = fmaf(st.g.y, b0.z, x[2]); x[3] = fmaf(st.g.y, b0.w, x[3]);
-        x[4] = fmaf(st.g.y, b1.x, x[4]); x[5] = fmaf(st.g.y, b1.y, x[5]); x[6] = fmaf(st.g.y, b1.z, x[6]); x[7] = fmaf(st.g.y, b1.w, x[7]);
-        const float4 c0 = head_ld4(c, 512u + col), c1 = head_ld4(c, 512u + col + 4u);
-        x[0] = fmaf(st.g.z, c0.x, x[0]); x[1] = fmaf(st.g.z, c0.y, x[1]); x[2] = fmaf(st.g.z, c0.z, x[2]); x[3] = fmaf(st.g.z, c0.w, x[3]);
-        x[4] = fmaf(st.g.z, c1.x, x[4]); x[5] = fmaf(st.g.z, c1.y, x[5]); x[6] = fmaf(st.g.z, c1.z, x[6]); x[7] = fmaf(st.g.z, c1.w, x[7]);
-      }
+      head_dc1(st.g, c.e_img, (uint32_t)(c.half * 64 + j * 8), x);
       const uint32_t w0 = pack_bf16x2(x[0], x[1]) & pair_mask_word(field, k0), w1 = pack_bf16x2(x[2], x[3]) & pair_mask_word(field, k0 + 1),
                      w2 = pack_bf16x2(x[4], x[5]) & pair_mask_word(field, k0 + 2), w3 = pack_bf16x2(x[6], x[7]) & pair_mask_word(field, k0 + 3);
       st_shared_v4(c.a_img + o, w0, w1, w2, w3);
     }
   }
 
-  // one thread per slot: delta tile image shared -> global (read back by wgrad)
-  __device__ static void store_tile(const Params& p, const TileCtx& c, int l) {
-    const int64_t T = p.num_tiles;
-#if NB_DG_L2HINT & 2
-    const uint64_t pol = l2_policy_evict_first();
-    if (l == -1) tma_bulk_s2g_hint(p.dscr + delta_tensor_off(0, T) + (size_t)c.tile * 32768, c.a_img, 32768, pol);   // delta_c1
-    else tma_bulk_s2g_hint(p.dscr + delta_tensor_off(l + kBl0, T) + (size_t)c.tile * 65536, c.a_img, 65536, pol);
-#else
-    if (l == -1) tma_bulk_s2g(p.dscr + delta_tensor_off(0, T) + (size_t)c.tile * 32768, c.a_img, 32768);   // delta_c1
-    else tma_bulk_s2g(p.dscr + delta_tensor_off(l + kBl0, T) + (size_t)c.tile * 65536, c.a_img, 65536);
-#endif
-  }
+  __device__ static void store_tile(const Params& p, const TileCtx& c, int l) { store_delta<false>(p, c, l < 0 ? 0 : bwd_layer<kTab>(l)); }
 
   // 16 accumulator columns -> masked bf16 delta chunk pair in A[slot] (the next layer's A operand and wgrad's operand)
   template <bool kMasked, bool kSigma>
@@ -1163,11 +1178,7 @@ struct DgradEpi {
       float x[8];
 #pragma unroll
       for (int e = 0; e < 8; ++e) x[e] = __uint_as_float(a[8 * j + e]);
-      if (kSigma) {   // + d_sigma * w_sigma (sigma head reads h7)
-        const float4 s0 = head_ld4(c, (uint32_t)(col0 + 8 * j)), s1 = head_ld4(c, (uint32_t)(col0 + 8 * j + 4));
-        x[0] = fmaf(gsig, s0.x, x[0]); x[1] = fmaf(gsig, s0.y, x[1]); x[2] = fmaf(gsig, s0.z, x[2]); x[3] = fmaf(gsig, s0.w, x[3]);
-        x[4] = fmaf(gsig, s1.x, x[4]); x[5] = fmaf(gsig, s1.y, x[5]); x[6] = fmaf(gsig, s1.z, x[6]); x[7] = fmaf(gsig, s1.w, x[7]);
-      }
+      if (kSigma) add_sigma_term(gsig, c.e_img, col0 + 8 * j, x);
       uint32_t w0 = pack_bf16x2(x[0], x[1]), w1 = pack_bf16x2(x[2], x[3]), w2 = pack_bf16x2(x[4], x[5]),
                w3 = pack_bf16x2(x[6], x[7]);
       if (kMasked) {
@@ -1198,7 +1209,7 @@ struct DgradEpi {
 
   __device__ static void layer(const Params&, State& st, const TileCtx& c, int l) {
     // ReLU mask (bit per element, loaded in prefetch): bl=2 -> h7, ..., bl=9 -> h0; bl=1 yields delta_g (no activation)
-    const int bl = l + kBl0;
+    const int bl = bwd_layer<kTab>(l);
     if (bl == 1) layer_t<false, false>(st, c);
     else if (bl == 2) layer_t<true, true>(st, c);
     else layer_t<true, false>(st, c);
@@ -1221,25 +1232,12 @@ struct DgradEpi3 {
   static constexpr int kNumLayers = 9;   // bl = 1..9
   static constexpr bool kReverseTiles = true;
   struct State { float4 g; uint2 mask; };
-  __device__ static constexpr int bias_row(int l) { return l; }
   __device__ static void after_publish(const Params&, State&, const TileCtx&, int) {}
-  // E[0] holds w_sigma (floats 0..255) and color_fc.2's weight (256..639) for the whole kernel
-  __device__ static void init_slot(const TileCtx& c) {
-    for (uint32_t i = threadIdx.x; i < 640u; i += 512u)
-      asm volatile("st.shared.f32 [%0], %1;" ::"r"(c.e_img + i * 4u), "f"(__ldg(c.gf + (i < 256u ? kF32WSig + (int)i : kF32WC1 + (int)(i - 256u)))) : "memory");
-    asm volatile("bar.sync 1, 512;" ::: "memory");
-  }
-  __device__ static __forceinline__ float4 head_ld4(const TileCtx& c, uint32_t i) {
-    float4 v;
-    asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(c.e_img + i * 4u));
-    return v;
-  }
+  __device__ static void init_slot(const TileCtx& c) { stage_head_weights<kSlots>(c); }
   // this thread's 8 bytes (64 columns) of the (row, column half) entry of a mask tensor
   __device__ static void prefetch(const Params& p, State& st, const TileCtx& c, int l) {
-    const int bl = l + 1;   // bl=2 -> h7, ..., bl=9 -> h0; bl=1 yields delta_g (no activation)
-    if (bl >= 2)
-      st.mask = __ldg(reinterpret_cast<const uint2*>(p.saved + mask_tensor_off3(9 - bl, p.num_tiles) + (size_t)c.tile * 4096 +
-                                                     ((size_t)((c.part >> 1) * 128) + c.r) * 16 + (size_t)(c.part & 1) * 8));
+    const int bl = bwd_layer<kTab>(l);   // bl=2 -> h7, ..., bl=9 -> h0; bl=1 yields delta_g (no activation)
+    if (bl >= 2) st.mask = __ldg(reinterpret_cast<const uint2*>(p.saved + mask_entry_off3(9 - bl, p.num_tiles, c)));
   }
 
   __device__ static void begin_tile(const Params& p, State& st, const TileCtx& c) {
@@ -1248,23 +1246,13 @@ struct DgradEpi3 {
     st.g = make_float4(0.f, 0.f, 0.f, 0.f);  // rows past M carry zero gradient
     if (m_raw < p.M) st.g = __ldg(reinterpret_cast<const float4*>(p.d_out) + m_raw);
     // delta_c1 = (d_rgb @ Wc1) * (c1 > 0) in fp32: this thread's 32 of the 128 columns
-    const uint32_t cbits = __ldg(reinterpret_cast<const uint32_t*>(p.saved + mask_tensor_off3(8, T) + (size_t)c.tile * 2048 +
-                                                                   ((size_t)((c.part >> 1) * 128) + c.r) * 8 + (size_t)(c.part & 1) * 4));
+    const uint32_t cbits = __ldg(reinterpret_cast<const uint32_t*>(p.saved + mask_entry_off3(8, T, c)));
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-      const uint32_t col = (uint32_t)(c.part * 32 + j * 8);
       const uint32_t field = (cbits >> (16 * (j >> 1))) & 0xFFFFu;
       const int k0 = 4 * (j & 1);
       float x[8];
-      const float4 a0 = head_ld4(c, 256u + col), a1 = head_ld4(c, 256u + col + 4u);
-      x[0] = st.g.x * a0.x; x[1] = st.g.x * a0.y; x[2] = st.g.x * a0.z; x[3] = st.g.x * a0.w;
-      x[4] = st.g.x * a1.x; x[5] = st.g.x * a1.y; x[6] = st.g.x * a1.z; x[7] = st.g.x * a1.w;
-      const float4 b0 = head_ld4(c, 384u + col), b1 = head_ld4(c, 384u + col + 4u);
-      x[0] = fmaf(st.g.y, b0.x, x[0]); x[1] = fmaf(st.g.y, b0.y, x[1]); x[2] = fmaf(st.g.y, b0.z, x[2]); x[3] = fmaf(st.g.y, b0.w, x[3]);
-      x[4] = fmaf(st.g.y, b1.x, x[4]); x[5] = fmaf(st.g.y, b1.y, x[5]); x[6] = fmaf(st.g.y, b1.z, x[6]); x[7] = fmaf(st.g.y, b1.w, x[7]);
-      const float4 c0 = head_ld4(c, 512u + col), c1 = head_ld4(c, 512u + col + 4u);
-      x[0] = fmaf(st.g.z, c0.x, x[0]); x[1] = fmaf(st.g.z, c0.y, x[1]); x[2] = fmaf(st.g.z, c0.z, x[2]); x[3] = fmaf(st.g.z, c0.w, x[3]);
-      x[4] = fmaf(st.g.z, c1.x, x[4]); x[5] = fmaf(st.g.z, c1.y, x[5]); x[6] = fmaf(st.g.z, c1.z, x[6]); x[7] = fmaf(st.g.z, c1.w, x[7]);
+      head_dc1(st.g, c.e_img, (uint32_t)(c.part * 32 + j * 8), x);
       uint32_t h[4], l[4];
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
@@ -1278,18 +1266,10 @@ struct DgradEpi3 {
     }
   }
 
-  // the store warp: delta tile images (hi from A[0], lo from A[1]) -> scratch, read back by wgrad
-  __device__ static void store_tile(const Params& p, const TileCtx& c, int l) {
-    const int64_t T = p.num_tiles;
-    const uint64_t pol = l2_policy_evict_first();
-    const uint32_t bytes = l == -1 ? 32768u : 65536u;
-    const size_t off = delta_tensor_off(l + 1, T) + (size_t)c.tile * bytes;   // l = -1: delta_c1 (tensor 0)
-    tma_bulk_s2g_hint(p.dscr + off, c.a_img, bytes, pol);
-    tma_bulk_s2g_hint(p.dscr + kDeltaTileBytes * (size_t)T + off, c.a_img + kABytes, bytes, pol);
-  }
+  __device__ static void store_tile(const Params& p, const TileCtx& c, int l) { store_delta<true>(p, c, l < 0 ? 0 : bwd_layer<kTab>(l)); }
 
   __device__ static void layer(const Params&, State& st, const TileCtx& c, int l) {
-    const int bl = l + 1;
+    const int bl = bwd_layer<kTab>(l);
     const int cbase = c.part * 64;
 #pragma unroll 1
     for (int q = 0; q < 4; ++q) {
@@ -1303,11 +1283,7 @@ struct DgradEpi3 {
         float x[8];
 #pragma unroll
         for (int e = 0; e < 8; ++e) x[e] = __uint_as_float(a[8 * j + e]);
-        if (bl == 2) {   // + d_sigma * w_sigma (the sigma head reads h7)
-          const float4 s0 = head_ld4(c, (uint32_t)(col0 + 8 * j)), s1 = head_ld4(c, (uint32_t)(col0 + 8 * j + 4));
-          x[0] = fmaf(st.g.w, s0.x, x[0]); x[1] = fmaf(st.g.w, s0.y, x[1]); x[2] = fmaf(st.g.w, s0.z, x[2]); x[3] = fmaf(st.g.w, s0.w, x[3]);
-          x[4] = fmaf(st.g.w, s1.x, x[4]); x[5] = fmaf(st.g.w, s1.y, x[5]); x[6] = fmaf(st.g.w, s1.z, x[6]); x[7] = fmaf(st.g.w, s1.w, x[7]);
-        }
+        if (bl == 2) add_sigma_term(st.g.w, c.e_img, col0 + 8 * j, x);
         uint32_t h[4], lo[4];
 #pragma unroll
         for (int e = 0; e < 4; ++e) {

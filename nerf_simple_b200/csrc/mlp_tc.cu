@@ -681,7 +681,7 @@ int tc_render(int precision, const float* rays, const float* poses, int H, int W
 static void wgrad_item(WItem& w, const uint8_t* ds, const uint8_t* sv, int64_t T, float* pad, float* const* G, int dt, int st,
                        int layer, int ldw, int col0, int ncols, int nrows, bool bias) {
   w.a_ptr = ds + delta_tensor_off(dt, T);
-  w.a_tile_bytes = dt == 0 ? 32768u : 65536u;
+  w.a_tile_bytes = delta_tile_bytes(dt);
   w.a_chunks = dt == 0 ? 2 : 4;
   w.b_ptr = sv + saved_tensor_off(st, T);
   w.b_tile_bytes = (uint32_t)saved_tile_bytes(st);

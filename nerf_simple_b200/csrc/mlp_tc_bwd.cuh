@@ -15,12 +15,13 @@
 //       cores) while h7 / c1 are staged, so the heads need no pass of their own.
 
 // ------------------------------------------------------------------ delta scratch layout
-// tensor 0 = delta_c1 (128 cols, 32 KB/tile); tensors 1..9 = delta_g, delta_h7, ..., delta_h0 (64 KB/tile).
-// The folded chain keeps this layout and leaves tensor 1 unwritten.
+// tensor 0 = delta_c1 (128 cols, 32 KB/tile); tensors 1..9 = delta_g, delta_h7, ..., delta_h0 (64 KB/tile): tensor bl
+// is the output of the delta chain's layer bl.  The folded chain keeps this layout and leaves tensor 1 unwritten.
 constexpr size_t kDeltaTileBytes = 32768 + 9 * 65536;
 __host__ __device__ __forceinline__ size_t delta_tensor_off(int t, int64_t num_tiles) {
   return (t == 0 ? (size_t)0 : (size_t)32768 + (size_t)(t - 1) * 65536) * (size_t)num_tiles;
 }
+__host__ __device__ __forceinline__ uint32_t delta_tile_bytes(int t) { return t == 0 ? 32768u : 65536u; }
 
 struct BwdParams {
   CUtensorMap tmap128, tmap64;
@@ -32,14 +33,6 @@ struct BwdParams {
   const float* d_out;  // [M,4]
   uint8_t* dscr;       // delta scratch
 };
-
-__device__ __forceinline__ uint32_t mask_pos_bf16x2(uint32_t v, uint32_t h) {
-  // ReLU backward on a packed pair: v * (h > 0), two instructions (HSET2.BF16.GT + HMUL2.BF16)
-  const __nv_bfloat162 hv = *reinterpret_cast<const __nv_bfloat162*>(&h);
-  const __nv_bfloat162 vv = *reinterpret_cast<const __nv_bfloat162*>(&v);
-  const __nv_bfloat162 r = __hmul2(vv, __hgt2(hv, __float2bfloat162_rn(0.f)));
-  return *reinterpret_cast<const uint32_t*>(&r);
-}
 
 // ------------------------------------------------------------------------------- wgrad
 __device__ __forceinline__ float warp_sum_f(float v) {

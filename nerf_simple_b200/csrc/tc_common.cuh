@@ -87,25 +87,11 @@ __device__ __forceinline__ void tma_bulk_store_wait_read() {
   asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 
-// Ask the TMA engine to pull a contiguous global range into L2 (no shared-memory destination).
-__device__ __forceinline__ void tma_prefetch_l2(const void* gmem, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(gmem), "r"(bytes) : "memory");
-}
-
-// L2 cache-policy variants (createpolicy): keep prefetched tiles against the streaming stores / mark
-// streamed-out tiles as first to go.
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
+// L2 cache policy for streamed-out tiles: first to go.
 __device__ __forceinline__ uint64_t l2_policy_evict_first() {
   uint64_t p;
   asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
   return p;
-}
-__device__ __forceinline__ void tma_prefetch_l2_hint(const void* gmem, uint32_t bytes, uint64_t policy) {
-  asm volatile("cp.async.bulk.prefetch.L2.global.L2::cache_hint [%0], %1, %2;" ::"l"(gmem), "r"(bytes), "l"(policy) : "memory");
 }
 __device__ __forceinline__ void tma_bulk_s2g_hint(void* dst_gmem, uint32_t src_smem, uint32_t bytes, uint64_t policy) {
   asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;" ::"l"(dst_gmem), "r"(src_smem),
@@ -311,6 +297,12 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
 }
 __device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
   asm volatile("st.shared.v4.b32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
+}
+// LDS.128 of four floats; at a warp-uniform address it is one broadcast (staged biases, head weights)
+__device__ __forceinline__ float4 ld_shared_f4(uint32_t addr) {
+  float4 v;
+  asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
+  return v;
 }
 // byte offset of 16-byte chunk j (0..7) of row r inside a [rows x 128 B] SWIZZLE_128B image
 __host__ __device__ __forceinline__ uint32_t sw128_off(uint32_t r, uint32_t j) {
